@@ -15,6 +15,12 @@ spp_ba_set_graph (H2D + symbolic analysis) + spp_ba_optimize + spp_ba_get_states
 Rank 0 prints ONE JSON line. Timing: CUDA events on the context's stream, barrier + synchronize on both sides,
 max over ranks. The working set (W, Y: 2 x 409 MB; S: 220 MB) is far larger than the 126 MB L2, so consecutive
 steps do not find their inputs in cache ("inputs larger than L2").
+
+--dump-outputs DIR writes what the last timed step handed its caller as DIR/<name>.npy (float64): the optimised
+camera states and landmark positions (spp_ba_get_states; `poses` on the pose-graph shapes) and the LM trace of the
+report, with the prefix `bal13682_` for the second block of the headline line. The graphs are seeded, so two builds
+run with the same arguments can be compared array for array. Landmark arrays above DUMP_MAX_ROWS rows are replaced by
+a fixed, seeded sample of rows (`<name>_rows.npy` holds their indices), which keeps a dump under 64 MB.
 """
 import argparse
 import json
@@ -33,6 +39,21 @@ import numpy as np  # noqa: E402
 METRIC = "ba_lm_iterations_per_s"
 UNIT = "LM iterations/s"
 REF_BIN = os.path.join(ROOT, "oracle", "_ref", "ref_driver_ba")
+DUMP_MAX_ROWS = 1 << 20  # Venice-871 (530 304 landmarks) is dumped whole, BAL-13682 (4.46 M) as a sample
+
+
+def dump_outputs(out_dir, prefix, rep, arrays):
+    """Writes the report's LM trace and the given (name -> 2-D float64 array) outputs as out_dir/<prefix><name>.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    out = {"chi2_trace": rep["trace_chi2"], "alpha_trace": rep["trace_alpha"], "dx_norm_trace": rep["trace_dx_norm"],
+           "accepted_trace": rep["trace_accepted"], "chi2": [rep["chi2_initial"], rep["chi2_final"]]}
+    for name, a in arrays.items():
+        if a.shape[0] > DUMP_MAX_ROWS:
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], DUMP_MAX_ROWS, replace=False))
+            out[name + "_rows"], a = rows, a[rows]
+        out[name] = a
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), np.asarray(a, np.float64))
 
 
 _REAL_STDOUT = None
@@ -133,7 +154,8 @@ def run_reference_steps(graph_path, warmup, steps, threads=None):
     the per-step seconds of Optimize(1, 0) calls on the resident system."""
     from slam_plus_plus_b200 import sppio
     if not os.path.exists(REF_BIN):
-        raise RuntimeError("oracle/_ref/ref_driver_ba is missing (built by __graft_entry__.build() where /root/reference exists)")
+        raise RuntimeError("oracle/_ref/ref_driver_ba is missing (built by __graft_entry__.build() where the reference's "
+                           "sources are present, see oracle/build_ref.sh)")
     out = os.path.join(tempfile.gettempdir(), f"spp_bench_ref_{os.getpid()}.dump")
     env = dict(os.environ)
     if threads:
@@ -225,9 +247,8 @@ def gpu_arm(args):
     if args.shape == "venice871" and not args.no_bal:
         a2 = copy.copy(args)
         a2.shape = "bal13682"
-        a2.steps = min(args.steps, 3)
         try:
-            bal = measure_ba(a2, torch, dist, dev, rank, world, local)
+            bal = measure_ba(a2, torch, dist, dev, rank, world, local, dump_prefix="bal13682_")
         except Exception as ex:  # the headline line must still be printed
             bal = {"failed": repr(ex)}
         if rank == 0:
@@ -241,7 +262,7 @@ def gpu_arm(args):
         dist.destroy_process_group()
 
 
-def measure_ba(args, torch, dist, dev, rank, world, local):
+def measure_ba(args, torch, dist, dev, rank, world, local, dump_prefix=""):
     """One BA shape on the rank's GPU; returns the bench line (rank 0) or None."""
     from slam_plus_plus_b200 import capi, graphs
 
@@ -298,6 +319,10 @@ def measure_ba(args, torch, dist, dev, rank, world, local):
         t = torch.tensor([phase[k] for k in keys], dtype=torch.float64, device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         phase = {k: float(v) for k, v in zip(keys, t.tolist())}
+    if args.dump_outputs:  # the states the last timed step left on the device, read back outside the timed window
+        cams, pts = ctx.ba_gather_states() if world > 1 else ctx.ba_get_states()
+        if rank == 0:
+            dump_outputs(args.dump_outputs, dump_prefix, rep, {"cams": cams, "points": pts})
     sparse_rcs = 6 * g.n_cams > 16384  # SPP_RCS_AUTO: block-sparse (supernodal) reduced camera system above 16 384 unknowns
     rcs_info = ctx.schur_get_rcs_info() if sparse_rcs else None
 
@@ -475,6 +500,8 @@ def pose_arm(args):
     sampler.stop_flag = True
     ms = e0.elapsed_time(e1)
     launches = ctx.kernel_launches - l0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, "", rep, {"poses": ctx.pose_get_states()})
     t0 = time.perf_counter()
     for _ in range(args.steps):  # end to end with host buffers: upload + structure + optimise + download
         ctx.pose_set_graph(g)
@@ -522,7 +549,7 @@ def pose_arm(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps of every shape measured (the BAL-13682 block included)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--shape", default="venice871")
@@ -532,6 +559,8 @@ def main():
                     help="fd: forward differences with delta = 1e-9, the reference's own Jacobians (parity mode, the default and "
                          "the configuration of the headline number); analytic: closed-form derivatives")
     ap.add_argument("--no-bal", action="store_true", help="skip the BAL-13682-shape block of the headline line")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR", help="write what the last timed step computed (optimised states, "
+                    "LM trace) to DIR/<name>.npy, float64, under 64 MB in all")
     ap.add_argument("--write-chi2-trace", default="", metavar="PATH", help="single-GPU run: record the final chi2 of each shape in this "
                     "JSON file (committed as profiles/chi2_trace.json, which every later run is checked against)")
     args = ap.parse_args()
@@ -539,6 +568,8 @@ def main():
     if args.shape in POSE_SHAPES and args.impl == "b200":
         pose_arm(args)
     elif args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs dumps the outputs of this repository's GPU path (--impl b200)")
         reference_arm(args)
     else:
         gpu_arm(args)

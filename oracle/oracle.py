@@ -94,7 +94,42 @@ def relative_to_absolute(v1, v2):
     return d
 
 
-def ba_optimize(g, max_iter=5, min_dx=0.0, max_trace=64):
+_BA_SOLVER = C.CFUNCTYPE(C.c_int, C.c_size_t, C.c_size_t, C.c_size_t, *([C.POINTER(C.c_double)] * 5), C.c_double,
+                         C.POINTER(C.c_double), C.POINTER(C.c_double))
+_POSE_SOLVER = C.CFUNCTYPE(C.c_int, C.c_size_t, C.POINTER(C.c_double), C.POINTER(C.c_double))
+
+
+def _arr(p, n):
+    return np.ctypeslib.as_array(p, shape=(n,))
+
+
+def ba_optimize(g, max_iter=5, min_dx=0.0, max_trace=64, linear_solver=None):
+    """The reference's LM loop. linear_solver(U, V, W, gc, gp, alpha) -> (status, dxc, dxp), if given, takes the place of
+    the oracle's own Schur solve (the reference's linear-solver slot)."""
+    if linear_solver is not None:
+        errors = []
+
+        def cb(c, p, o, U, V, W, gc, gp, alpha, dxc, dxp):
+            try:
+                rc, xc, xp = linear_solver(_arr(U, c * 36).reshape(c, 36), _arr(V, p * 9).reshape(p, 9),
+                                           _arr(W, o * 18).reshape(o, 18), _arr(gc, c * 6).reshape(c, 6),
+                                           _arr(gp, p * 3).reshape(p, 3), alpha)
+                if rc == 0:
+                    _arr(dxc, c * 6)[:] = np.ravel(xc)
+                    _arr(dxp, p * 3)[:] = np.ravel(xp)
+                return rc
+            except BaseException as ex:  # stops the C loop; raised again once it has returned
+                errors.append(ex)
+                return -1
+        fn = _BA_SOLVER(cb)
+        lib().spo_set_ba_linear_solver(fn)
+        try:
+            r = ba_optimize(g, max_iter, min_dx, max_trace)
+        finally:
+            lib().spo_set_ba_linear_solver(None)
+        if errors:
+            raise errors[0]
+        return r
     args, keep = _graph_args(g)
     cam_out, pts_out = np.zeros((g.n_cams, 6)), np.zeros((g.n_pts, 3))
     trace = np.zeros((max_trace, 6))
@@ -197,7 +232,30 @@ def pose_linearise_dense(g, poses=None):
     return lam, eta  # symmetric: row/column-major agree
 
 
-def pose_optimize(g, max_iter=5, min_dx=0.0):
+def pose_optimize(g, max_iter=5, min_dx=0.0, linear_solver=None):
+    """The reference's Gauss-Newton loop. linear_solver(lambda, eta) -> (status, dx), if given, takes the place of the
+    oracle's own dense solve (the reference's linear-solver slot); lambda is dense and symmetric."""
+    if linear_solver is not None:
+        errors = []
+
+        def cb(n, lam, eta):
+            try:
+                rc, dx = linear_solver(_arr(lam, n * n).reshape(n, n), _arr(eta, n).copy())
+                if rc == 0:
+                    _arr(eta, n)[:] = dx
+                return rc
+            except BaseException as ex:  # stops the C loop; raised again once it has returned
+                errors.append(ex)
+                return -1
+        fn = _POSE_SOLVER(cb)
+        lib().spo_set_pose_linear_solver(fn)
+        try:
+            r = pose_optimize(g, max_iter, min_dx)
+        finally:
+            lib().spo_set_pose_linear_solver(None)
+        if errors:
+            raise errors[0]
+        return r
     args, keep = _pose_args(g)
     out, norms = np.zeros(3), np.zeros(max(max_iter, 1))
     rc = _fn(g, "optimize")(*args, C.c_size_t(max_iter), C.c_double(min_dx), _p(out, C.c_double), _p(norms, C.c_double))

@@ -482,6 +482,14 @@ SPO_API void spo_relative_to_absolute(const double *v1, const double *v2, double
 	relative_to_absolute(v1, v2, dest);
 }
 
+/* Optional replacement of the linear solve inside spo_ba_optimize: the reference's linear-solver slot, so that a
+ * solver under test (the GPU library through its C ABI) can run inside the reference's LM loop. Receives the
+ * linearisation (U, V, W, gc, gp as spo_ba_linearise returns them) and the damping; writes dxc, dxp; nonzero = failed. */
+typedef int (*spo_ba_solver_t)(size_t C, size_t P, size_t O, const double *U, const double *V, const double *W,
+	const double *gc, const double *gp, double alpha, double *dxc, double *dxp);
+static spo_ba_solver_t g_ba_solver = 0;
+SPO_API void spo_set_ba_linear_solver(spo_ba_solver_t f) { g_ba_solver = f; }
+
 /* CNonlinearSolver_Lambda_LM::Optimize, LM:796-1116, batch use. trace: 6 doubles per solve
  * (alpha before, chi2 last, chi2 new, dx.(alpha dx + eta), accepted, alpha after), at most max_trace solves.
  * cam_out: C x 6, pts_out: P x 3. scalars: [0] chi2 initial, [1] chi2 final, [2] alpha initial, [3] n solves,
@@ -516,7 +524,8 @@ SPO_API int spo_ba_optimize(size_t nv, const uint8_t *vtype, const double *cams1
 			if(it && b_dirty) /* LM:942-949; after a rejected step only the damping changes */
 				ba_linearise(&g, U, V, W, gc, gp);
 			b_dirty = 0;
-			int rc = schur_solve(C, P, O, oc, op, U, V, W, gc, gp, f_alpha, dxc, dxp, 0, 0); /* LM:967, 1512-1568 */
+			int rc = (g_ba_solver)? g_ba_solver(C, P, O, U, V, W, gc, gp, f_alpha, dxc, dxp) :
+				schur_solve(C, P, O, oc, op, U, V, W, gc, gp, f_alpha, dxc, dxp, 0, 0); /* LM:967, 1512-1568 */
 			double *t = (n_solves < max_trace)? trace + n_solves * 6 : 0;
 			++ n_solves;
 			if(t) { t[0] = f_alpha; t[1] = f_last_error; t[2] = t[3] = t[4] = 0; t[5] = f_alpha; }
@@ -683,6 +692,22 @@ SPO_API int spo_se2_linearise_dense(size_t N, const double *states, size_t E, co
 	return 0;
 }
 
+/* Optional replacement of the linear solve inside spo_se2_optimize / spo_se3_optimize (the reference's linear-solver
+ * slot): solves lambda (n x n, dense, symmetric) dx = eta in place of eta; nonzero = failed. */
+typedef int (*spo_pose_solver_t)(size_t n, const double *lambda, double *eta);
+static spo_pose_solver_t g_pose_solver = 0;
+SPO_API void spo_set_pose_linear_solver(spo_pose_solver_t f) { g_pose_solver = f; }
+
+static int pose_solve(size_t n, double *lambda, double *eta)
+{
+	if(g_pose_solver)
+		return g_pose_solver(n, lambda, eta);
+	if(dense_llt_upper(n, lambda))
+		return 1;
+	dense_llt_solve(n, lambda, eta);
+	return 0;
+}
+
 /* CNonlinearSolver_Lambda::Optimize (GN:476-667) with a dense LLT standing in for the block-sparse one (the
  * Cholesky factor is unique: CLinearSolver_UberBlock, UB:312-426, yields the same increment up to rounding).
  * out[0] = chi2 before, out[1] = chi2 after, out[2] = number of solves; dx_norms[k] per solve. */
@@ -697,8 +722,7 @@ SPO_API int spo_se2_optimize(size_t N, double *states, size_t E, const uint64_t 
 	int rc = 0;
 	for(size_t it = 0; it < max_iter; ++ it) {
 		spo_se2_linearise_dense(N, states, E, from, to, z, info, lambda, eta);
-		if(dense_llt_upper(n, lambda)) { rc = 1; ++ n_solves; break; }
-		dense_llt_solve(n, lambda, eta);
+		if(pose_solve(n, lambda, eta)) { rc = 1; ++ n_solves; break; }
 		double s = 0;
 		for(size_t i = 0; i < n; ++ i) s += eta[i] * eta[i];
 		dx_norms[n_solves ++] = sqrt(s);
@@ -871,8 +895,7 @@ SPO_API int spo_se3_optimize(size_t N, double *states, size_t E, const uint64_t 
 	int rc = 0;
 	for(size_t it = 0; it < max_iter; ++ it) {
 		spo_se3_linearise_dense(N, states, E, from, to, z, info, lambda, eta);
-		if(dense_llt_upper(n, lambda)) { rc = 1; ++ n_solves; break; }
-		dense_llt_solve(n, lambda, eta);
+		if(pose_solve(n, lambda, eta)) { rc = 1; ++ n_solves; break; }
 		double s = 0;
 		for(size_t i = 0; i < n; ++ i) s += eta[i] * eta[i];
 		dx_norms[n_solves ++] = sqrt(s);

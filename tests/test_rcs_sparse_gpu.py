@@ -168,17 +168,23 @@ def test_bal_sixteenth_against_the_reference_itself(tmp_path):
     library with the block-sparse (supernodal) reduced-camera-system solver forced, and with the dense one -- the final
     chi2 of Optimize(2, 0) within the north-star 1e-6, the two device paths within 1e-7 of each other (measured 2e-9:
     their increments differ in the 13th digit, and the second linearisation -- forward differences with delta = 1e-9 --
-    amplifies that by 1e9 eps in the Jacobians)."""
+    amplifies that by 1e9 eps in the Jacobians). The reference's result is taken from its drivers where they are built,
+    and from tests/golden/oracle_runs.json where that file records it ("reference_chi2_final"). The same Optimize(2, 0)
+    by the CPU oracle (the reference's plain-C restatement), stored there as well, is held to the same bounds on every
+    run, so that the test also checks something where neither is available."""
+    import json
     import subprocess
     from slam_plus_plus_b200 import capi, graphs, sppio
-    ref_bin = os.path.join(os.path.dirname(GOLDEN), "..", "oracle", "_ref", "ref_driver_ba")
-    if not os.path.exists(ref_bin):
-        pytest.skip("oracle/_ref/ref_driver_ba not built (needs /root/reference at build time)")
     g = graphs.make_ba(13682 // 16, 4456117 // 16, 13682, mean_extra_track=4.5, max_track=120, max_stride=12, loops=1)
-    gp, dp = str(tmp_path / "g.bin"), str(tmp_path / "ref.dump")
-    sppio.write_graph(gp, g)
-    subprocess.run([ref_bin, "time", gp, dp, "2", "0"], check=True, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
-    chi2_ref = float(sppio.read_dump(dp)["chi2"][0])
+    with open(os.path.join(GOLDEN, "oracle_runs.json")) as f:
+        stored = json.load(f)["bal_sixteenth"]
+    chi2_refs = [stored["chi2_final"]] + ([stored["reference_chi2_final"]] if "reference_chi2_final" in stored else [])
+    ref_bin = os.path.join(os.path.dirname(GOLDEN), "..", "oracle", "_ref", "ref_driver_ba")
+    if os.path.exists(ref_bin):
+        gp, dp = str(tmp_path / "g.bin"), str(tmp_path / "ref.dump")
+        sppio.write_graph(gp, g)
+        subprocess.run([ref_bin, "time", gp, dp, "2", "0"], check=True, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+        chi2_refs.append(float(sppio.read_dump(dp)["chi2"][0]))
     chi2 = {}
     for mode in (capi.RCS_SPARSE, capi.RCS_DENSE):
         ctx = capi.Context(0)
@@ -190,6 +196,7 @@ def test_bal_sixteenth_against_the_reference_itself(tmp_path):
             info = ctx.schur_get_rcs_info()
             assert info["cameras"] == g.n_cams and info["supernodes"] >= 1
         ctx.close()
-    assert abs(chi2[capi.RCS_SPARSE] - chi2_ref) <= 1e-6 * chi2_ref, (chi2, chi2_ref)
-    assert abs(chi2[capi.RCS_DENSE] - chi2_ref) <= 1e-6 * chi2_ref, (chi2, chi2_ref)
-    assert abs(chi2[capi.RCS_SPARSE] - chi2[capi.RCS_DENSE]) <= 1e-7 * chi2_ref
+    for chi2_ref in chi2_refs:
+        assert abs(chi2[capi.RCS_SPARSE] - chi2_ref) <= 1e-6 * chi2_ref, (chi2, chi2_ref)
+        assert abs(chi2[capi.RCS_DENSE] - chi2_ref) <= 1e-6 * chi2_ref, (chi2, chi2_ref)
+        assert abs(chi2[capi.RCS_SPARSE] - chi2[capi.RCS_DENSE]) <= 1e-7 * chi2_ref
