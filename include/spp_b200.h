@@ -237,6 +237,13 @@ int spp_schur_solve(spp_ctx_t ctx, const double *p_values, double *p_eta_dx);
  * group in the order of the block columns. Same requirements and return values as spp_ba_marginals. */
 int spp_schur_marginals(spp_ctx_t ctx, double alpha, double *p_cam_cov, double *p_pt_cov);
 
+/* Block diagonal of (lambda + alpha I)^-1 like spp_ba_marginals, recovered from the block-sparse (supernodal)
+ * factorisation of the reduced camera system by selected inversion: no dense S^-1, any number of cameras. Uses the
+ * supernodal path whatever spp_schur_set_rcs_solver says. Same output layout and return values as spp_ba_marginals. */
+int spp_ba_marginals_sparse(spp_ctx_t ctx, double alpha, double *p_cam_cov, double *p_pt_cov);
+/* the same on the lambda of the last spp_schur_solve (slot 1), output as spp_schur_marginals */
+int spp_schur_marginals_sparse(spp_ctx_t ctx, double alpha, double *p_cam_cov, double *p_pt_cov);
+
 /* Stage outputs of the last Schur solve, for the parity tests (SURVEY 8(c) P1): the reduced camera system as a
  * dense column-major (6C x 6C) matrix (upper triangle valid), its right-hand side, and the pattern of non-zero
  * 6x6 blocks of the upper triangle (row-major bitmap, C*C bytes). Any pointer may be NULL. */

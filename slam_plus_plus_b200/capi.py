@@ -26,7 +26,7 @@ EXPORTED_SYMBOLS = [
     "spp_synchronize", "spp_set_allreduce", "spp_partition_landmarks", "spp_rcs_block_pattern", "spp_ba_get_partition", "spp_ba_set_graph", "spp_ba_append_graph", "spp_ba_set_states", "spp_ba_get_states", "spp_ba_gather_states",
     "spp_ba_restore_initial", "spp_ba_set_jacobian_mode", "spp_ba_linearise", "spp_ba_get_lambda", "spp_ba_get_blocks", "spp_ba_chi2", "spp_ba_solve_step",
     "spp_ba_optimize", "spp_ba_marginals", "spp_schur_symbolic", "spp_schur_solve", "spp_schur_marginals",
-    "spp_schur_get_reduced_system",
+    "spp_ba_marginals_sparse", "spp_schur_marginals_sparse", "spp_schur_get_reduced_system",
     "spp_schur_set_rcs_solver", "spp_schur_set_rcs_ordering", "spp_schur_get_rcs_info", "spp_schur_get_rcs_owners", "spp_schur_get_rcs_residual", "spp_block_ordering",
     "spp_block_symbolic_stats", "spp_block_subtree_owners", "spp_dense_posdef_solve", "spp_dense_panel_factor", "spp_nccl_get_unique_id", "spp_set_nccl",
     "spp_chol_symbolic", "spp_chol_solve", "spp_chol_get_factor",
@@ -109,6 +109,8 @@ def load_library() -> C.CDLL:
     lib.spp_schur_solve.argtypes = [vp, dp, dp]
     lib.spp_ba_marginals.argtypes = [vp, C.c_double, dp, dp]
     lib.spp_schur_marginals.argtypes = [vp, C.c_double, dp, dp]
+    lib.spp_ba_marginals_sparse.argtypes = [vp, C.c_double, dp, dp]
+    lib.spp_schur_marginals_sparse.argtypes = [vp, C.c_double, dp, dp]
     lib.spp_schur_get_reduced_system.argtypes = [vp, u64p, dp, dp, u8p]
     lib.spp_dense_posdef_solve.argtypes = [vp, C.c_size_t, dp, dp]
     lib.spp_dense_panel_factor.argtypes = [vp, C.c_size_t, C.c_size_t, dp]
@@ -444,6 +446,14 @@ class Context:
         self._check(self.lib.spp_ba_marginals(self.h, alpha, _dp(cc), _dp(pc)))
         return cc, pc
 
+    def ba_marginals_sparse(self, alpha: float = 0.0):
+        """ba_marginals through the block-sparse (supernodal) factorisation and its selected inversion: no dense inverse,
+        any number of cameras. (C, 6, 6), (P, 3, 3)."""
+        c, p, _, _ = self._ba_dims
+        cc, pc = np.empty((c, 6, 6)), np.empty((p, 3, 3))
+        self._check(self.lib.spp_ba_marginals_sparse(self.h, alpha, _dp(cc), _dp(pc)))
+        return cc, pc
+
     # ---- slot 1: Schur linear solver on a caller-supplied lambda ---------------------------------
     def schur_symbolic(self, col_dims, col_ptr, row_idx):
         cd = np.ascontiguousarray(col_dims, np.uint64)
@@ -462,6 +472,13 @@ class Context:
         c, p = self._schur_cut
         cc, pc = np.empty((c, 6, 6)), np.empty((p, 3, 3))
         self._check(self.lib.spp_schur_marginals(self.h, alpha, _dp(cc), _dp(pc)))
+        return cc, pc
+
+    def schur_marginals_sparse(self, alpha: float = 0.0):
+        """schur_marginals through the block-sparse (supernodal) factorisation and its selected inversion."""
+        c, p = self._schur_cut
+        cc, pc = np.empty((c, 6, 6)), np.empty((p, 3, 3))
+        self._check(self.lib.spp_schur_marginals_sparse(self.h, alpha, _dp(cc), _dp(pc)))
         return cc, pc
 
     def schur_solve(self, values, eta) -> np.ndarray:

@@ -28,6 +28,54 @@ __device__ __forceinline__ double minus_inv_at(const double *__restrict__ Ni, si
 	return (r <= c)? Ni[(size_t)c * ld + r] : Ni[(size_t)r * ld + c];
 }
 
+// (-S^-1)_ab of the dense path: the upper tiles of minus the inverse, ld x ld
+struct DenseMinusInverse {
+	const double *Ni;
+	size_t ld;
+	struct Block {
+		const double *Ni;
+		size_t ld;
+		unsigned r0, c0;
+		__device__ __forceinline__ double operator()(int i, int j) const { return minus_inv_at(Ni, ld, r0 + i, c0 + j); }
+	};
+	__device__ __forceinline__ Block block(unsigned ca, unsigned cb) const { Block b = {Ni, ld, ca * 6, cb * 6}; return b; }
+};
+
+// (-S^-1)_ab after the selected inversion (selinv.cu): block (min(a, b), max(a, b)) of S is found by a binary search in
+// its column of the upper block CSC; d_asm_dst gives where the factorisation assembled it in the panels, and so where
+// Z holds it now (bit 63: stored transposed). A diagonal block is read through its upper triangle.
+struct PanelInverse {
+	const double *L;
+	const uint64_t *csc_ptr, *dst;
+	const uint32_t *csc_row, *csc_blk, *ld;
+	struct Block {
+		const double *P;
+		size_t ld;
+		int mode; // 0: as stored, 1: transposed, 2: symmetric
+		__device__ __forceinline__ double operator()(int i, int j) const
+		{
+			const bool tr = mode == 1 || (mode == 2 && i > j);
+			return -(tr? P[(size_t)i * ld + j] : P[(size_t)j * ld + i]);
+		}
+	};
+	__device__ __forceinline__ Block block(unsigned ca, unsigned cb) const
+	{
+		const unsigned lo = min(ca, cb), hi = max(ca, cb);
+		uint64_t a = csc_ptr[hi], b = csc_ptr[hi + 1]; // the last entry with row <= lo: the block (it is in the pattern)
+		while(b - a > 1) {
+			const uint64_t m = (a + b) >> 1;
+			if(csc_row[m] <= lo) a = m; else b = m;
+		}
+		const uint32_t k = csc_blk[a];
+		const uint64_t d = dst[k];
+		Block r;
+		r.P = L + (d & ~((uint64_t)1 << 63));
+		r.ld = ld[k];
+		r.mode = (ca == cb)? 2 : ((((d >> 63) != 0) != (ca > cb))? 1 : 0);
+		return r;
+	}
+};
+
 // thread per element: cov[c * 36 + i * 6 + j] = (S^-1)(6c + i, 6c + j)
 __global__ void k_camera_marginals(size_t C, const double *__restrict__ Ni, size_t ld, double *__restrict__ cov)
 {
@@ -43,10 +91,13 @@ __global__ void k_camera_marginals(size_t C, const double *__restrict__ Ni, size
 // correct, but the whole call went from 13.9 ms to 40 - 70 ms on the Venice shape; the same happened with 16-byte loads of
 // the stored block columns (LDG.128 in the SASS, 22 - 67 ms). Both runs were erratic from call to call, which the kernel
 // alone does not explain; not resolved within the round's GPU budget -- the next step is a per-kernel ncu timing of both.)
+// The blocks (-S^-1)_ab come from an accessor: DenseMinusInverse (the dense path) or PanelInverse (selected inversion on
+// the supernodal panels).
 #define PM_WARPS 4
+template <class Inv>
 __global__ void __launch_bounds__(PM_WARPS * 32) k_point_marginals(size_t P, const uint32_t *__restrict__ pt_ptr,
 	const uint32_t *__restrict__ obs_cam, const double *__restrict__ Y, const double *__restrict__ Cinv,
-	const double *__restrict__ Ni, size_t ld, double *__restrict__ cov)
+	const Inv inv, double *__restrict__ cov)
 {
 	const size_t p = blockIdx.x * (size_t)PM_WARPS + (threadIdx.x >> 5);
 	if(p >= P) return;
@@ -69,11 +120,12 @@ __global__ void __launch_bounds__(PM_WARPS * 32) k_point_marginals(size_t P, con
 		double t[18]; // t = (-S^-1)_ab Y_b, 6 x 3 column-major
 		#pragma unroll
 		for(int i = 0; i < 18; ++ i) t[i] = 0;
+		const typename Inv::Block blk = inv.block(ca, cb);
 		#pragma unroll
 		for(int j = 0; j < 6; ++ j) {
 			#pragma unroll
 			for(int i = 0; i < 6; ++ i) {
-				const double m = minus_inv_at(Ni, ld, ca * 6 + i, cb * 6 + j);
+				const double m = blk(i, j);
 				t[i] += m * yb[j];
 				t[6 + i] += m * yb[6 + j];
 				t[12 + i] += m * yb[12 + j];
@@ -128,9 +180,82 @@ int schur_marginals_current(spp_ctx *ctx, double alpha, double *d_cam_cov, doubl
 		LAUNCH_CHECK(ctx);
 	}
 	if(d_pt_cov && s.P) {
+		const DenseMinusInverse inv = {s.Sinv.p(), ld};
 		k_point_marginals<<<n_blocks(s.P, PM_WARPS), PM_WARPS * 32, 0, ctx->stream>>>(s.P, s.pt_ptr.p(), s.obs_cam.p(),
-			s.Y.p(), s.Cinv.p(), s.Sinv.p(), ld, d_pt_cov);
+			s.Y.p(), s.Cinv.p(), inv, d_pt_cov);
 		LAUNCH_CHECK(ctx);
+	}
+	return SPP_OK;
+}
+
+// ---- block-sparse reduced camera system ----------------------------------------------------------------------
+// The same marginals without a dense S^-1: supernodal factorisation of S (supernodal_chol.cu) and selected inversion of
+// the factor (selinv.cu), which leaves the entries of S^-1 on the pattern of R in the panels. Every camera pair seen by
+// one landmark is a block of S, so the panels hold every block the landmark sums need.
+
+void snode_symbolic(spp_ctx *ctx, size_t n, const std::vector<uint32_t> &blk_row, const std::vector<uint32_t> &blk_col);
+void schur_fetch_host_pattern(spp_ctx *ctx);
+void snode_factor(spp_ctx *ctx, const double *d_Sblk, const double *d_b);
+void snode_selected_inverse(spp_ctx *ctx);
+
+// thread per element: cov[c * 36 + i * 6 + j] = Z(6c + i, 6c + j), the diagonal block read through its upper triangle
+__global__ void k_camera_marginals_panels(size_t C, const double *__restrict__ L, const uint64_t *__restrict__ diag,
+	const uint32_t *__restrict__ ld, double *__restrict__ cov)
+{
+	size_t k = blockIdx.x * (size_t)blockDim.x + threadIdx.x;
+	if(k >= C * 36) return;
+	const size_t c = k / 36;
+	const unsigned e = (unsigned)(k % 36), i = e / 6, j = e % 6;
+	const double *P = L + diag[c];
+	cov[k] = (i <= j)? P[(size_t)j * ld[c] + i] : P[(size_t)i * ld[c] + j];
+}
+
+// Marginals of the system held as (U, V, W) through the supernodal path, d_cam_cov [36 C], d_pt_cov [9 P] (either may be
+// null). Re-forms the block list of S at this damping and overwrites the panels with Z: the last solve's S is gone, so
+// the residual check of that solve is refused afterwards (sparse_solved); the next solve assembles its panels anew.
+// ms_phases (optional, [5]): Schur forming, factorisation, selected inversion, cameras, points. Returns SPP_OK /
+// SPP_NOT_POSDEF.
+int schur_marginals_sparse_current(spp_ctx *ctx, double alpha, double *d_cam_cov, double *d_pt_cov, float *ms_phases)
+{
+	SchurSystem &s = ctx->sys;
+	SupernodalChol &sc = ctx->snode;
+	cudaStream_t st = ctx->stream;
+	if(!sc.valid) { // as schur_solve_current makes it (one rank)
+		schur_fetch_host_pattern(ctx);
+		snode_symbolic(ctx, s.C, s.h_blk_row, s.h_blk_col);
+	}
+	cudaEvent_t *ev = ctx->ev + 10; // phase marks
+	SPP_CUDA(cudaEventRecord(ev[0], st));
+	schur_form_reduced_system(ctx, alpha, alpha, true); // Cinv, Y and the block list of S at this damping
+	s.sparse_solved = false;
+	SPP_CUDA(cudaEventRecord(ev[1], st));
+	snode_factor(ctx, s.Sblk.p(), 0);
+	SPP_CUDA(cudaEventRecord(ev[2], st));
+	ctx->h_scalars.resize(16);
+	int *h_info = reinterpret_cast<int*>(ctx->h_scalars.p());
+	SPP_CUDA(cudaMemcpyAsync(h_info, sc.d_info.p(), sizeof(int), cudaMemcpyDeviceToHost, st));
+	SPP_CUDA(cudaStreamSynchronize(st));
+	if(*h_info != 0)
+		return SPP_NOT_POSDEF;
+	SPP_CUDA(cudaEventRecord(sc.ev_factor[sc.sn.n_super() - 1], st)); // "factorisation complete" for the side lanes
+	snode_selected_inverse(ctx);
+	SPP_CUDA(cudaEventRecord(ev[3], st));
+	if(d_cam_cov && s.C) {
+		k_camera_marginals_panels<<<n_blocks(s.C * 36, 256), 256, 0, st>>>(s.C, sc.d_L.p(), sc.d_cam_diag.p(), sc.d_cam_ld.p(), d_cam_cov);
+		LAUNCH_CHECK(ctx);
+	}
+	SPP_CUDA(cudaEventRecord(ev[4], st));
+	if(d_pt_cov && s.P) {
+		const PanelInverse inv = {sc.d_L.p(), sc.d_csc_ptr.p(), sc.d_asm_dst.p(), sc.d_csc_row.p(), sc.d_csc_blk.p(), sc.d_asm_ld.p()};
+		k_point_marginals<<<n_blocks(s.P, PM_WARPS), PM_WARPS * 32, 0, st>>>(s.P, s.pt_ptr.p(), s.obs_cam.p(), s.Y.p(), s.Cinv.p(),
+			inv, d_pt_cov);
+		LAUNCH_CHECK(ctx);
+	}
+	SPP_CUDA(cudaEventRecord(ev[5], st));
+	if(ms_phases) {
+		SPP_CUDA(cudaEventSynchronize(ev[5]));
+		for(int i = 0; i < 5; ++ i)
+			SPP_CUDA(cudaEventElapsedTime(ms_phases + i, ev[i], ev[i + 1]));
 	}
 	return SPP_OK;
 }

@@ -44,6 +44,7 @@ void dense_chol_factor_panel(spp_ctx *ctx, double *A, size_t ld, size_t n_cols, 
 void dense_chol_factor_dataflow(spp_ctx *ctx, double *A, size_t ld, size_t n_cols, double *Rinv, int *info);
 bool dense_chol_dataflow_enabled();
 int schur_marginals_current(spp_ctx *ctx, double alpha, double *d_cam_cov, double *d_pt_cov);
+int schur_marginals_sparse_current(spp_ctx *ctx, double alpha, double *d_cam_cov, double *d_pt_cov, float *ms_phases);
 int pose_marginals(spp_ctx *ctx, double *d_cov);
 void slot_symbolic(spp_ctx *ctx, size_t n, const uint64_t *col_dims, const uint64_t *col_ptr, const uint64_t *row_idx,
 	uint64_t *p_order, uint64_t *p_cut);
@@ -1240,6 +1241,55 @@ int spp_schur_marginals(spp_ctx_t ctx, double alpha, double *p_cam_cov, double *
 	API_BEGIN(ctx)
 	if(!ctx->slot.valid || !ctx->slot.filled) throw invalid_error("no system: spp_schur_symbolic and spp_schur_solve first");
 	rc = marginals_to_host(ctx, alpha, p_cam_cov, p_pt_cov);
+	if(rc != SPP_OK) return rc;
+	API_END(ctx)
+}
+
+// the same through the block-sparse (supernodal) factorisation and its selected inversion, whatever the solver mode
+static int marginals_sparse_to_host(spp_ctx *ctx, double alpha, double *p_cam_cov, double *p_pt_cov)
+{
+	SchurSystem &s = ctx->sys;
+	if(ctx->world > 1) throw invalid_error("marginals are not available on a landmark-partitioned (multi-GPU) context");
+	if(!s.C) throw invalid_error("no cameras");
+	DBuf<double> &d_cam = s.cov_cam, &d_pt = s.cov_pt;
+	if(p_cam_cov) d_cam.resize(s.C * 36);
+	if(p_pt_cov) d_pt.resize(s.P * 9);
+	// SPP_MARGINALS_TIMING: the phases of the call to stderr
+	static const bool timing = getenv("SPP_MARGINALS_TIMING") != 0;
+	float ms[5] = {0, 0, 0, 0, 0};
+	int rc = schur_marginals_sparse_current(ctx, alpha, p_cam_cov? d_cam.p() : 0, p_pt_cov? d_pt.p() : 0, timing? ms : 0);
+	if(rc != SPP_OK)
+		return rc;
+	if(timing) {
+		const SupernodalChol &sc = ctx->snode;
+		fprintf(stderr, "[spp marginals sparse] schur %.3f ms, factor %.3f ms, selected inversion %.3f ms (%.3e flops, %.2f TFLOP/s), "
+			"cameras %.3f ms, points %.3f ms; scratch %.3f GB (main) + %d x %.3f GB (lanes), panels %.3f GB\n", ms[0], ms[1], ms[2],
+			sc.selinv_flops, sc.selinv_flops / ms[2] * 1e-9, ms[3], ms[4], sc.selinv_main_doubles * 8e-9, (int)SupernodalChol::N_STREAMS,
+			sc.selinv_lane_doubles * 8e-9, sc.d_L.size() * 8e-9);
+	}
+	if(p_cam_cov) d_cam.download(p_cam_cov, s.C * 36, ctx->stream);
+	if(p_pt_cov) d_pt.download(p_pt_cov, s.P * 9, ctx->stream);
+	SPP_CUDA(cudaStreamSynchronize(ctx->stream));
+	return SPP_OK;
+}
+
+int spp_ba_marginals_sparse(spp_ctx_t ctx, double alpha, double *p_cam_cov, double *p_pt_cov)
+{
+	int rc = SPP_OK;
+	API_BEGIN(ctx)
+	if(!ctx->ba.valid) throw invalid_error("no BA graph");
+	if(!ctx->ba.linearised) ba_linearise(ctx, true);
+	rc = marginals_sparse_to_host(ctx, alpha, p_cam_cov, p_pt_cov);
+	if(rc != SPP_OK) return rc;
+	API_END(ctx)
+}
+
+int spp_schur_marginals_sparse(spp_ctx_t ctx, double alpha, double *p_cam_cov, double *p_pt_cov)
+{
+	int rc = SPP_OK;
+	API_BEGIN(ctx)
+	if(!ctx->slot.valid || !ctx->slot.filled) throw invalid_error("no system: spp_schur_symbolic and spp_schur_solve first");
+	rc = marginals_sparse_to_host(ctx, alpha, p_cam_cov, p_pt_cov);
 	if(rc != SPP_OK) return rc;
 	API_END(ctx)
 }

@@ -156,6 +156,11 @@ struct SnodeUpdate { // contribution of supernode s to its ancestor t: panel_t -
 	uint64_t map_off; // block positions in panel t of the suffix blocks, then of the rhs column
 };
 
+// selected inversion (selinv.cu): the structure of a supernode is padded to a multiple of SN_SEL_HP columns in its
+// scratch; supernodes with one diagonal block and a structure of at most SN_SEL_LANE_MAX_H columns run on the side lanes
+enum { SN_SEL_HP = 64, SN_SEL_LANE_MAX_H = 2048 };
+inline bool selinv_on_lane(size_t ld, size_t hp) { return ld == 128 && hp <= SN_SEL_LANE_MAX_H; }
+
 struct SupernodalChol {
 	bool valid;
 	int mode;                              // SPP_RCS_*
@@ -172,6 +177,13 @@ struct SupernodalChol {
 	DBuf<uint64_t> d_asm_dst, d_rhs_dst, d_pad_off;
 	DBuf<double> d_L, d_Rinv, d_x, d_part;
 	DBuf<int> d_info;                      // [0] first non-positive pivot, [1..] backsolve flags
+	// marginals (selinv.cu): the upper block CSC of S in camera order with the block id of every entry, so that a device
+	// binary search finds the panel address of block (a, b) through d_asm_dst; the diagonal block of every camera
+	DBuf<uint64_t> d_csc_ptr, d_cam_diag;  // [n + 1], [n]
+	DBuf<uint32_t> d_csc_row, d_csc_blk, d_cam_ld;
+	double selinv_flops;                   // selected inversion, 2 w^3 / 3 + 2 w^2 h + 2 w h^2 per supernode (padding excluded)
+	size_t selinv_main_doubles, selinv_lane_doubles; // scratch: wide supernodes (main stream) / one side lane
+	DBuf<double> d_sel_main, d_sel_lane;
 	double factor_flops;                   // of the numeric phase as executed by THIS rank (amalgamation zeros included)
 	double factor_flops_total;             // the same for the whole factorisation (equal on one rank)
 	// several ranks: subtrees of the supernodal elimination tree belong to one rank each, the supernodes above them
@@ -191,7 +203,8 @@ struct SupernodalChol {
 	enum { N_STREAMS = 8 };
 	cudaStream_t side[N_STREAMS];
 	std::vector<cudaEvent_t> ev_factor, ev_target, ev_x;
-	SupernodalChol() : valid(false), mode(0), n(0), n_rinv_blocks(0), n_s_blocks(0), max_part(0), factor_flops(0),
+	SupernodalChol() : valid(false), mode(0), n(0), n_rinv_blocks(0), n_s_blocks(0), max_part(0), selinv_flops(0),
+		selinv_main_doubles(0), selinv_lane_doubles(0), factor_flops(0),
 		factor_flops_total(0), sym_world(0), sym_rank(0), sym_kept(false), distributed(false)
 	{
 		for(int i = 0; i < N_STREAMS; ++ i) side[i] = 0;

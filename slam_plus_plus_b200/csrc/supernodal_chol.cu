@@ -183,6 +183,36 @@ void snode_symbolic(spp_ctx *ctx, size_t n, const std::vector<uint32_t> &blk_row
 		const uint64_t ld = sc.panel_ld[t], h = 6 * (uint64_t)(sn.row_ptr[t + 1] - sn.row_ptr[t]);
 		rhs_dst[sc.h_order[j]] = sc.panel_off[t] + (ld + h) * ld + 6 * (uint64_t)(j - sn.first[t]);
 	}
+	// marginals: camera -> its diagonal block in the panels, and the block CSC (rows ascending, block id beside each row)
+	// through which a landmark finds the block of any camera pair of its track
+	std::vector<uint64_t> cam_diag(n);
+	std::vector<uint32_t> cam_ld(n), csc_row(nb), csc_blk(nb);
+	for(size_t c = 0; c < n; ++ c) {
+		const uint32_t j = inv[c];
+		const size_t t = sn.col_super[j];
+		cam_diag[c] = sc.panel_off[t] + 6 * (uint64_t)(j - sn.first[t]) * (sc.panel_ld[t] + 1);
+		cam_ld[c] = sc.panel_ld[t];
+	}
+	{
+		std::vector<std::pair<uint32_t, uint32_t> > entries(nb);
+		std::vector<uint64_t> fill(col_ptr.begin(), col_ptr.end() - 1);
+		for(size_t b = 0; b < nb; ++ b) entries[fill[blk_col[b]] ++] = std::make_pair(blk_row[b], (uint32_t)b);
+		for(size_t j = 0; j < n; ++ j) std::sort(entries.begin() + col_ptr[j], entries.begin() + col_ptr[j + 1]);
+		for(size_t e = 0; e < nb; ++ e) { csc_row[e] = entries[e].first; csc_blk[e] = entries[e].second; }
+	}
+	// selected inversion: flops, and scratch (W = R11^-1 and later, in the same place, G = Z_JJ; T = one block row of the
+	// W recursion; X = W R12). The supernodes with one diagonal block and a short structure run on the side lanes, each
+	// lane with scratch of its own; every other supernode runs on the main stream and shares one set
+	sc.selinv_flops = 0;
+	sc.selinv_main_doubles = sc.selinv_lane_doubles = 0;
+	for(size_t s = 0; s < ns; ++ s) {
+		const double w = 6.0 * (sn.first[s + 1] - sn.first[s]), h = 6.0 * (sn.row_ptr[s + 1] - sn.row_ptr[s]);
+		sc.selinv_flops += 2 * w * w * w / 3 + 2 * w * w * h + 2 * w * h * h;
+		const size_t ld = sc.panel_ld[s], hp = round_up((size_t)h, SN_SEL_HP);
+		const size_t need = std::max(ld * ld, hp * hp) + ld * (hp + SN_NB);
+		size_t &slot = selinv_on_lane(ld, hp)? sc.selinv_lane_doubles : sc.selinv_main_doubles;
+		slot = std::max(slot, need);
+	}
 	// updates s -> t with their relative-index maps
 	sc.updates.clear();
 	sc.upd_ptr.assign(ns + 1, 0);
@@ -220,6 +250,11 @@ void snode_symbolic(spp_ctx *ctx, size_t n, const std::vector<uint32_t> &blk_row
 	sc.d_pad_off.upload(pad_off, st);
 	sc.d_pad_ld.upload(pad_ld, st);
 	sc.d_pad_n0.upload(pad_n0, st);
+	sc.d_cam_diag.upload(cam_diag, st);
+	sc.d_cam_ld.upload(cam_ld, st);
+	sc.d_csc_ptr.upload(col_ptr, st);
+	sc.d_csc_row.upload(csc_row, st);
+	sc.d_csc_blk.upload(csc_blk, st);
 	sc.d_L.resize(total);
 	sc.d_Rinv.resize(n_rinv * SN_NB * SN_NB);
 	sc.d_Rinv.zero(st); // the diagonal-block kernel writes upper triangles only
@@ -456,9 +491,11 @@ __global__ void k_snode_flag_to_info(const double *__restrict__ flag, int *__res
 
 // ---- numeric phase ----------------------------------------------------------------------------------------
 
-// d_Sblk: compact 6x6 block list of S in the order of the list given to snode_symbolic; d_b: reduced right-hand side
-// (camera order); d_dx: camera increment out (camera order; may alias d_b). Returns SPP_OK / SPP_NOT_POSDEF.
-int snode_factor_solve(spp_ctx *ctx, const double *d_Sblk, const double *d_b, double *d_dx)
+// Numeric factorisation, enqueued: assembly of d_Sblk (compact 6x6 block list of S in the order of the list given to
+// snode_symbolic) and of d_b (reduced right-hand side, camera order; null: no right-hand side, the rhs columns stay zero)
+// into the panels, the elimination-order loop with its side streams (joined back into the context's stream), and the
+// status in d_info[0] (the same on every rank).
+void snode_factor(spp_ctx *ctx, const double *d_Sblk, const double *d_b)
 {
 	SupernodalChol &sc = ctx->snode;
 	if(!sc.valid)
@@ -502,8 +539,10 @@ int snode_factor_solve(spp_ctx *ctx, const double *d_Sblk, const double *d_b, do
 	}
 	k_snode_assemble<<<n_blocks(sc.n_s_blocks * 36, 256), 256, 0, st>>>(sc.n_s_blocks * 36, d_Sblk, sc.d_asm_dst.p(), sc.d_asm_ld.p(), L);
 	LAUNCH_CHECK(ctx);
-	k_snode_assemble_rhs<<<n_blocks(n * 6, 256), 256, 0, st>>>(n * 6, d_b, sc.d_rhs_dst.p(), L);
-	LAUNCH_CHECK(ctx);
+	if(d_b) {
+		k_snode_assemble_rhs<<<n_blocks(n * 6, 256), 256, 0, st>>>(n * 6, d_b, sc.d_rhs_dst.p(), L);
+		LAUNCH_CHECK(ctx);
+	}
 	const bool dist = sc.distributed && ctx->world > 1;
 	if(dist && ctx->rank != 0) { // the shared panels are summed over the ranks: S, the right-hand side and the identity
 		for(size_t s = 0; s < ns; ++ s) { // padding come from rank 0 alone, the others contribute their subtrees' updates
@@ -625,10 +664,7 @@ int snode_factor_solve(spp_ctx *ctx, const double *d_Sblk, const double *d_b, do
 		allreduce_device(ctx, sc.d_flag.p(), 1);
 		k_snode_flag_to_info<<<1, 1, 0, st>>>(sc.d_flag.p(), sc.d_info.p());
 		LAUNCH_CHECK(ctx);
-		SPP_CUDA(cudaMemsetAsync(d_dx, 0, n * 6 * sizeof(double), st)); // (d_b, which d_dx may alias, went into the panels)
 	}
-	if(!single_stream)
-		SPP_CUDA(cudaEventRecord(sc.ev_factor[ns - 1], st)); // "factorisation complete"
 	if(profile) {
 		double tf = 0, tu = 0, ff = 0, fu = 0, tf_small = 0, tu_small = 0;
 		size_t n_small = 0;
@@ -652,6 +688,30 @@ int snode_factor_solve(spp_ctx *ctx, const double *d_Sblk, const double *d_b, do
 				t_update[s], w * h * h / std::max(t_update[s], 1e-6f) * 1e-9);
 		}
 	}
+}
+
+// d_Sblk: compact 6x6 block list of S in the order of the list given to snode_symbolic; d_b: reduced right-hand side
+// (camera order); d_dx: camera increment out (camera order; may alias d_b). Returns SPP_OK / SPP_NOT_POSDEF.
+int snode_factor_solve(spp_ctx *ctx, const double *d_Sblk, const double *d_b, double *d_dx)
+{
+	snode_factor(ctx, d_Sblk, d_b);
+	SupernodalChol &sc = ctx->snode;
+	const Supernodes &sn = sc.sn;
+	const size_t ns = sn.n_super(), n = sc.n;
+	cudaStream_t st = ctx->stream;
+	double *L = sc.d_L.p();
+	static const bool profile = getenv("SPP_SNODE_PROFILE") != 0;
+	static const bool single_stream = profile || getenv("SPP_SNODE_SINGLE_STREAM") != 0;
+	const bool dist = sc.distributed && ctx->world > 1;
+	if(dist) // the increments of the subtrees are summed at the end: start from zero
+		SPP_CUDA(cudaMemsetAsync(d_dx, 0, n * 6 * sizeof(double), st)); // (d_b, which d_dx may alias, went into the panels)
+	if(!single_stream)
+		SPP_CUDA(cudaEventRecord(sc.ev_factor[ns - 1], st)); // "factorisation complete"
+	auto lap = [&](float *acc) {
+		cudaEventRecord(ctx->ev[5], st);
+		cudaEventSynchronize(ctx->ev[5]);
+		cudaEventElapsedTime(acc, ctx->ev[4], ctx->ev[5]);
+	};
 	// backward solve, root to leaves; y_s sits in the rhs column of panel s. A supernode needs the x of its ancestors
 	// only: supernodes go round-robin to the side streams and wait for their parent's event (which implies the
 	// grandparents'), so independent subtrees are solved side by side
