@@ -244,6 +244,25 @@ int spp_ba_marginals_sparse(spp_ctx_t ctx, double alpha, double *p_cam_cov, doub
 /* the same on the lambda of the last spp_schur_solve (slot 1), output as spp_schur_marginals */
 int spp_schur_marginals_sparse(spp_ctx_t ctx, double alpha, double *p_cam_cov, double *p_pt_cov);
 
+/* Selected blocks of (lambda + alpha I)^-1 in one factorisation + inversion, on the dense or supernodal reduced camera
+ * system as spp_schur_set_rcs_solver selects. Cameras by index (id order among cameras), observations by edge insertion
+ * index. p_pair_cov[36 n_pairs]: Cov(cam_a[k], cam_b[k]), 6x6 column-major; the pair must share a landmark or be equal.
+ * p_obs_cov[18 n_obs]: Cov(camera, point) of observation p_obs[k], 6x3 column-major (the layout of W in
+ * spp_ba_get_blocks). p_cam_cov / p_pt_cov: the block diagonal, bit-identical to spp_ba_marginals(_sparse) on that path.
+ * Any output may be NULL (with its count 0). SPP_OK / SPP_NOT_POSDEF / SPP_ERR_INVALID.
+ * Extends the marginals of CSchurComplement_Marginals::Schur_Marginals (include/slam/BAMarginals.h:579-760), which
+ * computes the block diagonal only. On the supernodal path the state rules of spp_ba_marginals_sparse apply. */
+int spp_ba_covariance_blocks(spp_ctx_t ctx, double alpha,
+	size_t n_pairs, const uint64_t *p_cam_a, const uint64_t *p_cam_b, double *p_pair_cov,
+	size_t n_obs, const uint64_t *p_obs, double *p_obs_cov,
+	double *p_cam_cov, double *p_pt_cov);
+
+/* Slot 1: (lambda + alpha I)^-1 restricted to the block pattern of the lambda of the last spp_schur_solve, written in the
+ * layout of that call's p_values (n_values doubles): diagonal blocks and every camera-landmark block. Extends
+ * Schur_Marginals (include/slam/BAMarginals.h:579-760), which computes the block diagonal only. Path as
+ * spp_ba_covariance_blocks. SPP_OK / SPP_NOT_POSDEF / SPP_ERR_INVALID. */
+int spp_schur_covariance_pattern(spp_ctx_t ctx, double alpha, double *p_cov_values);
+
 /* Stage outputs of the last Schur solve, for the parity tests (SURVEY 8(c) P1): the reduced camera system as a
  * dense column-major (6C x 6C) matrix (upper triangle valid), its right-hand side, and the pattern of non-zero
  * 6x6 blocks of the upper triangle (row-major bitmap, C*C bytes). Any pointer may be NULL. */

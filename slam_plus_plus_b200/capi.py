@@ -26,7 +26,8 @@ EXPORTED_SYMBOLS = [
     "spp_synchronize", "spp_set_allreduce", "spp_partition_landmarks", "spp_rcs_block_pattern", "spp_ba_get_partition", "spp_ba_set_graph", "spp_ba_append_graph", "spp_ba_set_states", "spp_ba_get_states", "spp_ba_gather_states",
     "spp_ba_restore_initial", "spp_ba_set_jacobian_mode", "spp_ba_linearise", "spp_ba_get_lambda", "spp_ba_get_blocks", "spp_ba_chi2", "spp_ba_solve_step",
     "spp_ba_optimize", "spp_ba_marginals", "spp_schur_symbolic", "spp_schur_solve", "spp_schur_marginals",
-    "spp_ba_marginals_sparse", "spp_schur_marginals_sparse", "spp_schur_get_reduced_system",
+    "spp_ba_marginals_sparse", "spp_schur_marginals_sparse", "spp_ba_covariance_blocks", "spp_schur_covariance_pattern",
+    "spp_schur_get_reduced_system",
     "spp_schur_set_rcs_solver", "spp_schur_set_rcs_ordering", "spp_schur_get_rcs_info", "spp_schur_get_rcs_owners", "spp_schur_get_rcs_residual", "spp_block_ordering",
     "spp_block_symbolic_stats", "spp_block_subtree_owners", "spp_dense_posdef_solve", "spp_dense_panel_factor", "spp_nccl_get_unique_id", "spp_set_nccl",
     "spp_chol_symbolic", "spp_chol_solve", "spp_chol_get_factor",
@@ -111,6 +112,8 @@ def load_library() -> C.CDLL:
     lib.spp_schur_marginals.argtypes = [vp, C.c_double, dp, dp]
     lib.spp_ba_marginals_sparse.argtypes = [vp, C.c_double, dp, dp]
     lib.spp_schur_marginals_sparse.argtypes = [vp, C.c_double, dp, dp]
+    lib.spp_ba_covariance_blocks.argtypes = [vp, C.c_double, C.c_size_t, u64p, u64p, dp, C.c_size_t, u64p, dp, dp, dp]
+    lib.spp_schur_covariance_pattern.argtypes = [vp, C.c_double, dp]
     lib.spp_schur_get_reduced_system.argtypes = [vp, u64p, dp, dp, u8p]
     lib.spp_dense_posdef_solve.argtypes = [vp, C.c_size_t, dp, dp]
     lib.spp_dense_panel_factor.argtypes = [vp, C.c_size_t, C.c_size_t, dp]
@@ -261,6 +264,7 @@ class Context:
             raise SppError(rc, self.lib.spp_last_error(None).decode())
         self.h = h
         self._cb = None
+        self._schur_n_values = 0  # set by schur_symbolic; without it the library refuses schur_covariance_pattern
 
     def close(self):
         if getattr(self, "h", None):
@@ -454,6 +458,36 @@ class Context:
         self._check(self.lib.spp_ba_marginals_sparse(self.h, alpha, _dp(cc), _dp(pc)))
         return cc, pc
 
+    def ba_covariance_blocks(self, alpha: float, cam_pairs=None, observations=None, diagonal: bool = False) -> dict:
+        """Selected blocks of (lambda + alpha I)^-1 at the current states in one factorisation and inversion, on the dense
+        or the supernodal reduced camera system as schur_set_rcs_solver selects.
+          cam_pairs (n, 2): camera indices (id order among cameras) of pairs that share a landmark or are equal
+                            -> "pairs" (n, 6, 6), [k] = Cov(cam a, cam b)
+          observations (m,): edge insertion indices -> "observations" (m, 6, 3), [k] = Cov(camera, point) of that edge
+          diagonal: also "cameras" (C, 6, 6) and "points" (P, 3, 3), bit-identical to ba_marginals / ba_marginals_sparse
+        Every block is indexed [k, row, column]; the library writes them column-major (as W in ba_get_blocks)."""
+        c, p, _, _ = self._ba_dims
+        pairs = np.zeros((0, 2), np.uint64) if cam_pairs is None else np.asarray(cam_pairs)
+        obs = np.zeros(0, np.uint64) if observations is None else np.asarray(observations)
+        if pairs.ndim != 2 or pairs.shape[1] != 2:
+            raise ValueError(f"cam_pairs must be (n, 2), got {pairs.shape}")
+        if obs.ndim != 1:
+            raise ValueError(f"observations must be a vector, got {obs.shape}")
+        if (pairs.size and pairs.min() < 0) or (obs.size and obs.min() < 0):
+            raise ValueError("indices must be non-negative")
+        cam_a = np.ascontiguousarray(pairs[:, 0], np.uint64)
+        cam_b = np.ascontiguousarray(pairs[:, 1], np.uint64)
+        obs = np.ascontiguousarray(obs, np.uint64)
+        n, m = len(cam_a), len(obs)
+        pc, oc = np.empty((n, 36)), np.empty((m, 18))
+        cc, ptc = (np.empty((c, 6, 6)), np.empty((p, 3, 3))) if diagonal else (None, None)
+        self._check(self.lib.spp_ba_covariance_blocks(self.h, alpha, n, _u64p(cam_a), _u64p(cam_b), _dp(pc), m, _u64p(obs), _dp(oc),
+                                                      _dp(cc), _dp(ptc)))
+        out = dict(pairs=pc.reshape(n, 6, 6).transpose(0, 2, 1), observations=oc.reshape(m, 3, 6).transpose(0, 2, 1))
+        if diagonal:
+            out.update(cameras=cc, points=ptc)
+        return out
+
     # ---- slot 1: Schur linear solver on a caller-supplied lambda ---------------------------------
     def schur_symbolic(self, col_dims, col_ptr, row_idx):
         cd = np.ascontiguousarray(col_dims, np.uint64)
@@ -464,6 +498,8 @@ class Context:
         self._check(self.lib.spp_schur_symbolic(self.h, cd.shape[0], _u64p(cd), _u64p(cp), _u64p(ri), _u64p(order),
                                                 C.byref(cut)))
         self._schur_n = int(cd.astype(np.int64).sum())
+        dims = cd.astype(np.int64)
+        self._schur_n_values = int((dims[ri.astype(np.int64)] * np.repeat(dims, np.diff(cp.astype(np.int64)))).sum())
         self._schur_cut = (int(cut.value), int(cd.shape[0]) - int(cut.value))
         return order.astype(np.int64), int(cut.value)
 
@@ -480,6 +516,13 @@ class Context:
         cc, pc = np.empty((c, 6, 6)), np.empty((p, 3, 3))
         self._check(self.lib.spp_schur_marginals_sparse(self.h, alpha, _dp(cc), _dp(pc)))
         return cc, pc
+
+    def schur_covariance_pattern(self, alpha: float = 0.0) -> np.ndarray:
+        """(lambda + alpha I)^-1 on the block pattern of the lambda of the last schur_solve, shaped like its values (the
+        reference's block layout: column-major blocks in the order of the structure given to schur_symbolic)."""
+        out = np.empty(self._schur_n_values)
+        self._check(self.lib.spp_schur_covariance_pattern(self.h, alpha, _dp(out)))
+        return out
 
     def schur_solve(self, values, eta) -> np.ndarray:
         v = np.ascontiguousarray(values, np.float64)

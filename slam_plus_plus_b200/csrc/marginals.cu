@@ -260,6 +260,203 @@ int schur_marginals_sparse_current(spp_ctx *ctx, double alpha, double *d_cam_cov
 	return SPP_OK;
 }
 
+// ---- off-diagonal blocks ---------------------------------------------------------------------------------------
+// With Z = S^-1 and Y = W C^-1, the camera-landmark block of observation a = (c_a, p) is
+//     Sigma_{c_a p} = -sum_{b in track(p)} Z_{c_a c_b} Y_b                       (6 x 3)
+// (and Sigma_pp = C_p^-1 - sum_a Y_a^T Sigma_{c_a p}, what k_point_marginals sums). Every Z_{c_a c_b} needed is a block of
+// S, so both paths have it: the dense S^-1, or the panels after the selected inversion. So is Z_ij of any covisible pair.
+
+// thread per element: out[k * 36 + c * 6 + r] = Sigma(6 a_k + r, 6 b_k + c), column-major 6 x 6. Both accessors read a
+// diagonal block through its upper triangle (as k_camera_marginals / _panels do) and give (j, i) as the exact
+// transpose of (i, j).
+template <class Inv>
+__global__ void k_cam_pair_cov(size_t n, const uint32_t *__restrict__ cam_a, const uint32_t *__restrict__ cam_b, const Inv inv,
+	double *__restrict__ out)
+{
+	const size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x;
+	if(i >= n * 36) return;
+	const size_t k = i / 36;
+	const unsigned e = (unsigned)(i % 36), c = e / 6, r = e % 6;
+	out[i] = -inv.block(cam_a[k], cam_b[k])(r, c);
+}
+
+// CP_LANES lanes per requested observation, strided over the track of its landmark: each lane adds (-Z)_{c_a c_b} Y_b
+// to its own 6 x 3 accumulator, a fixed xor tree sums the lanes (no atomics: reproducible). k block gathers per
+// observation, sum k^2 for all of them, as in k_point_marginals. obs (n entries): edge indices mapped to track positions
+// through pos; null: the n = O observations in track order.
+#define CP_LANES 8
+#define CP_THREADS 128
+template <class Inv>
+__global__ void __launch_bounds__(CP_THREADS) k_cam_point_cov(size_t n, const uint32_t *__restrict__ obs,
+	const uint32_t *__restrict__ pos, const uint32_t *__restrict__ obs_pt, const uint32_t *__restrict__ pt_ptr,
+	const uint32_t *__restrict__ obs_cam, const double *__restrict__ Y, const Inv inv, double *__restrict__ out)
+{
+	const size_t q = (blockIdx.x * (size_t)blockDim.x + threadIdx.x) / CP_LANES;
+	const unsigned g = threadIdx.x % CP_LANES;
+	unsigned beg = 0, k = 0, ca = 0;
+	if(q < n) { // lanes past the end still take part in the shuffles
+		const uint32_t t = obs? pos[obs[q]] : (uint32_t)q;
+		const uint32_t p = obs_pt[t];
+		beg = pt_ptr[p];
+		k = pt_ptr[p + 1] - beg;
+		ca = obs_cam[t];
+	}
+	double acc[18];
+	#pragma unroll
+	for(int i = 0; i < 18; ++ i) acc[i] = 0;
+	for(unsigned b = g; b < k; b += CP_LANES) {
+		const double *Yb = Y + (size_t)(beg + b) * 18; // column-major 6 x 3
+		double yb[18];
+		#pragma unroll
+		for(int i = 0; i < 18; i += 2) {
+			double2 t = *reinterpret_cast<const double2*>(Yb + i);
+			yb[i] = t.x; yb[i + 1] = t.y;
+		}
+		const typename Inv::Block blk = inv.block(ca, obs_cam[beg + b]);
+		#pragma unroll
+		for(int j = 0; j < 6; ++ j) {
+			#pragma unroll
+			for(int i = 0; i < 6; ++ i) {
+				const double m = blk(i, j);
+				acc[i] += m * yb[j];
+				acc[6 + i] += m * yb[6 + j];
+				acc[12 + i] += m * yb[12 + j];
+			}
+		}
+	}
+	#pragma unroll
+	for(int i = 0; i < 18; ++ i) {
+		#pragma unroll
+		for(int off = CP_LANES / 2; off; off >>= 1)
+			acc[i] += __shfl_xor_sync(0xffffffffu, acc[i], off);
+	}
+	if(q < n) {
+		#pragma unroll
+		for(int i = 0; i < 18; ++ i)
+			if(i % CP_LANES == (int)g) out[q * 18 + i] = acc[i];
+	}
+}
+
+// pos[obs_orig[t]] = t: edge insertion index -> track position
+__global__ void k_invert_obs_orig(size_t O, const uint32_t *__restrict__ obs_orig, uint32_t *__restrict__ pos)
+{
+	const size_t t = blockIdx.x * (size_t)blockDim.x + threadIdx.x;
+	if(t < O) pos[obs_orig[t]] = (uint32_t)t;
+}
+
+// slot 1, the reverse of k_slot_gather: the covariance on the block pattern of lambda into the caller's value layout.
+// cam [36 C] and pt [9 P] as the marginals write them (row-major, exactly / nearly symmetric), cp [18 O] column-major
+// 6 x 3 in track order; a camera-landmark block that lambda stores 3 x 6 receives the transpose.
+__global__ void k_slot_cov_scatter(size_t C, size_t P, size_t O, const double *__restrict__ cam, const double *__restrict__ pt,
+	const double *__restrict__ cp, const uint64_t *__restrict__ u_src, const uint64_t *__restrict__ v_src,
+	const uint64_t *__restrict__ w_src, const uint8_t *__restrict__ w_tr, double *__restrict__ vals)
+{
+	size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x;
+	const size_t nU = C * 36, nV = P * 9, nW = O * 18;
+	if(i < nU) {
+		const size_t c = i / 36, e = i % 36;
+		vals[u_src[c] + e] = cam[c * 36 + (e % 6) * 6 + e / 6];
+		return;
+	}
+	i -= nU;
+	if(i < nV) {
+		const size_t p = i / 9, e = i % 9;
+		vals[v_src[p] + e] = pt[p * 9 + (e % 3) * 3 + e / 3];
+		return;
+	}
+	i -= nV;
+	if(i < nW) {
+		const size_t o = i / 18, k = i % 18, r = k % 6, c = k / 6;
+		vals[w_src[o] + (w_tr[o]? r * 3 + c : k)] = cp[i];
+	}
+}
+
+// ev[0 .. 2]: marks around the pair and the observation kernels
+template <class Inv>
+static void launch_cov_blocks(spp_ctx *ctx, const Inv &inv, size_t n_pairs, const uint32_t *d_cam_a, const uint32_t *d_cam_b,
+	double *d_pair_cov, size_t n_obs, const uint32_t *d_obs, const uint32_t *d_pos, double *d_obs_cov, cudaEvent_t *ev)
+{
+	SchurSystem &s = ctx->sys;
+	cudaStream_t st = ctx->stream;
+	SPP_CUDA(cudaEventRecord(ev[0], st));
+	if(n_pairs) {
+		k_cam_pair_cov<<<n_blocks(n_pairs * 36, 256), 256, 0, st>>>(n_pairs, d_cam_a, d_cam_b, inv, d_pair_cov);
+		LAUNCH_CHECK(ctx);
+	}
+	SPP_CUDA(cudaEventRecord(ev[1], st));
+	if(n_obs) {
+		k_cam_point_cov<<<n_blocks(n_obs * CP_LANES, CP_THREADS), CP_THREADS, 0, st>>>(n_obs, d_obs, d_pos, s.obs_pt.p(),
+			s.pt_ptr.p(), s.obs_cam.p(), s.Y.p(), inv, d_obs_cov);
+		LAUNCH_CHECK(ctx);
+	}
+	SPP_CUDA(cudaEventRecord(ev[2], st));
+}
+
+// Selected blocks of (lambda + alpha I)^-1 of the system held as (U, V, W), on the dense path (sparse == false: S^-1 in
+// full) or the supernodal one (factorisation + selected inversion, same state rules as schur_marginals_sparse_current).
+// Device arrays, each may be null with its count 0: d_cam_cov [36 C] / d_pt_cov [9 P] the block diagonal, bit-identical
+// to the marginals of that path; d_pair_cov [36 n_pairs] Sigma(cam_a[k], cam_b[k]), column-major, every pair in the block
+// pattern of S or diagonal (the caller checks); d_obs_cov [18 n_obs] Sigma(camera, point) of observation d_obs[k] (edge
+// index, mapped through obs_orig; d_obs null: every observation in track order), column-major 6 x 3.
+// ms_phases (optional, [8]): the five of schur_marginals_sparse_current (zero on the dense path, which keeps no phase
+// marks of its own), the pair kernel, the observation kernel, and the whole path before them (forming, inverse, block
+// diagonal). Returns SPP_OK / SPP_NOT_POSDEF.
+int schur_covariance_blocks_current(spp_ctx *ctx, double alpha, bool sparse, double *d_cam_cov, double *d_pt_cov, size_t n_pairs,
+	const uint32_t *d_cam_a, const uint32_t *d_cam_b, double *d_pair_cov, size_t n_obs, const uint32_t *d_obs, double *d_obs_cov,
+	float *ms_phases)
+{
+	SchurSystem &s = ctx->sys;
+	cudaStream_t st = ctx->stream;
+	cudaEvent_t *ev = ctx->ev + 6; // [3]: start; [0 .. 2]: launch_cov_blocks
+	SPP_CUDA(cudaEventRecord(ev[3], st));
+	int rc = sparse? schur_marginals_sparse_current(ctx, alpha, d_cam_cov, d_pt_cov, ms_phases) :
+		schur_marginals_current(ctx, alpha, d_cam_cov, d_pt_cov);
+	if(rc != SPP_OK)
+		return rc;
+	const uint32_t *d_pos = 0;
+	if(d_obs && n_obs) {
+		s.cov_pos.resize(s.O);
+		k_invert_obs_orig<<<n_blocks(s.O, 256), 256, 0, st>>>(s.O, ctx->ba.d_obs_orig.p(), s.cov_pos.p());
+		LAUNCH_CHECK(ctx);
+		d_pos = s.cov_pos.p();
+	}
+	if(sparse) {
+		const SupernodalChol &sc = ctx->snode;
+		const PanelInverse inv = {sc.d_L.p(), sc.d_csc_ptr.p(), sc.d_asm_dst.p(), sc.d_csc_row.p(), sc.d_csc_blk.p(), sc.d_asm_ld.p()};
+		launch_cov_blocks(ctx, inv, n_pairs, d_cam_a, d_cam_b, d_pair_cov, n_obs, d_obs, d_pos, d_obs_cov, ev);
+	} else {
+		const DenseMinusInverse inv = {s.Sinv.p(), dense_chol_ld(s.C * 6)};
+		launch_cov_blocks(ctx, inv, n_pairs, d_cam_a, d_cam_b, d_pair_cov, n_obs, d_obs, d_pos, d_obs_cov, ev);
+	}
+	if(ms_phases) {
+		SPP_CUDA(cudaEventSynchronize(ev[2]));
+		SPP_CUDA(cudaEventElapsedTime(ms_phases + 5, ev[0], ev[1]));
+		SPP_CUDA(cudaEventElapsedTime(ms_phases + 6, ev[1], ev[2]));
+		SPP_CUDA(cudaEventElapsedTime(ms_phases + 7, ev[3], ev[0]));
+	}
+	return SPP_OK;
+}
+
+// slot 1: the covariance on the block pattern of the caller's lambda, into d_vals [n_values] in its value layout;
+// ms_phases as schur_covariance_blocks_current
+int slot_covariance_pattern(spp_ctx *ctx, double alpha, bool sparse, double *d_vals, float *ms_phases)
+{
+	SchurSystem &s = ctx->sys;
+	SchurSlot &sl = ctx->slot;
+	s.cov_cam.resize(s.C * 36);
+	s.cov_pt.resize(s.P * 9);
+	s.cov_obs.resize(s.O * 18);
+	int rc = schur_covariance_blocks_current(ctx, alpha, sparse, s.cov_cam.p(), s.cov_pt.p(), 0, 0, 0, 0, s.O, 0, s.cov_obs.p(),
+		ms_phases);
+	if(rc != SPP_OK)
+		return rc;
+	const size_t total = s.C * 36 + s.P * 9 + s.O * 18;
+	k_slot_cov_scatter<<<n_blocks(total, 256), 256, 0, ctx->stream>>>(s.C, s.P, s.O, s.cov_cam.p(), s.cov_pt.p(), s.cov_obs.p(),
+		sl.u_src.p(), sl.v_src.p(), sl.w_src.p(), sl.w_transposed.p(), d_vals);
+	LAUNCH_CHECK(ctx);
+	return SPP_OK;
+}
+
 // ---- pose graphs -------------------------------------------------------------------------------------------------
 // Reference replaced: the marginals step of CNonlinearSolver_Lambda::Optimize() (NonlinearSolver_Lambda.h:669-767 ->
 // CMarginals::Calculate_DenseMarginals_Recurrent_FBS on the Cholesky factor of lambda, policy mpart_Diagonal). The pose

@@ -45,6 +45,10 @@ void dense_chol_factor_dataflow(spp_ctx *ctx, double *A, size_t ld, size_t n_col
 bool dense_chol_dataflow_enabled();
 int schur_marginals_current(spp_ctx *ctx, double alpha, double *d_cam_cov, double *d_pt_cov);
 int schur_marginals_sparse_current(spp_ctx *ctx, double alpha, double *d_cam_cov, double *d_pt_cov, float *ms_phases);
+int schur_covariance_blocks_current(spp_ctx *ctx, double alpha, bool sparse, double *d_cam_cov, double *d_pt_cov, size_t n_pairs,
+	const uint32_t *d_cam_a, const uint32_t *d_cam_b, double *d_pair_cov, size_t n_obs, const uint32_t *d_obs, double *d_obs_cov,
+	float *ms_phases);
+int slot_covariance_pattern(spp_ctx *ctx, double alpha, bool sparse, double *d_vals, float *ms_phases);
 int pose_marginals(spp_ctx *ctx, double *d_cov);
 void slot_symbolic(spp_ctx *ctx, size_t n, const uint64_t *col_dims, const uint64_t *col_ptr, const uint64_t *row_idx,
 	uint64_t *p_order, uint64_t *p_cut);
@@ -1291,6 +1295,122 @@ int spp_schur_marginals_sparse(spp_ctx_t ctx, double alpha, double *p_cam_cov, d
 	if(!ctx->slot.valid || !ctx->slot.filled) throw invalid_error("no system: spp_schur_symbolic and spp_schur_solve first");
 	rc = marginals_sparse_to_host(ctx, alpha, p_cam_cov, p_pt_cov);
 	if(rc != SPP_OK) return rc;
+	API_END(ctx)
+}
+
+// SPP_MARGINALS_TIMING: the phases of a covariance-blocks call to stderr (ms[8] as schur_covariance_blocks_current fills it)
+static void print_covariance_timing(bool sparse, const float *ms, size_t n_pairs, size_t n_obs, double ms_check, double ms_copy,
+	double copy_gb)
+{
+	if(sparse)
+		fprintf(stderr, "[spp covariance blocks] supernodal path %.3f ms: schur %.3f ms, factor %.3f ms, selected inversion %.3f ms, "
+			"cameras %.3f ms, points %.3f ms;", ms[7], ms[0], ms[1], ms[2], ms[3], ms[4]);
+	else
+		fprintf(stderr, "[spp covariance blocks] dense path %.3f ms (schur, inverse, block diagonal);", ms[7]);
+	fprintf(stderr, " pairs %.3f ms (%zu), observations %.3f ms (%zu); pattern check %.3f ms, copy to host %.3f ms (%.3f GB)\n",
+		ms[5], n_pairs, ms[6], n_obs, ms_check, ms_copy, copy_gb);
+}
+
+// selected blocks of the covariance of the system held as (U, V, W) to host arrays; the path as the solver mode selects
+static int covariance_blocks_to_host(spp_ctx *ctx, double alpha, size_t n_pairs, const uint64_t *p_cam_a, const uint64_t *p_cam_b,
+	double *p_pair_cov, size_t n_obs, const uint64_t *p_obs, double *p_obs_cov, double *p_cam_cov, double *p_pt_cov)
+{
+	SchurSystem &s = ctx->sys;
+	if(ctx->world > 1) throw invalid_error("covariance blocks are not available on a landmark-partitioned (multi-GPU) context");
+	if(!s.C) throw invalid_error("no cameras");
+	if(n_pairs && (!p_cam_a || !p_cam_b || !p_pair_cov)) throw invalid_error("camera pairs requested without their arrays");
+	if(n_obs && (!p_obs || !p_obs_cov)) throw invalid_error("observations requested without their arrays");
+	static const bool timing = getenv("SPP_MARGINALS_TIMING") != 0;
+	auto t0 = std::chrono::steady_clock::now();
+	// the sparse accessor finds a block by a binary search in the pattern of S: only covisible or equal pairs are valid
+	std::vector<uint32_t> cam_a(n_pairs), cam_b(n_pairs), obs(n_obs);
+	std::vector<uint64_t> want; // off-diagonal pairs as lo * C + hi, sorted, unique
+	for(size_t k = 0; k < n_pairs; ++ k) {
+		if(p_cam_a[k] >= s.C || p_cam_b[k] >= s.C) throw invalid_error("camera index out of range");
+		cam_a[k] = (uint32_t)p_cam_a[k];
+		cam_b[k] = (uint32_t)p_cam_b[k];
+		if(cam_a[k] != cam_b[k])
+			want.push_back((uint64_t)std::min(cam_a[k], cam_b[k]) * s.C + std::max(cam_a[k], cam_b[k]));
+	}
+	for(size_t k = 0; k < n_obs; ++ k) {
+		if(p_obs[k] >= s.O) throw invalid_error("observation index out of range");
+		obs[k] = (uint32_t)p_obs[k];
+	}
+	if(!want.empty()) {
+		std::sort(want.begin(), want.end());
+		want.erase(std::unique(want.begin(), want.end()), want.end());
+		schur_fetch_host_pattern(ctx);
+		std::vector<char> found(want.size(), 0);
+		for(size_t b = 0; b < s.n_blocks; ++ b) {
+			const uint64_t key = (uint64_t)s.h_blk_row[b] * s.C + s.h_blk_col[b]; // upper blocks: row <= col
+			auto it = std::lower_bound(want.begin(), want.end(), key);
+			if(it != want.end() && *it == key) found[it - want.begin()] = 1;
+		}
+		for(size_t i = 0; i < want.size(); ++ i)
+			if(!found[i])
+				throw invalid_error("camera pair (" + std::to_string(want[i] / s.C) + ", " + std::to_string(want[i] % s.C) +
+					") shares no landmark: its covariance block is not on the pattern of the reduced camera system");
+	}
+	const double ms_check = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+	cudaStream_t st = ctx->stream;
+	s.cov_cam_a.upload(cam_a, st);
+	s.cov_cam_b.upload(cam_b, st);
+	s.cov_obs_idx.upload(obs, st);
+	if(p_cam_cov) s.cov_cam.resize(s.C * 36);
+	if(p_pt_cov) s.cov_pt.resize(s.P * 9);
+	s.cov_pair.resize(n_pairs * 36);
+	s.cov_obs.resize(n_obs * 18);
+	const bool sparse = rcs_is_sparse(ctx, s.C);
+	float ms[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+	int rc = schur_covariance_blocks_current(ctx, alpha, sparse, p_cam_cov? s.cov_cam.p() : 0, p_pt_cov? s.cov_pt.p() : 0, n_pairs,
+		s.cov_cam_a.p(), s.cov_cam_b.p(), s.cov_pair.p(), n_obs, s.cov_obs_idx.p(), s.cov_obs.p(), timing? ms : 0);
+	if(rc != SPP_OK)
+		return rc;
+	t0 = std::chrono::steady_clock::now();
+	if(p_cam_cov) s.cov_cam.download(p_cam_cov, s.C * 36, st);
+	if(p_pt_cov) s.cov_pt.download(p_pt_cov, s.P * 9, st);
+	s.cov_pair.download(p_pair_cov, n_pairs * 36, st);
+	s.cov_obs.download(p_obs_cov, n_obs * 18, st);
+	SPP_CUDA(cudaStreamSynchronize(st));
+	if(timing)
+		print_covariance_timing(sparse, ms, n_pairs, n_obs, ms_check,
+			std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count(),
+			8e-9 * ((p_cam_cov? s.C * 36 : 0) + (p_pt_cov? s.P * 9 : 0) + n_pairs * 36 + n_obs * 18));
+	return SPP_OK;
+}
+
+int spp_ba_covariance_blocks(spp_ctx_t ctx, double alpha, size_t n_pairs, const uint64_t *p_cam_a, const uint64_t *p_cam_b,
+	double *p_pair_cov, size_t n_obs, const uint64_t *p_obs, double *p_obs_cov, double *p_cam_cov, double *p_pt_cov)
+{
+	int rc = SPP_OK;
+	API_BEGIN(ctx)
+	if(!ctx->ba.valid) throw invalid_error("no BA graph");
+	if(!ctx->ba.linearised) ba_linearise(ctx, true);
+	rc = covariance_blocks_to_host(ctx, alpha, n_pairs, p_cam_a, p_cam_b, p_pair_cov, n_obs, p_obs, p_obs_cov, p_cam_cov, p_pt_cov);
+	if(rc != SPP_OK) return rc;
+	API_END(ctx)
+}
+
+int spp_schur_covariance_pattern(spp_ctx_t ctx, double alpha, double *p_cov_values)
+{
+	int rc = SPP_OK;
+	API_BEGIN(ctx)
+	SchurSlot &sl = ctx->slot;
+	SchurSystem &s = ctx->sys;
+	if(!sl.valid || !sl.filled) throw invalid_error("no system: spp_schur_symbolic and spp_schur_solve first");
+	if(!p_cov_values) throw invalid_error("null argument");
+	if(ctx->world > 1) throw invalid_error("covariance blocks are not available on a landmark-partitioned (multi-GPU) context");
+	static const bool timing = getenv("SPP_MARGINALS_TIMING") != 0;
+	const bool sparse = rcs_is_sparse(ctx, s.C);
+	float ms[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+	rc = slot_covariance_pattern(ctx, alpha, sparse, sl.vals.p(), timing? ms : 0); // the staged lambda is not needed again
+	if(rc != SPP_OK) return rc;
+	const auto t0 = std::chrono::steady_clock::now();
+	SPP_CUDA(cudaMemcpyAsync(p_cov_values, sl.vals.p(), sl.n_values * 8, cudaMemcpyDeviceToHost, ctx->stream));
+	SPP_CUDA(cudaStreamSynchronize(ctx->stream));
+	if(timing)
+		print_covariance_timing(sparse, ms, 0, s.O, 0, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count(),
+			sl.n_values * 8e-9);
 	API_END(ctx)
 }
 

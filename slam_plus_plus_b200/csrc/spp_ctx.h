@@ -43,6 +43,8 @@ struct SchurSystem {
 	DBuf<double> S_copy; // optional copy kept for spp_schur_get_reduced_system
 	DBuf<double> Sinv; // [ld * 2 ld] marginals: [S | I] -> [-S^-1 | R^-T] (marginals.cu)
 	DBuf<double> cov_cam, cov_pt; // marginals: staging of the covariance blocks (kept: no allocation per call)
+	DBuf<double> cov_pair, cov_obs; // covariance blocks: camera pairs, camera x point of observations
+	DBuf<uint32_t> cov_cam_a, cov_cam_b, cov_obs_idx, cov_pos; // the requested pairs / observations; edge index -> track position
 	DBuf<unsigned> schur_queue; // [1] work counter of k_schur_blocks
 	DBuf<double> b, b_copy; // [n] reduced right-hand side / camera increment
 	DBuf<double> dxc, dxp; // [6C], [3P] increments
