@@ -263,6 +263,22 @@ int spp_ba_covariance_blocks(spp_ctx_t ctx, double alpha,
  * spp_ba_covariance_blocks. SPP_OK / SPP_NOT_POSDEF / SPP_ERR_INVALID. */
 int spp_schur_covariance_pattern(spp_ctx_t ctx, double alpha, double *p_cov_values);
 
+/* Joint marginal covariance of sets of vertices: for set k (vertex ids p_vertices[p_set_ptr[k] .. p_set_ptr[k+1]]),
+ * the D_k x D_k matrix Sigma_KK of (lambda + alpha I)^-1, D_k = sum of the vertices' dims (6 camera, 3 point),
+ * column-major, vertices in the order given; sets one after another in p_cov (offset sum_{j<k} D_j^2).
+ * Any vertex pair may appear, on the block pattern of the reduced camera system or off it (cameras that share no
+ * landmark, landmark-landmark blocks). Forward solves with the factor of S: Sigma_uv = [u = v landmark] C_v^-1 +
+ * F_u^T F_v, F_v = R^-T P b_v; the blocks of the reference's computeMarginals(blockIndices) style queries, which
+ * Schur_Marginals (include/slam/BAMarginals.h:579-760) does not provide. Path as spp_ba_covariance_blocks; on the
+ * supernodal path the state rules of spp_ba_marginals_sparse apply. A set's result does not depend on the other sets of
+ * the call. SPP_OK / SPP_NOT_POSDEF / SPP_ERR_INVALID (vertex id out of range, empty set, set wider than 16 384
+ * columns, several ranks). */
+int spp_ba_joint_marginals(spp_ctx_t ctx, double alpha, size_t n_sets, const uint64_t *p_set_ptr,
+	const uint64_t *p_vertices, double *p_cov);
+/* the same on the lambda of the last spp_schur_solve; sets of block columns in the numbering given to spp_schur_symbolic */
+int spp_schur_joint_marginals(spp_ctx_t ctx, double alpha, size_t n_sets, const uint64_t *p_set_ptr,
+	const uint64_t *p_block_cols, double *p_cov);
+
 /* Stage outputs of the last Schur solve, for the parity tests (SURVEY 8(c) P1): the reduced camera system as a
  * dense column-major (6C x 6C) matrix (upper triangle valid), its right-hand side, and the pattern of non-zero
  * 6x6 blocks of the upper triangle (row-major bitmap, C*C bytes). Any pointer may be NULL. */

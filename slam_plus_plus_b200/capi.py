@@ -26,7 +26,7 @@ EXPORTED_SYMBOLS = [
     "spp_synchronize", "spp_set_allreduce", "spp_partition_landmarks", "spp_rcs_block_pattern", "spp_ba_get_partition", "spp_ba_set_graph", "spp_ba_append_graph", "spp_ba_set_states", "spp_ba_get_states", "spp_ba_gather_states",
     "spp_ba_restore_initial", "spp_ba_set_jacobian_mode", "spp_ba_linearise", "spp_ba_get_lambda", "spp_ba_get_blocks", "spp_ba_chi2", "spp_ba_solve_step",
     "spp_ba_optimize", "spp_ba_marginals", "spp_schur_symbolic", "spp_schur_solve", "spp_schur_marginals",
-    "spp_ba_marginals_sparse", "spp_schur_marginals_sparse", "spp_ba_covariance_blocks", "spp_schur_covariance_pattern",
+    "spp_ba_marginals_sparse", "spp_schur_marginals_sparse", "spp_ba_covariance_blocks", "spp_schur_covariance_pattern", "spp_ba_joint_marginals", "spp_schur_joint_marginals",
     "spp_schur_get_reduced_system",
     "spp_schur_set_rcs_solver", "spp_schur_set_rcs_ordering", "spp_schur_get_rcs_info", "spp_schur_get_rcs_owners", "spp_schur_get_rcs_residual", "spp_block_ordering",
     "spp_block_symbolic_stats", "spp_block_subtree_owners", "spp_dense_posdef_solve", "spp_dense_panel_factor", "spp_nccl_get_unique_id", "spp_set_nccl",
@@ -114,6 +114,8 @@ def load_library() -> C.CDLL:
     lib.spp_schur_marginals_sparse.argtypes = [vp, C.c_double, dp, dp]
     lib.spp_ba_covariance_blocks.argtypes = [vp, C.c_double, C.c_size_t, u64p, u64p, dp, C.c_size_t, u64p, dp, dp, dp]
     lib.spp_schur_covariance_pattern.argtypes = [vp, C.c_double, dp]
+    lib.spp_ba_joint_marginals.argtypes = [vp, C.c_double, C.c_size_t, u64p, u64p, dp]
+    lib.spp_schur_joint_marginals.argtypes = [vp, C.c_double, C.c_size_t, u64p, u64p, dp]
     lib.spp_schur_get_reduced_system.argtypes = [vp, u64p, dp, dp, u8p]
     lib.spp_dense_posdef_solve.argtypes = [vp, C.c_size_t, dp, dp]
     lib.spp_dense_panel_factor.argtypes = [vp, C.c_size_t, C.c_size_t, dp]
@@ -344,6 +346,7 @@ class Context:
         if z.shape != (n_o, 2) or info.shape != (n_o, 2, 2):
             raise ValueError(f"z must be ({n_o}, 2) and info ({n_o}, 2, 2), got {z.shape} and {info.shape}")
         self._ba_dims = (int(cams.shape[0]), int(pts.shape[0]), int(op.shape[0]), int(vtype.shape[0]))
+        self._ba_vertex_dims = np.where(vtype == 0, 6, 3)
         self._check(self.lib.spp_ba_set_graph(self.h, vtype.shape[0], _u8p(vtype), _dp(cams), _dp(pts), op.shape[0],
                                               _u64p(op), _u64p(oc), _dp(z), _dp(info)))
 
@@ -367,6 +370,7 @@ class Context:
                                                  _u64p(op), _u64p(oc), _dp(z), _dp(info)))
         c0, p0, o0, v0 = self._ba_dims
         self._ba_dims = (c0 + n_c, p0 + n_p, o0 + n_o, v0 + int(vtype.shape[0]))
+        self._ba_vertex_dims = np.concatenate([self._ba_vertex_dims, np.where(vtype == 0, 6, 3)])
 
     def ba_set_states(self, cam_states=None, pts=None):
         cs = None if cam_states is None else np.ascontiguousarray(cam_states, np.float64)
@@ -488,6 +492,37 @@ class Context:
             out.update(cameras=cc, points=ptc)
         return out
 
+    def ba_joint_marginals(self, alpha: float, sets) -> list:
+        """Joint marginal covariance of sets of vertices at the current states. sets: a list of integer arrays of vertex
+        ids (cameras and points mixed, any order; pairs on or off the block pattern, e.g. cameras that share no
+        landmark). Returns a list of (D_k, D_k) arrays, D_k = 6 per camera + 3 per point, rows and columns in the order
+        of the set. Dense or supernodal reduced camera system as schur_set_rcs_solver selects."""
+        return self._joint_call(self.lib.spp_ba_joint_marginals, alpha, sets, getattr(self, "_ba_vertex_dims", None))
+
+    def schur_joint_marginals(self, alpha: float, sets) -> list:
+        """ba_joint_marginals for the lambda of the last schur_solve: sets of block columns in the numbering given to
+        schur_symbolic."""
+        return self._joint_call(self.lib.spp_schur_joint_marginals, alpha, sets, getattr(self, "_schur_col_dims", None))
+
+    def _joint_call(self, fn, alpha: float, sets, vertex_dims) -> list:
+        ids = [np.asarray(v).reshape(-1) for v in sets]
+        for v in ids:
+            if v.size and (not np.issubdtype(v.dtype, np.integer) or v.min() < 0):
+                raise ValueError("vertex ids must be non-negative integers")
+        ptr = np.zeros(len(ids) + 1, np.uint64)
+        ptr[1:] = np.cumsum([len(v) for v in ids])
+        flat = np.ascontiguousarray(np.concatenate(ids) if ids else np.zeros(0), np.uint64)
+        vd = np.zeros(0, np.int64) if vertex_dims is None else np.asarray(vertex_dims, np.int64)
+        # ids out of range count 0 here: the library refuses them before it writes anything
+        dk = np.array([int(vd[v[v < len(vd)].astype(np.int64)].sum()) for v in ids], np.int64)
+        out = np.empty(max(int((dk * dk).sum()), 1))
+        self._check(fn(self.h, alpha, len(ids), _u64p(ptr), _u64p(flat), _dp(out)))
+        res, off = [], 0
+        for D in dk:
+            res.append(out[off:off + D * D].reshape(D, D).T)  # column-major in the library
+            off += D * D
+        return res
+
     # ---- slot 1: Schur linear solver on a caller-supplied lambda ---------------------------------
     def schur_symbolic(self, col_dims, col_ptr, row_idx):
         cd = np.ascontiguousarray(col_dims, np.uint64)
@@ -501,6 +536,7 @@ class Context:
         dims = cd.astype(np.int64)
         self._schur_n_values = int((dims[ri.astype(np.int64)] * np.repeat(dims, np.diff(cp.astype(np.int64)))).sum())
         self._schur_cut = (int(cut.value), int(cd.shape[0]) - int(cut.value))
+        self._schur_col_dims = dims
         return order.astype(np.int64), int(cut.value)
 
     def schur_marginals(self, alpha: float = 0.0):

@@ -49,6 +49,8 @@ int schur_covariance_blocks_current(spp_ctx *ctx, double alpha, bool sparse, dou
 	const uint32_t *d_cam_a, const uint32_t *d_cam_b, double *d_pair_cov, size_t n_obs, const uint32_t *d_obs, double *d_obs_cov,
 	float *ms_phases);
 int slot_covariance_pattern(spp_ctx *ctx, double alpha, bool sparse, double *d_vals, float *ms_phases);
+int joint_marginals_to_host(spp_ctx *ctx, double alpha, bool sparse, const std::vector<uint64_t> &set_ptr,
+	const std::vector<uint32_t> &verts, double *p_cov, bool timing);
 int pose_marginals(spp_ctx *ctx, double *d_cov);
 void slot_symbolic(spp_ctx *ctx, size_t n, const uint64_t *col_dims, const uint64_t *col_ptr, const uint64_t *row_idx,
 	uint64_t *p_order, uint64_t *p_cut);
@@ -1411,6 +1413,79 @@ int spp_schur_covariance_pattern(spp_ctx_t ctx, double alpha, double *p_cov_valu
 	if(timing)
 		print_covariance_timing(sparse, ms, 0, s.O, 0, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count(),
 			sl.n_values * 8e-9);
+	API_END(ctx)
+}
+
+// joint marginals: sets of vertices, each already mapped to (landmark ? 1 << 31 : 0) | local index << 3; checks the sets
+// and runs on the path the solver mode selects
+static int joint_marginals_checked(spp_ctx *ctx, double alpha, size_t n_sets, const uint64_t *p_set_ptr,
+	const std::vector<uint32_t> &verts, double *p_cov)
+{
+	SchurSystem &s = ctx->sys;
+	if(ctx->world > 1) throw invalid_error("joint marginals are not available on a landmark-partitioned (multi-GPU) context");
+	if(!s.C) throw invalid_error("no cameras");
+	std::vector<uint64_t> set_ptr(p_set_ptr, p_set_ptr + n_sets + 1);
+	for(size_t k = 0; k < n_sets; ++ k) {
+		if(set_ptr[k + 1] <= set_ptr[k]) throw invalid_error("joint marginals: set " + std::to_string(k) + " is empty");
+		uint64_t D = 0;
+		for(uint64_t q = set_ptr[k]; q < set_ptr[k + 1]; ++ q) D += (verts[q] & 0x80000000u)? 3 : 6;
+		if(D > 16384) throw invalid_error("joint marginals: set " + std::to_string(k) + " is wider than 16384 columns");
+	}
+	if(!n_sets) return SPP_OK;
+	static const bool timing = getenv("SPP_MARGINALS_TIMING") != 0;
+	return joint_marginals_to_host(ctx, alpha, rcs_is_sparse(ctx, s.C), set_ptr, verts, p_cov, timing);
+}
+
+static void joint_check_args(size_t n_sets, const uint64_t *p_set_ptr, const uint64_t *p_ids, double *p_cov)
+{
+	if(n_sets && (!p_set_ptr || !p_ids || !p_cov)) throw invalid_error("null argument");
+	if(p_set_ptr && p_set_ptr[0] != 0) throw invalid_error("joint marginals: p_set_ptr[0] must be 0");
+	for(size_t k = 0; k < n_sets; ++ k)
+		if(p_set_ptr[k + 1] < p_set_ptr[k]) throw invalid_error("joint marginals: p_set_ptr must not decrease");
+}
+
+int spp_ba_joint_marginals(spp_ctx_t ctx, double alpha, size_t n_sets, const uint64_t *p_set_ptr, const uint64_t *p_vertices,
+	double *p_cov)
+{
+	int rc = SPP_OK;
+	API_BEGIN(ctx)
+	BAProblem &ba = ctx->ba;
+	if(!ba.valid) throw invalid_error("no BA graph");
+	joint_check_args(n_sets, p_set_ptr, p_vertices, p_cov);
+	const size_t n_ids = n_sets? p_set_ptr[n_sets] : 0;
+	std::vector<uint32_t> verts(n_ids);
+	for(size_t q = 0; q < n_ids; ++ q) {
+		const uint64_t v = p_vertices[q];
+		if(v >= ba.n_vertices) throw invalid_error("joint marginals: vertex id " + std::to_string(v) + " out of range");
+		verts[q] = ((ba.vtype[v] == 0)? 0u : 0x80000000u) | (ba.vertex_local[v] << 3);
+	}
+	if(ctx->world > 1) throw invalid_error("joint marginals are not available on a landmark-partitioned (multi-GPU) context");
+	if(!ba.linearised) ba_linearise(ctx, true);
+	rc = joint_marginals_checked(ctx, alpha, n_sets, p_set_ptr, verts, p_cov);
+	if(rc != SPP_OK) return rc;
+	API_END(ctx)
+}
+
+int spp_schur_joint_marginals(spp_ctx_t ctx, double alpha, size_t n_sets, const uint64_t *p_set_ptr, const uint64_t *p_block_cols,
+	double *p_cov)
+{
+	int rc = SPP_OK;
+	API_BEGIN(ctx)
+	SchurSlot &sl = ctx->slot;
+	if(!sl.valid || !sl.filled) throw invalid_error("no system: spp_schur_symbolic and spp_schur_solve first");
+	joint_check_args(n_sets, p_set_ptr, p_block_cols, p_cov);
+	std::vector<uint32_t> new_pos(sl.n_bcols);
+	for(size_t i = 0; i < sl.n_bcols; ++ i) new_pos[sl.order[i]] = (uint32_t)i;
+	const size_t n_ids = n_sets? p_set_ptr[n_sets] : 0;
+	std::vector<uint32_t> verts(n_ids);
+	for(size_t q = 0; q < n_ids; ++ q) {
+		const uint64_t b = p_block_cols[q];
+		if(b >= sl.n_bcols) throw invalid_error("joint marginals: block column " + std::to_string(b) + " out of range");
+		const uint32_t p = new_pos[b];
+		verts[q] = (p < sl.cut)? (p << 3) : (0x80000000u | ((uint32_t)(p - sl.cut) << 3));
+	}
+	rc = joint_marginals_checked(ctx, alpha, n_sets, p_set_ptr, verts, p_cov);
+	if(rc != SPP_OK) return rc;
 	API_END(ctx)
 }
 

@@ -45,6 +45,12 @@ struct SchurSystem {
 	DBuf<double> cov_cam, cov_pt; // marginals: staging of the covariance blocks (kept: no allocation per call)
 	DBuf<double> cov_pair, cov_obs; // covariance blocks: camera pairs, camera x point of observations
 	DBuf<uint32_t> cov_cam_a, cov_cam_b, cov_obs_idx, cov_pos; // the requested pairs / observations; edge index -> track position
+	// joint marginals (joint_marginals.cu), one batch at a time: compact right-hand sides / forward solves, the sets'
+	// covariances, the batch's index arrays, set dimensions, set offsets and Gram problems
+	DBuf<double> joint_F, joint_out;
+	DBuf<uint32_t> joint_idx, joint_dim;
+	DBuf<uint64_t> joint_off;
+	DBuf<uint8_t> joint_jobs;
 	DBuf<unsigned> schur_queue; // [1] work counter of k_schur_blocks
 	DBuf<double> b, b_copy; // [n] reduced right-hand side / camera increment
 	DBuf<double> dxc, dxp; // [6C], [3P] increments
