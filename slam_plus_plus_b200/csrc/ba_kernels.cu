@@ -16,10 +16,11 @@
 //     (7 x 12 doubles) -- every observation then costs ten cheap projections instead of ten pose
 //     compositions with sin/cos/atan.
 //   * k_linearise_cams: one CTA per camera, camera [R|t]s staged in shared memory, observations gathered
-//     through the camera's list; writes W and the landmark share (V_e, g_e) of every observation, accumulates U_c
-//     and g_c in registers and reduces them with a fixed-shape tree (no atomics, bit-reproducible).
-//   * k_sum_point_records: one thread per landmark walks its (contiguous) track in insertion order and adds the
-//     records up into V_p and g_p -- the same summation order as the reference's reduction plan.
+//     through the camera's list; writes W and the landmark share (V_e, g_e) of every observation through shared
+//     memory, accumulates U_c and g_c in registers and reduces them with a fixed-shape tree (no atomics,
+//     bit-reproducible).
+//   * k_sum_point_records: a warp stages the contiguous records of 32 landmarks in shared memory, and the lane of each
+//     landmark adds its track's records in insertion order into V_p and g_p -- the reference's reduction plan's order.
 
 #include "spp_ctx.h"
 #include <stdlib.h>
@@ -181,6 +182,40 @@ __device__ __forceinline__ void dmma884(double &d0, double &d1, double a, double
 		: "+d"(d0), "+d"(d1) : "d"(a), "d"(b));
 }
 
+// W = T Jp (6x3, column-major) and the landmark's share of the observation, V_e = upper(Jp^T Sigma^-1 Jp) and
+// g_e = Jp^T (Sigma^-1 r) (record of 10 doubles, the last one padding): the Jacobian is at hand here, so the landmark
+// kernel only has to add these records up along its track (same expressions and the same summation order as the
+// landmark kernel that recomputed Jp: bit-identical V, gp)
+__device__ __forceinline__ void observation_outputs(const double *T0, const double *T1, const double *Jp, double2 i01,
+	double2 i23, double ru, double rv, double *Wo, double *rec, double &dmax)
+{
+	#pragma unroll
+	for(int cc = 0; cc < 3; ++ cc) {
+		double w[6];
+		#pragma unroll
+		for(int j = 0; j < 6; ++ j)
+			w[j] = T0[j] * Jp[cc] + T1[j] * Jp[3 + cc];
+		*reinterpret_cast<double2*>(Wo + cc * 6 + 0) = make_double2(w[0], w[1]);
+		*reinterpret_cast<double2*>(Wo + cc * 6 + 2) = make_double2(w[2], w[3]);
+		*reinterpret_cast<double2*>(Wo + cc * 6 + 4) = make_double2(w[4], w[5]);
+	}
+	double A0[3], A1[3];
+	#pragma unroll
+	for(int j = 0; j < 3; ++ j) {
+		A0[j] = Jp[j] * i01.x + Jp[3 + j] * i23.x;
+		A1[j] = Jp[j] * i01.y + Jp[3 + j] * i23.y;
+	}
+	const double e00 = A0[0] * Jp[0] + A1[0] * Jp[3], e01 = A0[0] * Jp[1] + A1[0] * Jp[4], e02 = A0[0] * Jp[2] + A1[0] * Jp[5];
+	const double e11 = A0[1] * Jp[1] + A1[1] * Jp[4], e12 = A0[1] * Jp[2] + A1[1] * Jp[5], e22 = A0[2] * Jp[2] + A1[2] * Jp[5];
+	const double s0 = i01.x * ru + i01.y * rv, s1 = i23.x * ru + i23.y * rv;
+	*reinterpret_cast<double2*>(rec + 0) = make_double2(e00, e01);
+	*reinterpret_cast<double2*>(rec + 2) = make_double2(e02, e11);
+	*reinterpret_cast<double2*>(rec + 4) = make_double2(e12, e22);
+	*reinterpret_cast<double2*>(rec + 6) = make_double2(Jp[0] * s0 + Jp[3] * s1, Jp[1] * s0 + Jp[4] * s1);
+	*reinterpret_cast<double2*>(rec + 8) = make_double2(Jp[2] * s0 + Jp[5] * s1, 0.0);
+	dmax = fmax(dmax, fmax(e00, fmax(e11, e22)));
+}
+
 static const size_t CAM_SMEM = (size_t)(CAM_THREADS / 32) * 2 * 8 * GR_LD * sizeof(double);
 
 // one CTA per camera. JAC: Jacobian mode as a compile-time constant (the other branch does not cost registers).
@@ -192,6 +227,9 @@ static const size_t CAM_SMEM = (size_t)(CAM_THREADS / 32) * 2 * 8 * GR_LD * size
 // profiles/r1k_full.csv). The expressions of the products are the reference's (U_e = T Jc, g = T r,
 // BaseTypes_Binary.h:813-843); the summation order is fixed (k ascending inside the warp, then the warps in order), so
 // the result is bit-reproducible.
+// After the products the warp's tile is free: W and the landmark records of its 32 observations are staged there and
+// stored as consecutive 16-byte pieces (Venice shape: 519 -> 352 us; DESIGN.md §4), and the indices of the next trip are
+// fetched one trip ahead (352 -> 348 us).
 // (Measured alternatives of round 1: ten lanes per observation -- one projection per lane, the Hessian algebra spread
 // over the lanes through shared memory -- 0.97 ms against 0.81 ms.)
 template <int JAC>
@@ -213,26 +251,33 @@ __global__ void __launch_bounds__(CAM_THREADS, CAM_MIN_CTAS) k_linearise_cams(in
 		sRt[i] = camRt[(size_t)c * 84 + i];
 	if(threadIdx.x < 5)
 		sK[threadIdx.x] = camK[(size_t)c * 5 + threadIdx.x];
-	for(int i = lane; i < 2 * 8 * GR_LD; i += 32) // rows 6, 7 of T and row 7 of [Jc | r] stay zero
-		sT[i] = 0;
 	__syncthreads();
 
 	double acc0 = 0, acc1 = 0, dmax = 0; // [U | g](g, 2 t), (g, 2 t + 1)
 	const unsigned beg = cam_ptr[c], end = cam_ptr[c + 1];
+	unsigned o_nx = 0, p_nx = 0;
+	if(beg + threadIdx.x < end) {
+		o_nx = cam_obs[beg + threadIdx.x];
+		p_nx = obs_pt[o_nx];
+	}
 	for(unsigned base = beg; base < end; base += CAM_THREADS) {
 		const unsigned idx = base + threadIdx.x;
 		double2 *pT = reinterpret_cast<double2*>(sT + 2 * lane), *pJ = reinterpret_cast<double2*>(sJ + 2 * lane);
+		double T0[6], T1[6], Jp[6], ru, rv;
+		double2 i01, i23;
+		const unsigned o = o_nx, p = p_nx;
+		if(idx + CAM_THREADS < end) // next trip's indices: its dependent chain becomes one memory round trip
+			o_nx = cam_obs[idx + CAM_THREADS];
 		if(idx < end) {
-			const unsigned o = cam_obs[idx];
-			const unsigned p = obs_pt[o];
 			const double X = pts[(size_t)p * 3], Y = pts[(size_t)p * 3 + 1], Z = pts[(size_t)p * 3 + 2];
 			const double2 zz = *reinterpret_cast<const double2*>(z + (size_t)o * 2);
-			const double2 i01 = *reinterpret_cast<const double2*>(info + (size_t)o * 4);
-			const double2 i23 = *reinterpret_cast<const double2*>(info + (size_t)o * 4 + 2);
-			double Jc[12], Jp[6], ru, rv;
+			i01 = *reinterpret_cast<const double2*>(info + (size_t)o * 4);
+			i23 = *reinterpret_cast<const double2*>(info + (size_t)o * 4 + 2);
+			if(idx + CAM_THREADS < end)
+				p_nx = obs_pt[o_nx];
+			double Jc[12];
 			observation_jacobians(JAC, sRt, sK, X, Y, Z, zz.x, zz.y, Jc, Jp, ru, rv, true, true);
 			// T = Jc^T Sigma^-1 (6x2): T(j,0) = Jc(0,j) s00 + Jc(1,j) s10 ; T(j,1) = Jc(0,j) s01 + Jc(1,j) s11
-			double T0[6], T1[6];
 			#pragma unroll
 			for(int j = 0; j < 6; ++ j) {
 				T0[j] = Jc[j] * i01.x + Jc[6 + j] * i23.x;
@@ -246,39 +291,6 @@ __global__ void __launch_bounds__(CAM_THREADS, CAM_MIN_CTAS) k_linearise_cams(in
 				dmax = fmax(dmax, T0[j] * Jc[j] + T1[j] * Jc[6 + j]); // the diagonal of U_e (initial damping, LM.h:162-166)
 			}
 			pJ[6 * (GR_LD / 2)] = make_double2(ru, rv);
-			// W = T Jp (6x3), column-major
-			double *Wo = W + (size_t)o * 18;
-			#pragma unroll
-			for(int cc = 0; cc < 3; ++ cc) {
-				double w[6];
-				#pragma unroll
-				for(int j = 0; j < 6; ++ j)
-					w[j] = T0[j] * Jp[cc] + T1[j] * Jp[3 + cc];
-				*reinterpret_cast<double2*>(Wo + cc * 6 + 0) = make_double2(w[0], w[1]);
-				*reinterpret_cast<double2*>(Wo + cc * 6 + 2) = make_double2(w[2], w[3]);
-				*reinterpret_cast<double2*>(Wo + cc * 6 + 4) = make_double2(w[4], w[5]);
-			}
-			// the landmark's share of this observation, V_e = upper(Jp^T Sigma^-1 Jp) and g_e = Jp^T (Sigma^-1 r): the Jacobian
-			// is at hand here, so the landmark kernel only has to add these records up along its track (same expressions and
-			// the same summation order as the landmark kernel that recomputed Jp: bit-identical V, gp)
-			{
-				double A0[3], A1[3];
-				#pragma unroll
-				for(int j = 0; j < 3; ++ j) {
-					A0[j] = Jp[j] * i01.x + Jp[3 + j] * i23.x;
-					A1[j] = Jp[j] * i01.y + Jp[3 + j] * i23.y;
-				}
-				const double e00 = A0[0] * Jp[0] + A1[0] * Jp[3], e01 = A0[0] * Jp[1] + A1[0] * Jp[4], e02 = A0[0] * Jp[2] + A1[0] * Jp[5];
-				const double e11 = A0[1] * Jp[1] + A1[1] * Jp[4], e12 = A0[1] * Jp[2] + A1[1] * Jp[5], e22 = A0[2] * Jp[2] + A1[2] * Jp[5];
-				const double s0 = i01.x * ru + i01.y * rv, s1 = i23.x * ru + i23.y * rv;
-				double *rec = PtRec + (size_t)o * 10;
-				*reinterpret_cast<double2*>(rec + 0) = make_double2(e00, e01);
-				*reinterpret_cast<double2*>(rec + 2) = make_double2(e02, e11);
-				*reinterpret_cast<double2*>(rec + 4) = make_double2(e12, e22);
-				*reinterpret_cast<double2*>(rec + 6) = make_double2(Jp[0] * s0 + Jp[3] * s1, Jp[1] * s0 + Jp[4] * s1);
-				*reinterpret_cast<double2*>(rec + 8) = make_double2(Jp[2] * s0 + Jp[5] * s1, 0.0);
-				dmax = fmax(dmax, fmax(e00, fmax(e11, e22)));
-			}
 		} else {
 			#pragma unroll
 			for(int j = 0; j < 6; ++ j) {
@@ -288,10 +300,33 @@ __global__ void __launch_bounds__(CAM_THREADS, CAM_MIN_CTAS) k_linearise_cams(in
 			pJ[6 * (GR_LD / 2)] = make_double2(0.0, 0.0);
 		}
 		__syncwarp();
-		// [U | g] += T [Jc | r]: A(m, k) = T(m, k), B(k, n) = [Jc | r](k, n), k = 0 .. 63
+		// [U | g] += T [Jc | r]: A(m, k) = T(m, k), B(k, n) = [Jc | r](k, n), k = 0 .. 63; rows 6, 7 of A and column 7 of B
+		// are zero (the tile holds other data between the products)
 		#pragma unroll 4
 		for(int k4 = 0; k4 < 64; k4 += 4)
-			dmma884(acc0, acc1, sT[g * GR_LD + k4 + t], sJ[g * GR_LD + k4 + t]);
+			dmma884(acc0, acc1, (g < 6)? sT[g * GR_LD + k4 + t] : 0.0, (g < 7)? sJ[g * GR_LD + k4 + t] : 0.0);
+		__syncwarp();
+		// W and the landmark record of the warp's 32 observations go through the tile: consecutive lanes then store
+		// consecutive 16-byte pieces of one observation's block instead of 32 scattered pieces per instruction
+		double *sW = sT, *sR = sT + 32 * 18;
+		if(idx < end)
+			observation_outputs(T0, T1, Jp, i01, i23, ru, rv, sW + lane * 18, sR + lane * 10, dmax);
+		__syncwarp();
+		const unsigned n_valid = (end - base > (unsigned)warp * 32)? end - base - (unsigned)warp * 32 : 0;
+		#pragma unroll
+		for(int k = 0; k < 9; ++ k) { // 32 x 9 pieces of W
+			const unsigned q = k * 32 + lane, ob = q / 9;
+			const unsigned oq = __shfl_sync(0xffffffffu, o, ob);
+			if(ob < n_valid)
+				reinterpret_cast<double2*>(W + (size_t)oq * 18)[q - ob * 9] = reinterpret_cast<const double2*>(sW)[q];
+		}
+		#pragma unroll
+		for(int k = 0; k < 5; ++ k) { // 32 x 5 pieces of the landmark records
+			const unsigned q = k * 32 + lane, ob = q / 5;
+			const unsigned oq = __shfl_sync(0xffffffffu, o, ob);
+			if(ob < n_valid)
+				reinterpret_cast<double2*>(PtRec + (size_t)oq * 10)[q - ob * 5] = reinterpret_cast<const double2*>(sR)[q];
+		}
 		__syncwarp();
 	}
 
@@ -326,29 +361,61 @@ __global__ void __launch_bounds__(CAM_THREADS, CAM_MIN_CTAS) k_linearise_cams(in
 		atomicMax(maxdiag, (unsigned long long)__double_as_longlong(sred[0][64]));
 }
 
-// thread per landmark: V_p, g_p = sum of the per-observation records written by k_linearise_cams, along the track in
-// edge insertion order (the reference's summation order, NonlinearSolver_Lambda_Base.h:152-197, 563-607)
-__global__ void k_sum_point_records(size_t P, const uint32_t *__restrict__ pt_ptr, const double *__restrict__ PtRec,
-	double *__restrict__ V, double *__restrict__ gp, long uf_pt)
+// warp per 32 consecutive landmarks: V_p, g_p = sum of the per-observation records written by k_linearise_cams. The
+// records of the warp's 32 tracks are one contiguous range; the warp stages it chunk by chunk in shared memory with
+// coalesced 16-byte loads, and the owning lane adds its landmark's records in edge insertion order (the reference's
+// summation order, NonlinearSolver_Lambda_Base.h:152-197, 563-607). V and g_p leave through shared memory as the
+// warp's contiguous 32 x 9 and 32 x 3 ranges.
+#define SR_WARPS 4
+#define SR_CHUNK 64 // records per chunk: 320 double2, ten loads per lane in flight
+
+__global__ void __launch_bounds__(SR_WARPS * 32) k_sum_point_records(size_t P, const uint32_t *__restrict__ pt_ptr,
+	const double *__restrict__ PtRec, double *__restrict__ V, double *__restrict__ gp, long uf_pt)
 {
-	size_t p = blockIdx.x * (size_t)blockDim.x + threadIdx.x;
-	if(p >= P) return;
+	__shared__ double2 sRec[SR_WARPS][SR_CHUNK * 5];
+	const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+	const size_t p0 = (blockIdx.x * (size_t)SR_WARPS + warp) * 32;
+	if(p0 >= P) return;
+	const unsigned np = (unsigned)((P - p0 < 32)? P - p0 : 32);
+	const unsigned wbeg = pt_ptr[p0], wend = pt_ptr[p0 + np];
+	const unsigned beg = ((unsigned)lane < np)? pt_ptr[p0 + lane] : wend, end = ((unsigned)lane < np)? pt_ptr[p0 + lane + 1] : wend;
+	double2 *s = sRec[warp];
+	const double2 *src = reinterpret_cast<const double2*>(PtRec);
 	double v00 = 0, v01 = 0, v02 = 0, v11 = 0, v12 = 0, v22 = 0, g0 = 0, g1 = 0, g2 = 0;
-	const unsigned beg = pt_ptr[p], end = pt_ptr[p + 1];
-	for(unsigned o = beg; o < end; ++ o) {
-		const double2 *rec = reinterpret_cast<const double2*>(PtRec + (size_t)o * 10);
-		const double2 a = rec[0], b = rec[1], c = rec[2], d = rec[3], e = rec[4];
-		v00 += a.x; v01 += a.y; v02 += b.x; v11 += b.y; v12 += c.x; v22 += c.y;
-		g0 += d.x; g1 += d.y; g2 += e.x;
+	for(unsigned b = wbeg; b < wend; b += SR_CHUNK) {
+		const unsigned n5 = ((wend - b < SR_CHUNK)? wend - b : SR_CHUNK) * 5;
+		#pragma unroll
+		for(unsigned k = 0; k < SR_CHUNK * 5 / 32; ++ k) {
+			const unsigned i = k * 32 + lane;
+			if(i < n5)
+				s[i] = src[(size_t)b * 5 + i];
+		}
+		__syncwarp();
+		const unsigned lo = (beg > b)? beg : b, hi = (end < b + SR_CHUNK)? end : b + SR_CHUNK;
+		for(unsigned o = lo; o < hi; ++ o) {
+			const double2 *rec = s + (o - b) * 5;
+			const double2 ra = rec[0], rb = rec[1], rc = rec[2], rd = rec[3], re = rec[4];
+			v00 += ra.x; v01 += ra.y; v02 += rb.x; v11 += rb.y; v12 += rc.x; v22 += rc.y;
+			g0 += rd.x; g1 += rd.y; g2 += re.x;
+		}
+		__syncwarp();
 	}
-	if((long)p == uf_pt) {
+	if(p0 + lane == (size_t)uf_pt) {
 		v00 += 1.0; v11 += 1.0; v22 += 1.0;
 	}
-	double *Vp = V + p * 9;
-	Vp[0] = v00; Vp[1] = v01; Vp[2] = v02;
-	Vp[3] = v01; Vp[4] = v11; Vp[5] = v12;
-	Vp[6] = v02; Vp[7] = v12; Vp[8] = v22;
-	gp[p * 3] = g0; gp[p * 3 + 1] = g1; gp[p * 3 + 2] = g2;
+	double *sv = reinterpret_cast<double*>(s), *sg = sv + 32 * 9;
+	if((unsigned)lane < np) {
+		double *Vp = sv + lane * 9;
+		Vp[0] = v00; Vp[1] = v01; Vp[2] = v02;
+		Vp[3] = v01; Vp[4] = v11; Vp[5] = v12;
+		Vp[6] = v02; Vp[7] = v12; Vp[8] = v22;
+		sg[lane * 3] = g0; sg[lane * 3 + 1] = g1; sg[lane * 3 + 2] = g2;
+	}
+	__syncwarp();
+	for(unsigned i = lane; i < np * 9; i += 32)
+		V[p0 * 9 + i] = sv[i];
+	for(unsigned i = lane; i < np * 3; i += 32)
+		gp[p0 * 3 + i] = sg[i];
 }
 
 // chi2: thread per observation, block partials, then a fixed-order final pass
@@ -493,7 +560,7 @@ void ba_linearise(spp_ctx *ctx, bool b_want_maxdiag)
 		LAUNCH_CHECK(ctx);
 	}
 	if(s.P) {
-		k_sum_point_records<<<n_blocks(s.P, 128), 128, 0, ctx->stream>>>(s.P, s.pt_ptr.p(), ba.pt_rec.p(), s.V.p(), s.gp.p(),
+		k_sum_point_records<<<n_blocks(s.P, SR_WARPS * 32), SR_WARPS * 32, 0, ctx->stream>>>(s.P, s.pt_ptr.p(), ba.pt_rec.p(), s.V.p(), s.gp.p(),
 			ba.uf_is_cam? -1 : ba.uf_index);
 		LAUNCH_CHECK(ctx);
 	}

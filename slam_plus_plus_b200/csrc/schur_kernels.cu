@@ -26,21 +26,27 @@ size_t dense_chol_storage(size_t n);
 #define LAUNCH_CHECK(ctx) do { ++ (ctx)->n_launches; SPP_CUDA(cudaGetLastError()); } while(0)
 
 // warp per 32 consecutive landmarks: lane l inverts landmark p0 + l, Cinv = (V + alpha I)^-1 by cofactors (what
-// Eigen's fixed 3x3 inverse() does, BlockMatrixBase.h:1256-1270); then the warp walks the CONTIGUOUS W range of its
-// 32 tracks element by element (coalesced) and writes Y_o = W_o Cinv.
+// Eigen's fixed 3x3 inverse() does, BlockMatrixBase.h:1256-1270); V is read and Cinv written as the warp's contiguous
+// 32 x 9 range through shared memory. Then the warp walks the CONTIGUOUS W range of its 32 tracks in 16-byte units
+// (coalesced loads, one double2 store of Y_o = W_o Cinv per unit). A lane's position (o, unit j of 9) advances by 32
+// units = 3 observations + 5 units per step, so there is no division; obs_pt[o] names the unit's landmark.
 #define LI_WARPS 8
 
 __global__ void __launch_bounds__(LI_WARPS * 32) k_landmark_inverse(size_t P, double alpha, const uint32_t *__restrict__ pt_ptr,
-	const double *__restrict__ V, const double *__restrict__ W, double *__restrict__ Cinv, double *__restrict__ Y)
+	const uint32_t *__restrict__ obs_pt, const double *__restrict__ V, const double *__restrict__ W, double *__restrict__ Cinv,
+	double *__restrict__ Y)
 {
-	__shared__ double sC[LI_WARPS][32][9];
-	__shared__ unsigned sPtr[LI_WARPS][33];
+	__shared__ double sC[LI_WARPS][32 * 9];
 	const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 	const size_t p0 = (blockIdx.x * (size_t)LI_WARPS + warp) * 32;
 	if(p0 >= P) return;
-	const size_t p = p0 + lane;
-	if(p < P) {
-		const double *Vp = V + p * 9; // column-major
+	const unsigned np = (unsigned)((P - p0 < 32)? P - p0 : 32);
+	double *sc = sC[warp];
+	for(unsigned i = lane; i < np * 9; i += 32)
+		sc[i] = V[p0 * 9 + i];
+	__syncwarp();
+	if((unsigned)lane < np) {
+		double *Vp = sc + lane * 9; // column-major; overwritten by this lane's inverse
 		double m00 = Vp[0] + alpha, m10 = Vp[1], m20 = Vp[2];
 		double m01 = Vp[3], m11 = Vp[4] + alpha, m21 = Vp[5];
 		double m02 = Vp[6], m12 = Vp[7], m22 = Vp[8] + alpha;
@@ -52,26 +58,25 @@ __global__ void __launch_bounds__(LI_WARPS * 32) k_landmark_inverse(size_t P, do
 		inv[0] = c00 * id; inv[3] = c10 * id; inv[6] = c20 * id;
 		inv[1] = (m12 * m20 - m10 * m22) * id; inv[4] = (m22 * m00 - m20 * m02) * id; inv[7] = (m02 * m10 - m00 * m12) * id;
 		inv[2] = (m10 * m21 - m11 * m20) * id; inv[5] = (m20 * m01 - m21 * m00) * id; inv[8] = (m00 * m11 - m01 * m10) * id;
-		double *Ci = Cinv + p * 9;
 		#pragma unroll
-		for(int i = 0; i < 9; ++ i) {
-			Ci[i] = inv[i];
-			sC[warp][lane][i] = inv[i];
-		}
+		for(int i = 0; i < 9; ++ i)
+			Vp[i] = inv[i];
 	}
-	sPtr[warp][lane] = pt_ptr[(p < P)? p : P];
-	if(lane == 0)
-		sPtr[warp][32] = pt_ptr[(p0 + 32 < P)? p0 + 32 : P];
 	__syncwarp();
-	const size_t e_end = (size_t)sPtr[warp][32] * 18;
-	int pl = 0; // landmark (relative to p0) of the current observation; e grows monotonically per lane
-	for(size_t e = (size_t)sPtr[warp][0] * 18 + lane; e < e_end; e += 32) {
-		const unsigned o = (unsigned)(e / 18), q = (unsigned)(e - (size_t)o * 18);
-		const unsigned c = q / 6, r = q - c * 6;
-		while(sPtr[warp][pl + 1] <= o)
-			++ pl;
-		const double *Wo = W + (size_t)o * 18, *Ci = sC[warp][pl];
-		Y[e] = Wo[r] * Ci[c * 3] + Wo[6 + r] * Ci[c * 3 + 1] + Wo[12 + r] * Ci[c * 3 + 2];
+	for(unsigned i = lane; i < np * 9; i += 32)
+		Cinv[p0 * 9 + i] = sc[i];
+	// unit j of a 6 x 3 column-major block holds rows r, r + 1 (r = 2 (j mod 3)) of column c = j / 3
+	const unsigned o_end = pt_ptr[p0 + np];
+	unsigned o = pt_ptr[p0] + lane / 9, j = lane % 9;
+	while(o < o_end) {
+		const unsigned c = j / 3, r = 2 * (j - 3 * c);
+		const double *Ci = sc + (obs_pt[o] - (unsigned)p0) * 9 + c * 3;
+		const double2 *Wo = reinterpret_cast<const double2*>(W + (size_t)o * 18 + r);
+		const double2 w0 = Wo[0], w1 = Wo[3], w2 = Wo[6];
+		*reinterpret_cast<double2*>(Y + (size_t)o * 18 + 2 * j) = make_double2(w0.x * Ci[0] + w1.x * Ci[1] + w2.x * Ci[2],
+			w0.y * Ci[0] + w1.y * Ci[1] + w2.y * Ci[2]);
+		o += 3; j += 5;
+		if(j >= 9) { j -= 9; ++ o; }
 	}
 }
 
@@ -469,8 +474,8 @@ void schur_form_reduced_system(spp_ctx *ctx, double alpha, double alpha_diag, bo
 	double *S_out = sparse_rcs? s.Sblk.p() : s.S.p();
 	s.b.resize(n);
 	if(s.P) {
-		k_landmark_inverse<<<n_blocks(s.P, LI_WARPS * 32), LI_WARPS * 32, 0, ctx->stream>>>(s.P, alpha, s.pt_ptr.p(), s.V.p(),
-			s.W.p(), s.Cinv.p(), s.Y.p());
+		k_landmark_inverse<<<n_blocks(s.P, LI_WARPS * 32), LI_WARPS * 32, 0, ctx->stream>>>(s.P, alpha, s.pt_ptr.p(), s.obs_pt.p(),
+			s.V.p(), s.W.p(), s.Cinv.p(), s.Y.p());
 		LAUNCH_CHECK(ctx);
 	}
 	if(!sparse_rcs)
