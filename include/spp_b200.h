@@ -172,6 +172,35 @@ int spp_ba_restore_initial(spp_ctx_t ctx);
 
 int spp_ba_set_jacobian_mode(spp_ctx_t ctx, int mode); /* SPP_JAC_* ; default SPP_JAC_FD_REFERENCE */
 
+/* Robust loss of the BA observations (g2o-style IRLS; the reference's kernels: RobustUtils.h:368-586). With s2 = r^T
+ * Omega r the squared Mahalanobis error of an observation (r = z - h; s is in pixels when Omega = I) and k the scale:
+ *   SPP_LOSS_NONE    rho = s2                                      w = 1
+ *   SPP_LOSS_HUBER   rho = s2 if s2 <= k^2, else 2 k sqrt(s2) - k^2 w = 1 if s2 <= k^2, else k / sqrt(s2)
+ *   SPP_LOSS_CAUCHY  rho = k^2 log1p(s2 / k^2)                      w = 1 / (1 + s2 / k^2)
+ * The linearisation replaces Omega by w Omega before any other use, so U, g_c, W, V, g_p and the initial damping are
+ * those of the weighted problem -- and so are spp_ba_get_lambda, spp_ba_get_blocks, spp_ba_solve_step and every
+ * marginal / covariance entry point (the convention of Ceres and g2o for the covariance of a robust problem). Both
+ * vertices of an observation see the same weight: this is NOT the reference's robust binary edge, which weights vertex
+ * 0's gradient by w^2 and vertex 1's by w (BaseTypes_Binary.h:820-843). spp_ba_chi2, chi2_initial / chi2_final /
+ * trace_chi2 of spp_report_t and the LM acceptance test then hold sum rho; the predicted decrease stays
+ * dx^T (alpha dx + eta) (the IRLS model). An observation with w = 1 contributes exactly what it does without a loss. */
+#define SPP_LOSS_NONE 0   /* default */
+#define SPP_LOSS_HUBER 1
+#define SPP_LOSS_CAUCHY 2
+
+/* Context state, like the Jacobian mode: kept across spp_ba_set_graph, spp_ba_append_graph and spp_ba_restore_initial;
+ * marks the linearisation stale. scale (k, in units of s) must be finite and > 0 for HUBER and CAUCHY and is ignored for
+ * NONE. An unknown kind or a bad scale returns SPP_ERR_INVALID and keeps the previous setting. No reference counterpart
+ * for BA (the reference sets a robust kernel per edge type at compile time). */
+int spp_ba_set_robust_loss(spp_ctx_t ctx, int kind, double scale);
+
+/* s2 (p_sq_error[O]) and the weight w = rho'(s2) (p_weight[O]) of every observation at the current states, in EDGE
+ * INSERTION order (as W of spp_ba_get_blocks). The residual is computed as the linearisation in the current Jacobian mode
+ * computes it, so w is bit for bit the weight a linearisation at these states uses. Either pointer may be NULL. Lets a
+ * caller find and drop outliers between two optimisations. Refused on a landmark-partitioned (multi-GPU) context. No
+ * reference counterpart. */
+int spp_ba_get_observation_errors(spp_ctx_t ctx, double *p_sq_error, double *p_weight);
+
 /* Replaces CLambdaOps2::Refresh_Lambda + Collect_RightHandSide_Vector (Lambda_Base.h:1659-1706):
  * per-edge Jacobians (CEdgeP2C3D::Calculate_Jacobians_Expectation_Error, BA_Types.h:494-505), Hessian blocks
  * (CBaseEdgeImpl::Calculate_Hessians_v2, BaseTypes_Binary.h:759-848) and their reduction into lambda / eta. */
@@ -190,7 +219,7 @@ int spp_ba_get_lambda(spp_ctx_t ctx, uint64_t *p_n_block_cols, uint64_t *p_n_blo
 int spp_ba_get_blocks(spp_ctx_t ctx, double *p_U, double *p_V, double *p_W, double *p_eta_c, double *p_eta_p);
 
 /* Replaces CNonlinearSolver_Lambda_LM::f_Chi_Squared_Error_Denorm (NonlinearSolver_Base.h:278-297 ->
- * CEdgeP2C3D::f_Chi_Squared_Error, BA_Types.h:511-531). */
+ * CEdgeP2C3D::f_Chi_Squared_Error, BA_Types.h:511-531). Under a robust loss (spp_ba_set_robust_loss): sum rho(s2). */
 int spp_ba_chi2(spp_ctx_t ctx, double *p_chi2);
 
 /* One damped Newton step on the current linearisation: solves (lambda + alpha I) dx = eta through the landmark

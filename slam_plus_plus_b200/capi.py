@@ -17,6 +17,7 @@ LIB_PATH = os.path.join(_HERE, "libspp_b200.so")
 SPP_OK, SPP_NOT_POSDEF = 0, 1
 SPP_ERR_INVALID, SPP_ERR_CUDA, SPP_ERR_NOMEM, SPP_ERR_COMM = -1, -2, -3, -4
 JAC_FD_REFERENCE, JAC_ANALYTIC = 0, 1
+LOSS_NONE, LOSS_HUBER, LOSS_CAUCHY = 0, 1, 2
 RCS_AUTO, RCS_DENSE, RCS_SPARSE = 0, 1, 2
 MAX_TRACE = 64
 
@@ -24,7 +25,7 @@ MAX_TRACE = 64
 EXPORTED_SYMBOLS = [
     "spp_create", "spp_destroy", "spp_last_error", "spp_describe", "spp_kernel_launches", "spp_stream",
     "spp_synchronize", "spp_set_allreduce", "spp_partition_landmarks", "spp_rcs_block_pattern", "spp_ba_get_partition", "spp_ba_set_graph", "spp_ba_append_graph", "spp_ba_set_states", "spp_ba_get_states", "spp_ba_gather_states",
-    "spp_ba_restore_initial", "spp_ba_set_jacobian_mode", "spp_ba_linearise", "spp_ba_get_lambda", "spp_ba_get_blocks", "spp_ba_chi2", "spp_ba_solve_step",
+    "spp_ba_restore_initial", "spp_ba_set_jacobian_mode", "spp_ba_set_robust_loss", "spp_ba_get_observation_errors", "spp_ba_linearise", "spp_ba_get_lambda", "spp_ba_get_blocks", "spp_ba_chi2", "spp_ba_solve_step",
     "spp_ba_optimize", "spp_ba_marginals", "spp_schur_symbolic", "spp_schur_solve", "spp_schur_marginals",
     "spp_ba_marginals_sparse", "spp_schur_marginals_sparse", "spp_ba_covariance_blocks", "spp_schur_covariance_pattern", "spp_ba_joint_marginals", "spp_schur_joint_marginals",
     "spp_schur_get_reduced_system",
@@ -100,6 +101,8 @@ def load_library() -> C.CDLL:
     lib.spp_ba_get_states.argtypes = [vp, dp, dp]
     lib.spp_ba_restore_initial.argtypes = [vp]
     lib.spp_ba_set_jacobian_mode.argtypes = [vp, C.c_int]
+    lib.spp_ba_set_robust_loss.argtypes = [vp, C.c_int, C.c_double]
+    lib.spp_ba_get_observation_errors.argtypes = [vp, dp, dp]
     lib.spp_ba_linearise.argtypes = [vp]
     lib.spp_ba_get_lambda.argtypes = [vp, u64p, u64p, u64p, u64p, u64p, u64p, dp, dp]
     lib.spp_ba_get_blocks.argtypes = [vp, dp, dp, dp, dp, dp]
@@ -407,6 +410,20 @@ class Context:
 
     def ba_set_jacobian_mode(self, mode: int):
         self._check(self.lib.spp_ba_set_jacobian_mode(self.h, mode))
+
+    def ba_set_robust_loss(self, kind: int, scale: float = 1.0):
+        """Robust loss of every BA observation: LOSS_NONE (default), LOSS_HUBER or LOSS_CAUCHY with scale k > 0 in units of
+        the Mahalanobis error (pixels for identity information). Context state: kept across ba_set_graph, ba_append_graph and
+        ba_restore_initial. The linearisation, the marginals and ba_chi2 (then sum rho) follow it."""
+        self._check(self.lib.spp_ba_set_robust_loss(self.h, int(kind), float(scale)))
+
+    def ba_observation_errors(self):
+        """(sq_error, weight): s2 = r^T Omega r and the loss weight w of every observation at the current states, in edge
+        insertion order; w is bit for bit the weight a linearisation at these states uses."""
+        o = self._ba_dims[2]
+        s2, w = np.empty(o), np.empty(o)
+        self._check(self.lib.spp_ba_get_observation_errors(self.h, _dp(s2), _dp(w)))
+        return s2, w
 
     def ba_linearise(self):
         self._check(self.lib.spp_ba_linearise(self.h))

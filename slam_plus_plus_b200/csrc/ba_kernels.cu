@@ -21,6 +21,11 @@
 //     bit-reproducible).
 //   * k_sum_point_records: a warp stages the contiguous records of 32 landmarks in shared memory, and the lane of each
 //     landmark adds its track's records in insertion order into V_p and g_p -- the reference's reduction plan's order.
+//
+// Robust losses (spp_ba_set_robust_loss): k_linearise_cams, k_chi2_partial and k_obs_errors take the loss as a template
+// parameter and share robust_loss(). The SPP_LOSS_NONE instantiations are the plain kernels (the loss code is compiled
+// out); under a loss the weight of an observation is computed on the fly from its residual, so no per-observation array
+// is added to the LM path.
 
 #include "spp_ctx.h"
 #include <stdlib.h>
@@ -156,6 +161,35 @@ __device__ __forceinline__ void observation_jacobians(int jac_mode, const double
 	}
 }
 
+// squared Mahalanobis error s2 = e^T Sigma^-1 e (the expression and operation order of the chi2 kernel: with e = -r the
+// same bits)
+__device__ __forceinline__ double obs_sq_error(double eu, double ev, double2 i01, double2 i23)
+{
+	return (eu * i01.x + ev * i23.x) * eu + (eu * i01.y + ev * i23.y) * ev;
+}
+
+// cost rho(s2) and IRLS weight w = rho'(s2) of one observation under the loss LOSS with scale k (spp_b200.h; the
+// reference's robust kernels: RobustUtils.h:368-586). Below the Huber threshold rho = s2 and w = 1 exactly.
+template <int LOSS>
+__device__ __forceinline__ double robust_loss(double s2, double k, double &w)
+{
+	if(LOSS == SPP_LOSS_HUBER) {
+		if(s2 <= k * k) {
+			w = 1.0;
+			return s2;
+		}
+		const double s = sqrt(s2);
+		w = k / s;
+		return 2 * k * s - k * k;
+	} else if(LOSS == SPP_LOSS_CAUCHY) {
+		const double q = s2 / (k * k);
+		w = 1.0 / (1.0 + q);
+		return k * k * log1p(q);
+	}
+	w = 1.0;
+	return s2;
+}
+
 __device__ __forceinline__ double warp_sum(double v)
 {
 	#pragma unroll
@@ -232,12 +266,14 @@ static const size_t CAM_SMEM = (size_t)(CAM_THREADS / 32) * 2 * 8 * GR_LD * size
 // fetched one trip ahead (352 -> 348 us).
 // (Measured alternatives of round 1: ten lanes per observation -- one projection per lane, the Hessian algebra spread
 // over the lanes through shared memory -- 0.97 ms against 0.81 ms.)
-template <int JAC>
+// LOSS: robust loss as a compile-time constant; under a loss the observation's information matrix is scaled by its weight
+// before any other use, so U_c, g_c, W, the landmark record and the damping maximum are those of the weighted problem.
+template <int JAC, int LOSS>
 __global__ void __launch_bounds__(CAM_THREADS, CAM_MIN_CTAS) k_linearise_cams(int, const uint32_t *__restrict__ cam_ptr,
 	const uint32_t *__restrict__ cam_obs, const uint32_t *__restrict__ obs_pt, const double *__restrict__ pts,
 	const double *__restrict__ z, const double *__restrict__ info, const double *__restrict__ camRt,
 	const double *__restrict__ camK, double *__restrict__ W, double *__restrict__ U, double *__restrict__ gc,
-	unsigned long long *__restrict__ maxdiag, long uf_cam, double *__restrict__ PtRec)
+	unsigned long long *__restrict__ maxdiag, long uf_cam, double *__restrict__ PtRec, double loss_k)
 {
 	extern __shared__ __align__(16) double gram[]; // per warp: T [8][GR_LD], then [Jc | r] [8][GR_LD]
 	__shared__ double sRt[7 * 12];
@@ -277,6 +313,12 @@ __global__ void __launch_bounds__(CAM_THREADS, CAM_MIN_CTAS) k_linearise_cams(in
 				p_nx = obs_pt[o_nx];
 			double Jc[12];
 			observation_jacobians(JAC, sRt, sK, X, Y, Z, zz.x, zz.y, Jc, Jp, ru, rv, true, true);
+			if(LOSS != SPP_LOSS_NONE) { // Sigma^-1 <- w Sigma^-1
+				double w;
+				robust_loss<LOSS>(obs_sq_error(ru, rv, i01, i23), loss_k, w);
+				i01.x *= w; i01.y *= w;
+				i23.x *= w; i23.y *= w;
+			}
 			// T = Jc^T Sigma^-1 (6x2): T(j,0) = Jc(0,j) s00 + Jc(1,j) s10 ; T(j,1) = Jc(0,j) s01 + Jc(1,j) s11
 			#pragma unroll
 			for(int j = 0; j < 6; ++ j) {
@@ -418,13 +460,14 @@ __global__ void __launch_bounds__(SR_WARPS * 32) k_sum_point_records(size_t P, c
 		gp[p0 * 3 + i] = sg[i];
 }
 
-// chi2: thread per observation, block partials, then a fixed-order final pass
+// chi2 (under a loss: sum rho(s2)): thread per observation, block partials, then a fixed-order final pass
 #define RED_THREADS 256
 
+template <int LOSS>
 __global__ void __launch_bounds__(RED_THREADS) k_chi2_partial(size_t O, const uint32_t *__restrict__ obs_cam,
 	const uint32_t *__restrict__ obs_pt, const double *__restrict__ pts, const double *__restrict__ z,
 	const double *__restrict__ info, const double *__restrict__ camRt, const double *__restrict__ camK,
-	double *__restrict__ partial)
+	double *__restrict__ partial, double loss_k)
 {
 	__shared__ double sred[RED_THREADS / 32];
 	double acc = 0;
@@ -439,7 +482,8 @@ __global__ void __launch_bounds__(RED_THREADS) k_chi2_partial(size_t O, const ui
 		const double2 i23 = *reinterpret_cast<const double2*>(info + o * 4 + 2);
 		double eu = u - zz.x, ev = v - zz.y;
 		// (e^T Sigma^-1) . e
-		acc += (eu * i01.x + ev * i23.x) * eu + (eu * i01.y + ev * i23.y) * ev;
+		double w;
+		acc += robust_loss<LOSS>(obs_sq_error(eu, ev, i01, i23), loss_k, w);
 	}
 	acc = warp_sum(acc);
 	if((threadIdx.x & 31) == 0) sred[threadIdx.x >> 5] = acc;
@@ -449,6 +493,33 @@ __global__ void __launch_bounds__(RED_THREADS) k_chi2_partial(size_t O, const ui
 		for(int w = 1; w < RED_THREADS / 32; ++ w) v += sred[w];
 		partial[blockIdx.x] = v;
 	}
+}
+
+// s2 and w of every observation at the current states, written in edge insertion order (spp_ba_get_observation_errors).
+// The residual comes from observation_jacobians in the Jacobian mode JAC (FD: project_Rt of the base pose, analytic:
+// project_with_dx), as in k_linearise_cams, so w is bit for bit the weight of the linearisation.
+template <int JAC, int LOSS>
+__global__ void __launch_bounds__(RED_THREADS) k_obs_errors(size_t O, const uint32_t *__restrict__ obs_cam,
+	const uint32_t *__restrict__ obs_pt, const uint32_t *__restrict__ obs_orig, const double *__restrict__ pts,
+	const double *__restrict__ z, const double *__restrict__ info, const double *__restrict__ camRt,
+	const double *__restrict__ camK, double loss_k, double *__restrict__ sq_err, double *__restrict__ weight)
+{
+	const size_t o = blockIdx.x * (size_t)RED_THREADS + threadIdx.x;
+	if(o >= O)
+		return;
+	const unsigned c = obs_cam[o], p = obs_pt[o];
+	const double2 zz = *reinterpret_cast<const double2*>(z + o * 2);
+	const double2 i01 = *reinterpret_cast<const double2*>(info + o * 4);
+	const double2 i23 = *reinterpret_cast<const double2*>(info + o * 4 + 2);
+	double Jc[12], Jp[6], ru, rv;
+	observation_jacobians(JAC, camRt + (size_t)c * 84, camK + (size_t)c * 5, pts[(size_t)p * 3], pts[(size_t)p * 3 + 1],
+		pts[(size_t)p * 3 + 2], zz.x, zz.y, Jc, Jp, ru, rv, false, false);
+	const double s2 = obs_sq_error(ru, rv, i01, i23);
+	double w;
+	robust_loss<LOSS>(s2, loss_k, w);
+	const size_t e = obs_orig[o];
+	sq_err[e] = s2;
+	weight[e] = w;
 }
 
 // out[k] = sum_i partial[k * stride + i], i < n ; single block, fixed order
@@ -530,6 +601,34 @@ void ba_prepare_cameras(spp_ctx *ctx, bool b_with_perturbations)
 	LAUNCH_CHECK(ctx);
 }
 
+template <int JAC, int LOSS>
+static void launch_linearise_cams(spp_ctx *ctx, unsigned long long *p_max)
+{
+	BAProblem &ba = ctx->ba;
+	SchurSystem &s = ctx->sys;
+	k_linearise_cams<JAC, LOSS><<<(unsigned)s.C, CAM_THREADS, CAM_SMEM, ctx->stream>>>(ba.jac_mode, s.cam_ptr.p(),
+		s.cam_obs.p(), s.obs_pt.p(), ba.pts.p(), ba.z.p(), ba.info.p(), ba.camRt.p(), ba.camK.p(), s.W.p(), s.U.p(), s.gc.p(),
+		p_max, ba.uf_is_cam? ba.uf_index : -1, ba.pt_rec.p(), ba.loss_scale);
+}
+
+template <int JAC>
+static void launch_linearise_cams_loss(spp_ctx *ctx, unsigned long long *p_max)
+{
+	switch(ctx->ba.loss_kind) {
+	case SPP_LOSS_HUBER: launch_linearise_cams<JAC, SPP_LOSS_HUBER>(ctx, p_max); break;
+	case SPP_LOSS_CAUCHY: launch_linearise_cams<JAC, SPP_LOSS_CAUCHY>(ctx, p_max); break;
+	default: launch_linearise_cams<JAC, SPP_LOSS_NONE>(ctx, p_max); break;
+	}
+}
+
+template <int JAC>
+static void set_linearise_cams_smem()
+{
+	SPP_CUDA(cudaFuncSetAttribute(k_linearise_cams<JAC, SPP_LOSS_NONE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CAM_SMEM));
+	SPP_CUDA(cudaFuncSetAttribute(k_linearise_cams<JAC, SPP_LOSS_HUBER>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CAM_SMEM));
+	SPP_CUDA(cudaFuncSetAttribute(k_linearise_cams<JAC, SPP_LOSS_CAUCHY>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CAM_SMEM));
+}
+
 void ba_linearise(spp_ctx *ctx, bool b_want_maxdiag)
 {
 	BAProblem &ba = ctx->ba;
@@ -545,18 +644,14 @@ void ba_linearise(spp_ctx *ctx, bool b_want_maxdiag)
 	if(s.C) {
 		static bool attr_done[64] = {false};
 		if(ctx->device >= 0 && ctx->device < 64 && !attr_done[ctx->device]) {
-			SPP_CUDA(cudaFuncSetAttribute(k_linearise_cams<SPP_JAC_FD_REFERENCE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CAM_SMEM));
-			SPP_CUDA(cudaFuncSetAttribute(k_linearise_cams<SPP_JAC_ANALYTIC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CAM_SMEM));
+			set_linearise_cams_smem<SPP_JAC_FD_REFERENCE>();
+			set_linearise_cams_smem<SPP_JAC_ANALYTIC>();
 			attr_done[ctx->device] = true;
 		}
-#define LAUNCH_CAMS(JAC) k_linearise_cams<JAC><<<(unsigned)s.C, CAM_THREADS, CAM_SMEM, ctx->stream>>>(ba.jac_mode, s.cam_ptr.p(), \
-			s.cam_obs.p(), s.obs_pt.p(), ba.pts.p(), ba.z.p(), ba.info.p(), ba.camRt.p(), ba.camK.p(), s.W.p(), s.U.p(), s.gc.p(), \
-			p_max, ba.uf_is_cam? ba.uf_index : -1, ba.pt_rec.p())
 		if(ba.jac_mode == SPP_JAC_FD_REFERENCE)
-			LAUNCH_CAMS(SPP_JAC_FD_REFERENCE);
+			launch_linearise_cams_loss<SPP_JAC_FD_REFERENCE>(ctx, p_max);
 		else
-			LAUNCH_CAMS(SPP_JAC_ANALYTIC);
-#undef LAUNCH_CAMS
+			launch_linearise_cams_loss<SPP_JAC_ANALYTIC>(ctx, p_max);
 		LAUNCH_CHECK(ctx);
 	}
 	if(s.P) {
@@ -575,10 +670,46 @@ void ba_chi2_device(spp_ctx *ctx, double *d_out)
 	ba_prepare_cameras(ctx, false);
 	const unsigned G = 148 * 4;
 	ba.partial.resize(4 * 1024);
-	k_chi2_partial<<<G, RED_THREADS, 0, ctx->stream>>>(s.O, s.obs_cam.p(), s.obs_pt.p(), ba.pts.p(), ba.z.p(),
-		ba.info.p(), ba.camRt.p(), ba.camK.p(), ba.partial.p());
+#define LAUNCH_CHI2(LOSS) k_chi2_partial<LOSS><<<G, RED_THREADS, 0, ctx->stream>>>(s.O, s.obs_cam.p(), s.obs_pt.p(), ba.pts.p(), \
+		ba.z.p(), ba.info.p(), ba.camRt.p(), ba.camK.p(), ba.partial.p(), ba.loss_scale)
+	switch(ba.loss_kind) {
+	case SPP_LOSS_HUBER: LAUNCH_CHI2(SPP_LOSS_HUBER); break;
+	case SPP_LOSS_CAUCHY: LAUNCH_CHI2(SPP_LOSS_CAUCHY); break;
+	default: LAUNCH_CHI2(SPP_LOSS_NONE); break;
+	}
+#undef LAUNCH_CHI2
 	LAUNCH_CHECK(ctx);
 	k_final_sum<<<1, RED_THREADS, 0, ctx->stream>>>(ba.partial.p(), G, 0, d_out);
+	LAUNCH_CHECK(ctx);
+}
+
+template <int JAC>
+static void launch_obs_errors(spp_ctx *ctx, double *d_sq_err, double *d_weight)
+{
+	BAProblem &ba = ctx->ba;
+	SchurSystem &s = ctx->sys;
+#define LAUNCH_ERR(LOSS) k_obs_errors<JAC, LOSS><<<n_blocks(s.O, RED_THREADS), RED_THREADS, 0, ctx->stream>>>(s.O, s.obs_cam.p(), \
+		s.obs_pt.p(), ba.d_obs_orig.p(), ba.pts.p(), ba.z.p(), ba.info.p(), ba.camRt.p(), ba.camK.p(), ba.loss_scale, d_sq_err, d_weight)
+	switch(ba.loss_kind) {
+	case SPP_LOSS_HUBER: LAUNCH_ERR(SPP_LOSS_HUBER); break;
+	case SPP_LOSS_CAUCHY: LAUNCH_ERR(SPP_LOSS_CAUCHY); break;
+	default: LAUNCH_ERR(SPP_LOSS_NONE); break;
+	}
+#undef LAUNCH_ERR
+}
+
+// d_sq_err[O], d_weight[O]: s2 and w of every observation at the current states, in edge insertion order
+void ba_obs_errors_device(spp_ctx *ctx, double *d_sq_err, double *d_weight)
+{
+	BAProblem &ba = ctx->ba;
+	SchurSystem &s = ctx->sys;
+	if(!s.O)
+		return;
+	ba_prepare_cameras(ctx, false); // the base pose: all the residual needs in either Jacobian mode
+	if(ba.jac_mode == SPP_JAC_FD_REFERENCE)
+		launch_obs_errors<SPP_JAC_FD_REFERENCE>(ctx, d_sq_err, d_weight);
+	else
+		launch_obs_errors<SPP_JAC_ANALYTIC>(ctx, d_sq_err, d_weight);
 	LAUNCH_CHECK(ctx);
 }
 

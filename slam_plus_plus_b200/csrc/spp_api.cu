@@ -31,6 +31,7 @@ void map_blocks_to_global(size_t C, const std::vector<uint32_t> &l_row, const st
 	const std::vector<uint32_t> &g_row, const std::vector<uint32_t> &g_col, std::vector<uint32_t> &slot);
 void ba_linearise(spp_ctx *ctx, bool b_want_maxdiag);
 void ba_chi2_device(spp_ctx *ctx, double *d_out);
+void ba_obs_errors_device(spp_ctx *ctx, double *d_sq_err, double *d_weight);
 void ba_step_dots_device(spp_ctx *ctx, double alpha, double *d_out);
 void ba_apply_update(spp_ctx *ctx);
 void schur_form_reduced_system(spp_ctx *ctx, double alpha, double alpha_diag, bool sparse_rcs);
@@ -1042,6 +1043,33 @@ int spp_ba_set_jacobian_mode(spp_ctx_t ctx, int mode)
 	ctx->ba.jac_mode = mode;
 	ctx->ba.linearised = false;
 	return SPP_OK;
+}
+
+int spp_ba_set_robust_loss(spp_ctx_t ctx, int kind, double scale)
+{
+	if(!ctx || (kind != SPP_LOSS_NONE && kind != SPP_LOSS_HUBER && kind != SPP_LOSS_CAUCHY))
+		return SPP_ERR_INVALID;
+	if(kind != SPP_LOSS_NONE && !(std::isfinite(scale) && scale > 0))
+		return SPP_ERR_INVALID;
+	ctx->ba.loss_kind = kind;
+	ctx->ba.loss_scale = kind == SPP_LOSS_NONE? 1.0 : scale;
+	ctx->ba.linearised = false;
+	return SPP_OK;
+}
+
+int spp_ba_get_observation_errors(spp_ctx_t ctx, double *p_sq_error, double *p_weight)
+{
+	API_BEGIN(ctx)
+	BAProblem &ba = ctx->ba;
+	SchurSystem &s = ctx->sys;
+	if(!ba.valid) throw invalid_error("no BA graph");
+	if(ctx->world > 1) throw invalid_error("not available on a landmark-partitioned (multi-GPU) context");
+	ba.obs_err.resize(2 * s.O + 2);
+	ba_obs_errors_device(ctx, ba.obs_err.p(), ba.obs_err.p() + s.O);
+	if(p_sq_error) ba.obs_err.download(p_sq_error, s.O, ctx->stream);
+	if(p_weight && s.O) SPP_CUDA(cudaMemcpyAsync(p_weight, ba.obs_err.p() + s.O, s.O * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+	SPP_CUDA(cudaStreamSynchronize(ctx->stream));
+	API_END(ctx)
 }
 
 int spp_ba_linearise(spp_ctx_t ctx)

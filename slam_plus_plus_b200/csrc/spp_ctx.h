@@ -74,6 +74,7 @@ struct BAProblem {
 	int uf_is_cam; long uf_index;        // vertex id 0 carries the unary factor (-1: added by another rank)
 	size_t P_global, pt_begin, pt_end;   // landmark slice of this rank (multi-GPU)
 	int jac_mode;
+	int loss_kind; double loss_scale;    // robust loss of the observations (SPP_LOSS_*, scale k), context state like jac_mode
 	// device state
 	DBuf<double> cam_state, cam_intr, pts;        // [6C], [5C], [3P]
 	DBuf<double> cam_state_saved, pts_saved;
@@ -84,9 +85,10 @@ struct BAProblem {
 	DBuf<double> pt_rec;                          // [O*10] per observation: upper(Jp^T Sigma^-1 Jp) (6), Jp^T Sigma^-1 r (3), pad
 	DBuf<double> partial;                         // reduction scratch
 	DBuf<unsigned long long> maxdiag;             // [1] bits of the max per-edge Hessian diagonal
+	DBuf<double> obs_err;                         // [2O] scratch of spp_ba_get_observation_errors (s2, w; edge insertion order)
 	bool linearised;
 	BAProblem() : valid(false), n_vertices(0), host_maps_valid(false), raw_on_device(false), n_obs_raw(0), uf_is_cam(1), uf_index(0), P_global(0), pt_begin(0),
-		pt_end(0), jac_mode(0), linearised(false) {}
+		pt_end(0), jac_mode(0), loss_kind(0), loss_scale(1.0), linearised(false) {}
 };
 
 // slot-1 state: map from the caller's lambda values to the SchurSystem arrays

@@ -129,6 +129,17 @@ def make_ba(n_cams: int, n_pts: int, seed: int, mean_extra_track: float = 3.35, 
     return BAGraph(vtype, cams, pts_n, obs_pt.astype(np.int64), obs_cam.astype(np.int64), z, info)
 
 
+def add_outliers(g: BAGraph, fraction: float, seed: int):
+    """A copy of `g` in which a seeded `fraction` of the measurements is replaced by pixels drawn uniformly from
+    [0, 800)^2 (gross mismatches, as automatic feature matching leaves them), and the sorted edge indices replaced."""
+    rng = np.random.default_rng(seed)
+    n = len(g.obs_pt)
+    idx = np.sort(rng.choice(n, int(round(fraction * n)), replace=False))
+    z = np.array(g.z, np.float64, copy=True)
+    z[idx] = rng.uniform(0.0, 800.0, (len(idx), 2))
+    return BAGraph(g.vtype, g.cams, g.pts, g.obs_pt, g.obs_cam, z, g.info), idx
+
+
 BA_SHAPES = {
     # name: (n_cams, n_pts, seed, kwargs)
     "venice871": (871, 530304, 871, dict(mean_extra_track=3.35, max_track=60, max_stride=11)),
