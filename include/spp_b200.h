@@ -400,12 +400,17 @@ int spp_chol_symbolic(spp_ctx_t ctx, size_t n_block_cols, size_t block_size, con
  * Cholesky (CUberBlockMatrix::CholeskyOf_FBS, include/slam/BlockMatrixFBS.inl:2341-2513) and the two triangular
  * solves (:2136-2275). p_values: the blocks in the order of the structure (column-major blocks; of the diagonal
  * blocks the full symmetric block is read); p_eta_dx: right-hand side in, solution out.
- * Returns SPP_NOT_POSDEF where the reference returns false. */
+ * Returns SPP_NOT_POSDEF where the reference returns false.
+ * The slot and the pose-graph solves (spp_pose_solve_step, spp_pose_optimize) share one analysis per context. A pose
+ * solve replaces the slot's analysis with its own, and the slot does not keep its structure: spp_chol_solve after a pose
+ * solve returns SPP_ERR_INVALID until spp_chol_symbolic is called again. A pose solve after spp_chol_symbolic repeats
+ * the pose graph's analysis by itself. */
 int spp_chol_solve(spp_ctx_t ctx, const double *p_values, double *p_eta_dx);
 
 /* The factor of the last spp_chol_solve / spp_pose_* solve in the reference's form, the upper factor R with
  * R^T R = P lambda P^T (block CSC in the permuted order, rows ascending, diagonal last; column-major blocks), for the
  * parity tests: with the reference's ordering the block pattern of R must be the reference's, bit for bit.
+ * After a pose solve this is the pose graph's factor: n_poses block columns of dim x dim blocks.
  * Call with NULL arrays to obtain the block count. */
 int spp_chol_get_factor(spp_ctx_t ctx, uint64_t *p_n_blocks, uint64_t *p_col_ptr, uint64_t *p_row_idx, double *p_values);
 

@@ -26,7 +26,7 @@
 
 namespace spp {
 
-void sparse_chol_symbolic(spp_ctx *ctx, size_t n, size_t B, const uint64_t *col_ptr, const uint64_t *row_idx,
+void sparse_chol_symbolic(spp_ctx *ctx, int owner, size_t n, size_t B, const uint64_t *col_ptr, const uint64_t *row_idx,
 	const uint64_t *p_order_in);
 int sparse_chol_solve_device(spp_ctx *ctx, const double *d_A, const double *d_rhs, double *d_x);
 
@@ -531,8 +531,10 @@ static double pose_dx_norm(spp_ctx *ctx)
 int pose_solve(spp_ctx *ctx)
 {
 	PoseProblem &pp = ctx->pose;
-	if(!pp.symbolic_done) { // FinalBlockStructure: once per structure (Lambda.h:607-612)
-		sparse_chol_symbolic(ctx, pp.N, pp.dim, pp.h_col_ptr.data(), pp.h_row_idx.data(),
+	// FinalBlockStructure: once per structure (Lambda.h:607-612), and again after spp_chol_symbolic has put the slot's
+	// analysis in the shared SparseChol
+	if(!pp.symbolic_done || ctx->schol.owner != SC_OWNER_POSE) {
+		sparse_chol_symbolic(ctx, SC_OWNER_POSE, pp.N, pp.dim, pp.h_col_ptr.data(), pp.h_row_idx.data(),
 			pp.h_order_in.size() == pp.N? pp.h_order_in.data() : 0);
 		pp.symbolic_done = true;
 	}

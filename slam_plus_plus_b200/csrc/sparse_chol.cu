@@ -42,12 +42,14 @@ int dense_chol_solve_device(spp_ctx *ctx, double *A, size_t n, double *d_rhs_x);
 // ---- host: symbolic analysis ---------------------------------------------------------------------------
 
 // Input: upper block structure in the caller's order (CSC, rows ascending, diagonal present), the ordering
-// order[new] = old. Builds everything the numeric kernels need and uploads it.
-void sparse_chol_symbolic(spp_ctx *ctx, size_t n, size_t B, const uint64_t *col_ptr, const uint64_t *row_idx,
+// order[new] = old. Builds everything the numeric kernels need and uploads it; owner (SC_OWNER_SLOT / SC_OWNER_POSE)
+// is recorded once the analysis is complete.
+void sparse_chol_symbolic(spp_ctx *ctx, int owner, size_t n, size_t B, const uint64_t *col_ptr, const uint64_t *row_idx,
 	const uint64_t *p_order_in)
 {
 	SparseChol &sc = ctx->schol;
 	sc.valid = false;
+	sc.owner = SC_OWNER_NONE;
 	sc.n = n; sc.B = B;
 	if(n >= 0x7fffffffu)
 		throw invalid_error("sparse Cholesky: too many block columns for 32-bit indices");
@@ -290,6 +292,7 @@ void sparse_chol_symbolic(spp_ctx *ctx, size_t n, size_t B, const uint64_t *col_
 		fprintf(stderr, "[spp sparse chol] n %zu (B = %zu), A blocks %zu, L blocks %zu, levels %u (cooperative 0..%u, single CTA ..%u), "
 			"dense root front %zu columns (%zu blocks)\n", n, B, sc.n_a_blocks, nb, n_levels_all, tail, n_levels, m, sc.n_root_blocks);
 	sc.valid = true;
+	sc.owner = owner;
 }
 
 // ---- device: numeric phase ------------------------------------------------------------------------------
@@ -607,12 +610,14 @@ static int sparse_chol_numeric_t(spp_ctx *ctx, SparseCholArgs &a)
 	SparseChol &sc = ctx->schol;
 	cudaStream_t st = ctx->stream;
 	SPP_CUDA(cudaMemsetAsync(sc.d_info.p(), 0, sizeof(int), st));
-	if(!sc.max_coop_ctas) {
-		int per_sm = 0, n_sm = 0, dev = 0;
+	if(sc.coop_B != B) { // both cooperative kernels of this block size must be co-resident on the grid
+		int per_sm = 0, per_sm_bs = 0, n_sm = 0, dev = 0;
 		SPP_CUDA(cudaGetDevice(&dev));
 		SPP_CUDA(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev));
 		SPP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sparse_chol<B, true>, SC_WARPS * 32, 0));
-		sc.max_coop_ctas = std::max(1, std::min(per_sm, 2) * n_sm);
+		SPP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_bs, k_sparse_backsolve<B, true>, SC_WARPS * 32, 0));
+		sc.max_coop_ctas = std::max(1, std::min(std::min(per_sm, per_sm_bs), 2) * n_sm);
+		sc.coop_B = B;
 	}
 	uint32_t zero = 0, tail = sc.tail_level, nl = sc.n_levels;
 	if(tail > 0) {

@@ -57,7 +57,7 @@ void slot_symbolic(spp_ctx *ctx, size_t n, const uint64_t *col_dims, const uint6
 	uint64_t *p_order, uint64_t *p_cut);
 int slot_solve(spp_ctx *ctx, const double *p_values, double *p_eta_dx);
 
-void sparse_chol_symbolic(spp_ctx *ctx, size_t n, size_t B, const uint64_t *col_ptr, const uint64_t *row_idx,
+void sparse_chol_symbolic(spp_ctx *ctx, int owner, size_t n, size_t B, const uint64_t *col_ptr, const uint64_t *row_idx,
 	const uint64_t *p_order_in);
 int sparse_chol_solve_device(spp_ctx *ctx, const double *d_A, const double *d_rhs, double *d_x);
 void pose_set_graph(spp_ctx *ctx, int dim, size_t N, const double *p_states, size_t E, const uint64_t *p_from,
@@ -1706,7 +1706,7 @@ int spp_chol_symbolic(spp_ctx_t ctx, size_t n_block_cols, size_t block_size, con
 	API_BEGIN(ctx)
 	if(!n_block_cols || !p_col_ptr || !p_row_idx) throw invalid_error("null argument");
 	if(block_size != 2 && block_size != 3 && block_size != 6) throw invalid_error("block size must be 2, 3 or 6");
-	sparse_chol_symbolic(ctx, n_block_cols, block_size, p_col_ptr, p_row_idx, p_order_in);
+	sparse_chol_symbolic(ctx, SC_OWNER_SLOT, n_block_cols, block_size, p_col_ptr, p_row_idx, p_order_in);
 	if(p_order_out)
 		for(size_t i = 0; i < n_block_cols; ++ i) p_order_out[i] = ctx->schol.h_order[i];
 	API_END(ctx)
@@ -1718,6 +1718,8 @@ int spp_chol_solve(spp_ctx_t ctx, const double *p_values, double *p_eta_dx)
 	API_BEGIN(ctx)
 	SparseChol &sc = ctx->schol;
 	if(!sc.valid) throw invalid_error("spp_chol_symbolic() has not been called");
+	// the slot does not keep its structure: after a pose solve, the analysis in memory is the pose graph's
+	if(sc.owner != SC_OWNER_SLOT) throw invalid_error("the block-sparse analysis in use is the pose graph's: call spp_chol_symbolic again");
 	if(!p_values || !p_eta_dx) throw invalid_error("null argument");
 	const size_t nv = sc.n_a_blocks * sc.B * sc.B, ns = sc.n * sc.B;
 	sc.slot_vals.upload(p_values, nv, ctx->stream);

@@ -119,12 +119,15 @@ struct SymbolicScratch {
 	DBuf<uint32_t> sl_flag, sl_pos, sl_kept, sl_ocam, sl_opt; // several ranks: compaction of this rank's edges
 };
 
-// block-sparse Cholesky (sparse_chol.cu): symbolic structures and the factor
+// block-sparse Cholesky (sparse_chol.cu): symbolic structures and the factor. The spp_chol_* slot and the pose path share
+// it; owner names the one whose structure the analysis in memory was made for.
+enum { SC_OWNER_NONE = 0, SC_OWNER_SLOT, SC_OWNER_POSE };
 struct SparseChol {
 	bool valid;
+	int owner;                       // SC_OWNER_*
 	size_t n, B, n_a_blocks, n_l_blocks;
 	uint32_t n_levels, tail_level;
-	int max_coop_ctas;
+	int max_coop_ctas, coop_B;       // cooperative grid size, computed for the kernels of block size coop_B
 	std::vector<uint32_t> h_order;   // new position -> caller's block column
 	std::vector<uint64_t> h_lptr;    // column pointers of L
 	std::vector<uint32_t> h_lrow, h_parent;
@@ -139,8 +142,8 @@ struct SparseChol {
 	DBuf<uint32_t> d_root_blk, d_root_ua, d_root_ub, d_root_rblk, d_root_cols, d_ridx;
 	DBuf<uint64_t> d_root_uptr, d_root_rptr;
 	DBuf<double> d_root_S, d_root_rhs;
-	SparseChol() : valid(false), n(0), B(0), n_a_blocks(0), n_l_blocks(0), n_levels(0), tail_level(0), max_coop_ctas(0),
-		n_root(0), n_root_blocks(0) {}
+	SparseChol() : valid(false), owner(SC_OWNER_NONE), n(0), B(0), n_a_blocks(0), n_l_blocks(0), n_levels(0), tail_level(0),
+		max_coop_ctas(0), coop_B(0), n_root(0), n_root_blocks(0) {}
 };
 
 // pose graph resident on the device (pose_kernels.cu)
