@@ -16,7 +16,7 @@
 //   k_gemm_tn<TRSM> block row right of the diagonal: P <- Rinv_kk^T P        (FP64 tensor cores)
 //   k_gemm_tn<SYRK> trailing update C -= P^T P, upper tiles only             (FP64 tensor cores)
 //                   critical stream: the tile row that the next panel needs (64x64 tiles, look-ahead)
-//                   bulk stream    : everything below it (128x128 tiles)
+//                   bulk stream    : everything below it (128x64 tiles)
 // The GEMM kernel stages K-contiguous operand tiles with a 3-deep cp.async pipeline and issues
 // mma.sync.m8n8k4.f64 (DMMA); tcgen05 has no FP64 kind, so this is the tensor path for FP64 on sm_100a.
 // Backward solve: one persistent CTA per block row consumes x_j as soon as block row j publishes it and
@@ -52,8 +52,7 @@ enum { GEMM_SYRK = 0, GEMM_TRSM = 1, GEMM_GRAM = 2 };
 //       slot): C(i0.., j0..) -= Z(k0.., i0..)^T Z(k0.., j0..) -- the inverse of a factored matrix as Z^T Z, Z = R^-T.
 // WM x WN is the warp tile (multiples of 8): 32 x 32 for the bulk updates, smaller for the few tiles on the critical
 // chain, where more warps with shorter DMMA chains finish sooner.
-// KN: number of operand rows = K of the product (128: one panel; 256: two consecutive panels applied in one pass).
-template <int MODE, int BM, int BN, int WM = 32, int WN = 32, int STAGES = CH_STAGES, int KN = CH_NB>
+template <int MODE, int BM, int BN, int WM = 32, int WN = 32, int STAGES = CH_STAGES>
 __global__ void __launch_bounds__((BM / WM) * (BN / WN) * 32) k_gemm_tn(double *__restrict__ A, size_t ld, size_t k0,
 	size_t rbase, size_t cbase, const double *__restrict__ Rinv)
 {
@@ -97,7 +96,7 @@ __global__ void __launch_bounds__((BM / WM) * (BN / WN) * 32) k_gemm_tn(double *
 
 	double acc[MA][NB][2];
 
-	constexpr int KT = KN / CH_BK;
+	constexpr int KT = CH_NB / CH_BK;
 	#pragma unroll
 	for(int s = 0; s < STAGES - 1; ++ s) {
 		stage_load(s, s);
@@ -272,7 +271,6 @@ static void chol_init_attributes(int device)
 	if(device < 0 || device >= 64 || done[device]) return;
 	SPP_CUDA(cudaFuncSetAttribute(k_potrf128, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)POTRF_SMEM_EXCLUSIVE));
 	SPP_CUDA(cudaFuncSetAttribute(k_backsolve, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)BACKSOLVE_SMEM));
-	SPP_CUDA(cudaFuncSetAttribute(k_gemm_tn<GEMM_SYRK, 128, 128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gemm_smem<128, 128>()));
 	SPP_CUDA(cudaFuncSetAttribute(k_gemm_tn<GEMM_SYRK, 128, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gemm_smem<128, 64>()));
 	SPP_CUDA(cudaFuncSetAttribute(k_gemm_tn<GEMM_SYRK, 64, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gemm_smem<64, 64>()));
 	SPP_CUDA(cudaFuncSetAttribute(k_gemm_tn<GEMM_TRSM, 128, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gemm_smem<128, 64>()));
@@ -280,10 +278,6 @@ static void chol_init_attributes(int device)
 	SPP_CUDA(cudaFuncSetAttribute(k_gemm_tn<GEMM_GRAM, 64, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gemm_smem<64, 64>()));
 	SPP_CUDA(cudaFuncSetAttribute((k_gemm_tn<GEMM_TRSM, 128, 16, 32, 16, 8>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gemm_smem<128, 16, 8>()));
 	SPP_CUDA(cudaFuncSetAttribute((k_gemm_tn<GEMM_SYRK, 32, 32, 16, 16, 8>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gemm_smem<32, 32, 8>()));
-	SPP_CUDA(cudaFuncSetAttribute((k_gemm_tn<GEMM_SYRK, 128, 128, 32, 32, CH_STAGES, 256>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gemm_smem<128, 128>()));
-	SPP_CUDA(cudaFuncSetAttribute((k_gemm_tn<GEMM_SYRK, 128, 64, 32, 32, CH_STAGES, 256>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gemm_smem<128, 64>()));
-	SPP_CUDA(cudaFuncSetAttribute((k_gemm_tn<GEMM_SYRK, 64, 64, 32, 32, CH_STAGES, 256>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gemm_smem<64, 64>()));
-	SPP_CUDA(cudaFuncSetAttribute((k_gemm_tn<GEMM_SYRK, 32, 32, 16, 16, 8, 256>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gemm_smem<32, 32, 8>()));
 	done[device] = true;
 }
 
@@ -306,9 +300,6 @@ static void chol_init_streams(spp_ctx *ctx)
 		SPP_CUDA(cudaEventCreateWithFlags(&ch.ev_bulk[i], cudaEventDisableTiming));
 		SPP_CUDA(cudaEventCreateWithFlags(&ch.ev_row[i], cudaEventDisableTiming));
 	}
-	ch.profile = getenv("SPP_CHOL_PROFILE") != 0;
-	ch.force_tile = getenv("SPP_CHOL_TILE")? atoi(getenv("SPP_CHOL_TILE")) : -1;
-	ch.potrf_exclusive = getenv("SPP_CHOL_SHARED_SM") == 0;
 }
 
 // Partial right-looking factorisation of a block ROW panel: A is column-major with ld rows (a multiple of 128) and
@@ -325,212 +316,95 @@ void dense_chol_factor_panel(spp_ctx *ctx, double *A, size_t ld, size_t n_cols_a
 	DenseChol &ch = ctx->chol;
 	chol_init_streams(ctx);
 	const size_t n_blk = ld / CH_NB;
-	const size_t n = ld; // for the profile print
-	cudaStream_t st = ctx->stream;
 	// factorisation with one-step look-ahead on three streams:
 	//   sA (critical): potrf(b) -> trsm(b) -> update of the next diagonal tile -> potrf(b+1) ...
 	//   sC           : update of the rest of the next panel's tile row (needed by trsm(b+1) only)
 	//   sB (bulk)    : update of everything below that row, overlapping potrf/trsm of the next panel
-	{
-		cudaStream_t sA = st, sB = ch.bulk_stream, sC = ch.row_stream;
-		const bool prof = ch.profile;
-		if(prof) {
-			sB = sC = sA;
-			ch.dbg.resize(16);
-		}
-		float t_acc[5] = {0, 0, 0, 0, 0};
-		// SPP_CHOL_TIMELINE: time stamps on the critical stream only (no serialisation): per panel, before potrf, after
-		// potrf, after the first-tile solve, after the diagonal look-ahead update
-		static const bool timeline = getenv("SPP_CHOL_TIMELINE") != 0;
-		std::vector<cudaEvent_t> tl;
-		auto stamp = [&]() {
-			if(timeline && !prof) {
-				cudaEvent_t e;
-				cudaEventCreate(&e);
-				cudaEventRecord(e, sA);
-				tl.push_back(e);
-			}
-		};
-		auto tic = [&]() { if(prof) cudaEventRecord(ctx->ev[4], sA); };
-		auto toc = [&](int k) {
-			if(prof) {
-				cudaEventRecord(ctx->ev[5], sA);
-				cudaEventSynchronize(ctx->ev[5]);
-				float ms;
-				cudaEventElapsedTime(&ms, ctx->ev[4], ctx->ev[5]);
-				t_acc[k] += ms;
-			}
-		};
-		// C(rows r0.., cols c0..) -= P^T P on the upper tiles of a (n_r x n_c) region, tile shape by size
-		// two_panels: P = the 256 rows from k0 on (the deferred update of the previous panel rides along)
-		auto syrk = [&](cudaStream_t s, size_t k0, size_t r0, size_t c0, size_t n_r, size_t n_c, int tile, bool two_panels) {
-			if(tile == 0) {
-				dim3 grid((unsigned)(n_c / 128), (unsigned)(n_r / 128));
-				if(two_panels)
-					k_gemm_tn<GEMM_SYRK, 128, 128, 32, 32, CH_STAGES, 256><<<grid, 512, gemm_smem<128, 128>(), s>>>(A, ld, k0, r0, c0, 0);
-				else
-					k_gemm_tn<GEMM_SYRK, 128, 128><<<grid, 512, gemm_smem<128, 128>(), s>>>(A, ld, k0, r0, c0, 0);
-			} else if(tile == 1) {
-				dim3 grid((unsigned)(n_c / 64), (unsigned)(n_r / 128));
-				if(two_panels)
-					k_gemm_tn<GEMM_SYRK, 128, 64, 32, 32, CH_STAGES, 256><<<grid, 256, gemm_smem<128, 64>(), s>>>(A, ld, k0, r0, c0, 0);
-				else
-					k_gemm_tn<GEMM_SYRK, 128, 64><<<grid, 256, gemm_smem<128, 64>(), s>>>(A, ld, k0, r0, c0, 0);
-			} else {
-				dim3 grid((unsigned)(n_c / 64), (unsigned)(n_r / 64));
-				if(two_panels)
-					k_gemm_tn<GEMM_SYRK, 64, 64, 32, 32, CH_STAGES, 256><<<grid, 128, gemm_smem<64, 64>(), s>>>(A, ld, k0, r0, c0, 0);
-				else
-					k_gemm_tn<GEMM_SYRK, 64, 64><<<grid, 128, gemm_smem<64, 64>(), s>>>(A, ld, k0, r0, c0, 0);
-			}
-			LAUNCH_CHECK(ctx);
-		};
-		// Bulk updates in pairs (SPP_CHOL_PAIRS=1, off by default): the bulk update of an even panel is deferred and applied
-		// together with the next panel's as one rank-256 pass (half the launches, half the read-modify-write traffic of the
-		// trailing matrix, twice the K per tile); the look-ahead of the odd panel then carries both panels into the next
-		// tile row. Bit-identical results, but MEASURED SLOWER on the Venice system (5226^2: 3.55 ms against 3.39 ms per
-		// factorisation): the deferred update starts one panel later, so less of it hides behind the critical chain, and
-		// the rank-256 look-ahead of the diagonal tile sits on that chain.
-		static const int pair_min_rows = getenv("SPP_CHOL_PAIRS")? atoi(getenv("SPP_CHOL_PAIRS")) : 0; // pair while at least this many tile rows are left
-		const bool pair_updates = pair_min_rows > 0;
-		bool pending = false; // panel b - 1 has not been applied below tile row b yet
-		bool bulk_in_flight = false, row_in_flight = false;
-		int bulk_slot = 0; // the event the last bulk update was recorded in
-		for(size_t b = 0; b < n_blk; ++ b) {
-			const size_t k0 = b * CH_NB, c0 = k0 + CH_NB;
-			const size_t n_cols = identity_tail? ld + (b + 1) * CH_NB : n_cols_all;
-			const int e = int(b & 1);
-			double *Rinv_b = Rinv + b * (size_t)(CH_NB * CH_NB);
-			stamp();
-			tic();
-			// the diagonal block asks for a whole SM's shared memory: co-resident update CTAs would compete for the FP64
-			// pipe and stretch the critical chain (measured: 33 -> 45 us)
-			k_potrf128<<<1, PT, ch.potrf_exclusive? POTRF_SMEM_EXCLUSIVE : POTRF_SMEM, sA>>>(A, ld, k0, Rinv_b, info,
-				(prof && b == 1)? ch.dbg.p() : 0);
-			LAUNCH_CHECK(ctx);
-			toc(0);
-			stamp();
-			if(!prof) {
-				SPP_CUDA(cudaEventRecord(ch.ev_potrf[e], sA));
-				if(row_in_flight) { // tile row b was last updated by the look-ahead of panel b - 1 on sC
-					SPP_CUDA(cudaStreamWaitEvent(sA, ch.ev_row[e ^ 1], 0));
-					row_in_flight = false;
-				}
-			}
-			// panel solve, critical part: the tile right of the diagonal (the rhs block for the last panel)
-			tic();
-			k_gemm_tn<GEMM_TRSM, 128, 16, 32, 16, 8><<<CH_NB / 16, 128, gemm_smem<128, 16, 8>(), sA>>>(A, ld, k0, 0, c0, Rinv_b);
-			LAUNCH_CHECK(ctx);
-			toc(1);
-			stamp();
-			if(c0 >= ld) { // last diagonal block: what is left of its block row (more than the first tile only for a panel)
-				if(n_cols > c0 + CH_NB) {
-					k_gemm_tn<GEMM_TRSM, 128, 64><<<(unsigned)((n_cols - c0 - CH_NB) / 64), 256, gemm_smem<128, 64>(), sA>>>(A, ld, k0, 0,
-						c0 + CH_NB, Rinv_b);
-					LAUNCH_CHECK(ctx);
-				}
-				break;
-			}
-			if(!prof) {
-				SPP_CUDA(cudaEventRecord(ch.ev_first[e], sA));
-				SPP_CUDA(cudaStreamWaitEvent(sC, ch.ev_potrf[e], 0));
-			}
-			// panel solve, the rest of the block row (sC; its input was written by sC itself)
-			tic();
-			k_gemm_tn<GEMM_TRSM, 128, 64><<<(unsigned)((n_cols - c0 - CH_NB) / 64), 256, gemm_smem<128, 64>(), sC>>>(A, ld, k0, 0,
-				c0 + CH_NB, Rinv_b);
-			LAUNCH_CHECK(ctx);
-			toc(1);
-			if(!prof) {
-				SPP_CUDA(cudaEventRecord(ch.ev_panel[e], sC)); // panel b is final (together with ev_first)
-				// the look-ahead updates write tile row b + 1, which the bulk update of step b - 1 also wrote
-				if(bulk_in_flight) {
-					SPP_CUDA(cudaStreamWaitEvent(sA, ch.ev_bulk[bulk_slot], 0));
-					SPP_CUDA(cudaStreamWaitEvent(sC, ch.ev_bulk[bulk_slot], 0));
-					bulk_in_flight = false;
-				}
-			}
-			// look-ahead, critical part: the next diagonal tile (32 x 32 tiles of four 16 x 16 warps: short chains)
-			const size_t ku = pending? k0 - CH_NB : k0; // first row of the panels this step applies
-			tic();
-			if(pending)
-				k_gemm_tn<GEMM_SYRK, 32, 32, 16, 16, 8, 256><<<dim3(CH_NB / 32, CH_NB / 32), 128, gemm_smem<32, 32, 8>(), sA>>>(A, ld, ku, c0, c0, 0);
-			else
-				k_gemm_tn<GEMM_SYRK, 32, 32, 16, 16, 8><<<dim3(CH_NB / 32, CH_NB / 32), 128, gemm_smem<32, 32, 8>(), sA>>>(A, ld, k0, c0, c0, 0);
-			LAUNCH_CHECK(ctx);
-			toc(3);
-			stamp();
-			// look-ahead, rest of the next panel's tile row (rhs block included)
-			if(!prof)
-				SPP_CUDA(cudaStreamWaitEvent(sC, ch.ev_first[e], 0));
-			tic();
-			// 64 x 64 tiles while they are needed to occupy the SMs (a dense matrix), 128 x 64 for the long block rows of a
-			// supernode panel
-			syrk(sC, ku, c0, c0 + CH_NB, CH_NB, n_cols - (c0 + CH_NB), ((n_cols - (c0 + CH_NB)) / 64 >= 148)? 1 : 2, pending);
-			toc(4);
-			if(!prof)
-				SPP_CUDA(cudaEventRecord(ch.ev_row[e], sC));
-			row_in_flight = true;
-			const size_t r1 = c0 + CH_NB; // first row below the next panel's tile row
-			if(r1 < ld && pair_updates && !pending && r1 + CH_NB < ld && (ld - r1) / CH_NB >= (size_t)pair_min_rows)
-				pending = true; // an even panel with at least two tile rows below the next one: its bulk update waits for the next panel
-			else if(r1 < ld) {
-				if(!prof) {
-					SPP_CUDA(cudaStreamWaitEvent(sB, ch.ev_panel[e], 0));
-					SPP_CUDA(cudaStreamWaitEvent(sB, ch.ev_first[e], 0));
-				}
-				const size_t T = (ld - r1) / 128, n_tiles = T * (T + 1) / 2 + T;
-				// 128 x 64 tiles (two CTAs per SM overlap each other's pipeline fill and epilogue: 5 % faster than 128 x 128
-				// even on the largest trailing matrices), 64 x 64 when few tiles are left
-				int tile = (n_tiles >= 74)? 1 : 2;
-				if(ch.force_tile >= 0) tile = ch.force_tile;
-				tic();
-				syrk(sB, ku, r1, r1, ld - r1, n_cols - r1, tile, pending);
-				toc(2);
-				if(!prof)
-					SPP_CUDA(cudaEventRecord(ch.ev_bulk[e], sB));
-				bulk_in_flight = true;
-				bulk_slot = e;
-				pending = false;
-			} else
-				pending = false;
-		}
-		if(timeline && !prof && !tl.empty()) {
-			cudaEventSynchronize(tl.back());
-			double t_potrf = 0, t_wait_trsm = 0, t_diag = 0, t_gap = 0;
-			size_t np = 0;
-			for(size_t i = 0; i + 3 < tl.size(); i += 4, ++ np) {
-				float a, b2, c, d = 0;
-				cudaEventElapsedTime(&a, tl[i], tl[i + 1]);
-				cudaEventElapsedTime(&b2, tl[i + 1], tl[i + 2]);
-				cudaEventElapsedTime(&c, tl[i + 2], tl[i + 3]);
-				if(i + 4 < tl.size()) cudaEventElapsedTime(&d, tl[i + 3], tl[i + 4]);
-				t_potrf += a; t_wait_trsm += b2; t_diag += c; t_gap += d;
-				if(np < 3 || np % 10 == 0)
-					fprintf(stderr, "[spp chol timeline] panel %zu: potrf %.1f us, wait+trsm_first %.1f, wait+la_diag %.1f, to next %.1f\n",
-						np, a * 1e3, b2 * 1e3, c * 1e3, d * 1e3);
-			}
-			float total;
-			cudaEventElapsedTime(&total, tl.front(), tl.back());
-			fprintf(stderr, "[spp chol timeline] %zu panels, chain total %.3f ms: potrf %.3f, wait+trsm_first %.3f, wait+la_diag %.3f, gaps %.3f\n",
-				np, total, t_potrf, t_wait_trsm, t_diag, t_gap);
-			for(size_t i = 0; i < tl.size(); ++ i) cudaEventDestroy(tl[i]);
-		}
-		if(!prof) {
-			for(int i = 0; i < 2; ++ i) { // join: whatever is still in flight on the side streams
-				if(bulk_in_flight)
-					SPP_CUDA(cudaStreamWaitEvent(sA, ch.ev_bulk[i], 0));
-				if(row_in_flight)
-					SPP_CUDA(cudaStreamWaitEvent(sA, ch.ev_row[i], 0));
-			}
+	cudaStream_t sA = ctx->stream, sB = ch.bulk_stream, sC = ch.row_stream;
+	// C(rows r0.., cols c0..) -= P^T P on the upper tiles of a (n_r x n_c) region, in 128 x 64 or 64 x 64 tiles
+	auto syrk = [&](cudaStream_t s, size_t k0, size_t r0, size_t c0, size_t n_r, size_t n_c, bool tile128) {
+		if(tile128) {
+			dim3 grid((unsigned)(n_c / 64), (unsigned)(n_r / 128));
+			k_gemm_tn<GEMM_SYRK, 128, 64><<<grid, 256, gemm_smem<128, 64>(), s>>>(A, ld, k0, r0, c0, 0);
 		} else {
-			long long h[16];
-			cudaMemcpy(h, ch.dbg.p(), sizeof(h), cudaMemcpyDeviceToHost);
-			fprintf(stderr, "[spp potrf clocks] load %lld | leaf0+rowsolve %lld | rank8 update %lld | first 32 rows %lld | factor total %lld | store %lld | inverse %lld | storeinv %lld\n",
-				h[1] - h[0], h[2] - h[1], h[3] - h[2], h[4] - h[1], h[5] - h[1], h[6] - h[5], h[7] - h[6], h[8] - h[7]);
-			fprintf(stderr, "[spp chol profile] n=%zu potrf %.3f ms, trsm %.3f, bulk %.3f, la_diag %.3f, la_row %.3f (serialised)\n",
-				n, t_acc[0], t_acc[1], t_acc[2], t_acc[3], t_acc[4]);
+			dim3 grid((unsigned)(n_c / 64), (unsigned)(n_r / 64));
+			k_gemm_tn<GEMM_SYRK, 64, 64><<<grid, 128, gemm_smem<64, 64>(), s>>>(A, ld, k0, r0, c0, 0);
 		}
+		LAUNCH_CHECK(ctx);
+	};
+	// Measured and rejected: bulk updates in pairs -- the bulk update of an even panel deferred and applied together with
+	// the next panel's as one rank-256 pass (half the launches, half the read-modify-write traffic of the trailing matrix,
+	// twice the K per tile). Bit-identical results, but slower on the Venice system (5226^2: 3.55 ms against 3.39 ms per
+	// factorisation): the deferred update starts one panel later, so less of it hides behind the critical chain, and the
+	// rank-256 look-ahead of the diagonal tile sits on that chain.
+	bool bulk_in_flight = false, row_in_flight = false;
+	int bulk_slot = 0; // the event the last bulk update was recorded in
+	for(size_t b = 0; b < n_blk; ++ b) {
+		const size_t k0 = b * CH_NB, c0 = k0 + CH_NB;
+		const size_t n_cols = identity_tail? ld + (b + 1) * CH_NB : n_cols_all;
+		const int e = int(b & 1);
+		double *Rinv_b = Rinv + b * (size_t)(CH_NB * CH_NB);
+		// the diagonal block asks for a whole SM's shared memory: co-resident update CTAs would compete for the FP64
+		// pipe and stretch the critical chain (measured: 33 -> 45 us)
+		k_potrf128<<<1, PT, POTRF_SMEM_EXCLUSIVE, sA>>>(A, ld, k0, Rinv_b, info, 0);
+		LAUNCH_CHECK(ctx);
+		SPP_CUDA(cudaEventRecord(ch.ev_potrf[e], sA));
+		if(row_in_flight) { // tile row b was last updated by the look-ahead of panel b - 1 on sC
+			SPP_CUDA(cudaStreamWaitEvent(sA, ch.ev_row[e ^ 1], 0));
+			row_in_flight = false;
+		}
+		// panel solve, critical part: the tile right of the diagonal (the rhs block for the last panel)
+		k_gemm_tn<GEMM_TRSM, 128, 16, 32, 16, 8><<<CH_NB / 16, 128, gemm_smem<128, 16, 8>(), sA>>>(A, ld, k0, 0, c0, Rinv_b);
+		LAUNCH_CHECK(ctx);
+		if(c0 >= ld) { // last diagonal block: what is left of its block row (more than the first tile only for a panel)
+			if(n_cols > c0 + CH_NB) {
+				k_gemm_tn<GEMM_TRSM, 128, 64><<<(unsigned)((n_cols - c0 - CH_NB) / 64), 256, gemm_smem<128, 64>(), sA>>>(A, ld, k0, 0,
+					c0 + CH_NB, Rinv_b);
+				LAUNCH_CHECK(ctx);
+			}
+			break;
+		}
+		SPP_CUDA(cudaEventRecord(ch.ev_first[e], sA));
+		SPP_CUDA(cudaStreamWaitEvent(sC, ch.ev_potrf[e], 0));
+		// panel solve, the rest of the block row (sC; its input was written by sC itself)
+		k_gemm_tn<GEMM_TRSM, 128, 64><<<(unsigned)((n_cols - c0 - CH_NB) / 64), 256, gemm_smem<128, 64>(), sC>>>(A, ld, k0, 0,
+			c0 + CH_NB, Rinv_b);
+		LAUNCH_CHECK(ctx);
+		SPP_CUDA(cudaEventRecord(ch.ev_panel[e], sC)); // panel b is final (together with ev_first)
+		// the look-ahead updates write tile row b + 1, which the bulk update of step b - 1 also wrote
+		if(bulk_in_flight) {
+			SPP_CUDA(cudaStreamWaitEvent(sA, ch.ev_bulk[bulk_slot], 0));
+			SPP_CUDA(cudaStreamWaitEvent(sC, ch.ev_bulk[bulk_slot], 0));
+			bulk_in_flight = false;
+		}
+		// look-ahead, critical part: the next diagonal tile (32 x 32 tiles of four 16 x 16 warps: short chains)
+		k_gemm_tn<GEMM_SYRK, 32, 32, 16, 16, 8><<<dim3(CH_NB / 32, CH_NB / 32), 128, gemm_smem<32, 32, 8>(), sA>>>(A, ld, k0, c0, c0, 0);
+		LAUNCH_CHECK(ctx);
+		// look-ahead, rest of the next panel's tile row (rhs block included)
+		SPP_CUDA(cudaStreamWaitEvent(sC, ch.ev_first[e], 0));
+		// 64 x 64 tiles while they are needed to occupy the SMs (a dense matrix), 128 x 64 for the long block rows of a
+		// supernode panel
+		syrk(sC, k0, c0, c0 + CH_NB, CH_NB, n_cols - (c0 + CH_NB), (n_cols - (c0 + CH_NB)) / 64 >= 148);
+		SPP_CUDA(cudaEventRecord(ch.ev_row[e], sC));
+		row_in_flight = true;
+		const size_t r1 = c0 + CH_NB; // first row below the next panel's tile row
+		if(r1 < ld) {
+			SPP_CUDA(cudaStreamWaitEvent(sB, ch.ev_panel[e], 0));
+			SPP_CUDA(cudaStreamWaitEvent(sB, ch.ev_first[e], 0));
+			const size_t T = (ld - r1) / 128, n_tiles = T * (T + 1) / 2 + T;
+			// 128 x 64 tiles (two CTAs per SM overlap each other's pipeline fill and epilogue: 5 % faster than 128 x 128
+			// even on the largest trailing matrices), 64 x 64 when few tiles are left
+			syrk(sB, k0, r1, r1, ld - r1, n_cols - r1, n_tiles >= 74);
+			SPP_CUDA(cudaEventRecord(ch.ev_bulk[e], sB));
+			bulk_in_flight = true;
+			bulk_slot = e;
+		}
+	}
+	for(int i = 0; i < 2; ++ i) { // join: whatever is still in flight on the side streams
+		if(bulk_in_flight)
+			SPP_CUDA(cudaStreamWaitEvent(sA, ch.ev_bulk[i], 0));
+		if(row_in_flight)
+			SPP_CUDA(cudaStreamWaitEvent(sA, ch.ev_row[i], 0));
 	}
 }
 
@@ -586,21 +460,19 @@ void dense_chol_factor_dataflow(spp_ctx *ctx, double *A, size_t ld, size_t n_col
 	}
 	DenseChol::DfTaskList &tl = ch.df_tasks[((uint64_t)NB << 32) | NJH];
 	if(!tl.n_tasks) {
-		// Worker tasks sorted by the key  i + (j - i) / beta  (row i, tile column j): row-major order with the tiles far from the
-		// diagonal pushed back behind the near-diagonal tiles of the following rows, which the critical chain needs first. Any
-		// beta > 1 keeps the order topological (a tile's operands (k, i), (k, j), k < i, have smaller keys). The partial sums
-		// of the four half tiles on the chain itself (the diagonal tile and the tile right of it) are queued `lead` rows early:
-		// a worker that takes them follows the factorisation slab by slab and is one slab away from done when the chain gets
-		// there (their operands come later in the queue: fine as long as there are more workers than 4 (lead + 1) open chain
-		// tasks; a starved launch ends in the watchdog, not in a hang).
-		static const int lead = getenv("SPP_CHOL_DF_LEAD")? atoi(getenv("SPP_CHOL_DF_LEAD")) : 1;
-		static const double beta = getenv("SPP_CHOL_DF_BETA")? atof(getenv("SPP_CHOL_DF_BETA")) : 0;
+		// Worker tasks in row-major order (row i, tile column j). The partial sums of the four half tiles on the chain itself
+		// (the diagonal tile and the tile right of it) are queued one row early: a worker that takes them follows the
+		// factorisation slab by slab and is one slab away from done when the chain gets there (their operands come later in
+		// the queue: fine as long as there are more workers than the 8 open chain tasks; a starved launch ends in the
+		// watchdog, not in a hang). Measured and rejected (profiles/r2d_*, r2e_*): queueing them 0, 2, 3, 4 or 6 rows early, and
+		// skewing the row-major order to push the tiles far from the diagonal back behind the near-diagonal tiles of the
+		// following rows.
 		std::vector<std::pair<double, uint32_t> > keyed;
 		for(size_t i = 0; i < NB; ++ i) {
 			for(size_t jh = 2 * i; jh < NJH; ++ jh) {
 				const size_t j = jh / 2;
 				const bool chain = j == i || (j == i + 1 && j < NB);
-				const double key = chain? (double)i - lead - 0.5 : (beta > 1)? i + (double)(j - i) / beta : (double)i;
+				const double key = chain? (double)i - 1.5 : (double)i;
 				keyed.push_back(std::make_pair(key, (uint32_t)((i << 16) | jh)));
 			}
 		}
@@ -695,8 +567,7 @@ void dense_chol_factor_dataflow(spp_ctx *ctx, double *A, size_t ld, size_t n_col
 void dense_chol_factor_single_panel(spp_ctx *ctx, cudaStream_t stream, double *A, size_t n_cols, double *Rinv, int *info)
 {
 	chol_init_streams(ctx);
-	DenseChol &ch = ctx->chol;
-	k_potrf128<<<1, PT, ch.potrf_exclusive? POTRF_SMEM_EXCLUSIVE : POTRF_SMEM, stream>>>(A, CH_NB, 0, Rinv, info, 0);
+	k_potrf128<<<1, PT, POTRF_SMEM_EXCLUSIVE, stream>>>(A, CH_NB, 0, Rinv, info, 0);
 	LAUNCH_CHECK(ctx);
 	if(n_cols > CH_NB) {
 		k_gemm_tn<GEMM_TRSM, 128, 64><<<(unsigned)((n_cols - CH_NB) / 64), 256, gemm_smem<128, 64>(), stream>>>(A, CH_NB, 0, 0, CH_NB, Rinv);

@@ -56,6 +56,8 @@ bool dense_chol_dataflow_enabled();
 #define JM_STAGES 3
 #define JM_THREADS 256
 
+static const double JM_BUDGET_BYTES = 4e9; // device memory of the compact F of one batch (reach rows x batch columns)
+
 enum { JM_SUB = 1 /* C -= A B (else C = A B) */, JM_A_LOWER = 2 /* A(i, k) = 0 for k > i */, JM_UPPER = 4 /* upper tiles only */ };
 
 // C(i, j) = [C(i, j) -] sum_k A(i, k) B(k, j), i < M, j < N, K = 16 n_kt; A and B both k-contiguous:
@@ -398,7 +400,6 @@ int joint_marginals_to_host(spp_ctx *ctx, double alpha, bool sparse, const std::
 		std::sort(out.begin(), out.end());
 	};
 	static const size_t forced_cols = getenv("SPP_JOINT_BATCH_COLS")? (size_t)atol(getenv("SPP_JOINT_BATCH_COLS")) : 0;
-	static const double budget = getenv("SPP_JOINT_BUDGET_GB")? atof(getenv("SPP_JOINT_BUDGET_GB")) * 1e9 : 4e9;
 	std::vector<uint64_t> out_off(n_sets + 1, 0);
 	for(size_t k = 0; k < n_sets; ++ k) {
 		uint64_t D = 0;
@@ -430,7 +431,7 @@ int joint_marginals_to_host(spp_ctx *ctx, double alpha, bool sparse, const std::
 					add_cols += (verts[q] & 0x80000000u)? 3 : 6;
 				}
 			const size_t r2 = rows + add_rows, m2 = m + add_cols;
-			const bool fits = forced_cols? m2 <= forced_cols : (double)r2 * round_up(m2, JM_BN) * 8 <= budget;
+			const bool fits = forced_cols? m2 <= forced_cols : (double)r2 * round_up(m2, JM_BN) * 8 <= JM_BUDGET_BYTES;
 			if(k1 > k0 && !fits) break;
 			for(uint32_t x : reach) if(batch_stamp[x] != bid) { batch_stamp[x] = bid; b_reach.push_back(x); }
 			for(uint64_t q = set_ptr[k1]; q < set_ptr[k1 + 1]; ++ q)

@@ -15,7 +15,6 @@
 // -- so there are no floating-point atomics and the result is bit-reproducible.
 
 #include "spp_ctx.h"
-#include <stdlib.h>
 #include <algorithm>
 
 namespace spp {
@@ -83,93 +82,33 @@ __global__ void __launch_bounds__(LI_WARPS * 32) k_landmark_inverse(size_t P, do
 // ---- the Schur product ---------------------------------------------------------------------------------
 // S(i,j) = [i == j] (U_i + alpha I) - sum_pairs Y_a W_b^T ; for i == j also b_i = gc_i - sum_a Y_a gp_{p(a)}
 //
-// Lane mapping: a warp is three groups of nine lanes (27 of 32 lanes work). Lane q = r3 + 3 c3 of a group owns the
-// 2 x 2 sub-block of ADJACENT rows {2 r3, 2 r3 + 1} x columns {2 c3, 2 c3 + 1} of the 6 x 6 product: the two rows of
-// Y_a and the two rows of W_b it needs are one 16-byte load per column of the 6 x 3 blocks (three + three LDG.128 per
-// pair, half the L1 wavefronts of 8-byte loads -- the kernel is bound by L1 wavefronts), 12 FMAs per pair; no
-// accumulator ever crosses a lane until the three groups are summed at the end (fixed order, so the result is
-// bit-reproducible). Group g of a warp takes pairs g, g + 3 * n_warps, ... of the list.
-// (Measured alternatives, Venice shape: one DMMA m8n8k4 per pair with one value per lane -- warp per block 1.15 ms,
-// pair lists cut into 128-pair work items 1.25 ms -- against 0.75 ms for this kernel: a pair is a dependent gather of two
-// 144-byte blocks and the product is bound by the latency / L2 traffic of those gathers, not by the 108 FMAs.)
+// Lane mapping: a warp is three groups of nine lanes (27 of 32 lanes work); group g of a warp takes pairs g, g + 3 * n_warps,
+// ... of the list. Lane q = r3 + 3 k of a group owns the rows {2 r3, 2 r3 + 1} of the product and ONE value k of the
+// summation index (a column of Y_a / W_b): per pair it loads its own 16-byte chunk of Y_a -- the nine lanes of a group
+// cover the 144-byte block exactly once -- and the 48 bytes of column k of W_b, i.e. four 16-byte loads and ~10 L1
+// wavefronts per pair (the kernel is L1-throughput bound); twelve accumulators per lane. No accumulator crosses a lane
+// until the end, where the three k-partials of a row pair and then the three groups are added in a fixed order, so the
+// result is bit-reproducible.
+// (Measured alternatives, Venice shape: a lane owning a 2 x 2 sub-block of the product and all three k -- six 16-byte
+// loads and ~16 L1 wavefronts per pair, L1 at 74 % of peak (profiles/r2q_full.csv). Against that mapping at 0.75 ms,
+// one DMMA m8n8k4 per pair with one value per lane -- warp per block 1.15 ms, pair lists cut into 128-pair work items
+// 1.25 ms: a pair is a dependent gather of two 144-byte blocks and the product is bound by the latency / L2 traffic of
+// those gathers, not by the 108 FMAs.)
 #define SB_WARPS 8
+#define SB_UNROLL 4 // pairs in flight per lane group
 
-struct SchurAcc {
-	double s00, s01, s10, s11, b0, b1; // (row 2 r3 + i, column 2 c3 + j) -> s_ij; b_i: rhs rows 2 r3 + i
-};
-
-template <bool RHS, int SB_UNROLL>
-__device__ __forceinline__ void schur_accumulate(uint64_t k0, uint64_t end, uint64_t stride, int r3, int c3,
-	const uint32_t *__restrict__ pair_a, const uint32_t *__restrict__ pair_b, const double *__restrict__ Y,
-	const double *__restrict__ W, const double *__restrict__ gp, const uint32_t *__restrict__ obs_pt, SchurAcc &acc)
-{
-	const double2 zero2 = make_double2(0.0, 0.0);
-	// the observation indices of a trip are fetched one trip ahead, so that the dependent chain of a trip is one
-	// memory round trip (the Y / W blocks) instead of two (index, then block)
-	unsigned oa[SB_UNROLL], ob[SB_UNROLL];
-	bool ok[SB_UNROLL];
-	#pragma unroll
-	for(int u = 0; u < SB_UNROLL; ++ u) {
-		const uint64_t kk = k0 + u * stride;
-		ok[u] = kk < end;
-		oa[u] = ok[u]? pair_a[kk] : 0u;
-		ob[u] = RHS? oa[u] : (ok[u]? pair_b[kk] : 0u);
-	}
-	for(uint64_t k = k0; k < end; k += SB_UNROLL * stride) {
-		double2 y[SB_UNROLL][3], w[SB_UNROLL][3];
-		double g[SB_UNROLL][3];
-		#pragma unroll
-		for(int u = 0; u < SB_UNROLL; ++ u) {
-			const double2 *Ya = reinterpret_cast<const double2*>(Y + (size_t)oa[u] * 18 + 2 * r3);
-			const double2 *Wb = reinterpret_cast<const double2*>(W + (size_t)ob[u] * 18 + 2 * c3);
-			#pragma unroll
-			for(int q = 0; q < 3; ++ q) { // column q of the 6 x 3 blocks: 6 doubles = 3 double2 further on
-				y[u][q] = ok[u]? Ya[q * 3] : zero2;
-				w[u][q] = ok[u]? Wb[q * 3] : zero2;
-			}
-			if(RHS) {
-				const unsigned p = ok[u]? obs_pt[oa[u]] : 0u;
-				#pragma unroll
-				for(int q = 0; q < 3; ++ q)
-					g[u][q] = ok[u]? gp[(size_t)p * 3 + q] : 0.0;
-			}
-		}
-		#pragma unroll
-		for(int u = 0; u < SB_UNROLL; ++ u) { // next trip's indices
-			const uint64_t kk = k + (SB_UNROLL + u) * stride;
-			ok[u] = kk < end;
-			oa[u] = ok[u]? pair_a[kk] : 0u;
-			ob[u] = RHS? oa[u] : (ok[u]? pair_b[kk] : 0u);
-		}
-		#pragma unroll
-		for(int u = 0; u < SB_UNROLL; ++ u) {
-			acc.s00 += y[u][0].x * w[u][0].x + y[u][1].x * w[u][1].x + y[u][2].x * w[u][2].x;
-			acc.s10 += y[u][0].y * w[u][0].x + y[u][1].y * w[u][1].x + y[u][2].y * w[u][2].x;
-			acc.s01 += y[u][0].x * w[u][0].y + y[u][1].x * w[u][1].y + y[u][2].x * w[u][2].y;
-			acc.s11 += y[u][0].y * w[u][0].y + y[u][1].y * w[u][1].y + y[u][2].y * w[u][2].y;
-			if(RHS) {
-				acc.b0 += y[u][0].x * g[u][0] + y[u][1].x * g[u][1] + y[u][2].x * g[u][2];
-				acc.b1 += y[u][0].y * g[u][0] + y[u][1].y * g[u][1] + y[u][2].y * g[u][2];
-			}
-		}
-	}
-}
-
-// Second lane mapping (MAP_K): lane q = r3 + 3 k of a group owns the rows {2 r3, 2 r3 + 1} of the product and ONE value k of
-// the summation index (a column of Y_a / W_b): per pair it loads its own 16-byte chunk of Y_a -- the nine lanes of a group
-// cover the 144-byte block exactly once -- and the 48 bytes of column k of W_b, i.e. four 16-byte loads instead of six and
-// ~10 instead of ~16 L1 wavefronts per pair (the kernel is L1-throughput bound: 74 %, profiles/r2q_full.csv); twelve
-// accumulators per lane, the three k-partials of a row pair are added at the very end (k ascending: fixed order).
 struct SchurAccK {
 	double s[2][6], b[2]; // (row 2 r3 + i, column c) partial over this lane's k; rhs rows
 };
 
-template <bool RHS, int SB_UNROLL>
+template <bool RHS>
 __device__ __forceinline__ void schur_accumulate_k(uint64_t k0, uint64_t end, uint64_t stride, int r3, int kk,
 	const uint32_t *__restrict__ pair_a, const uint32_t *__restrict__ pair_b, const double *__restrict__ Y,
 	const double *__restrict__ W, const double *__restrict__ gp, const uint32_t *__restrict__ obs_pt, SchurAccK &acc)
 {
 	const double2 zero2 = make_double2(0.0, 0.0);
+	// the observation indices of a trip are fetched one trip ahead, so that the dependent chain of a trip is one
+	// memory round trip (the Y / W blocks) instead of two (index, then block)
 	unsigned oa[SB_UNROLL], ob[SB_UNROLL];
 	bool ok[SB_UNROLL];
 	#pragma unroll
@@ -223,8 +162,13 @@ __device__ __forceinline__ double sum_over_k(double v, int lane)
 	return (v + v1) + v2;
 }
 
-// off-diagonal blocks, MAP_K lane mapping
-template <int UNROLL>
+// off-diagonal blocks (list entries first_blk ..): one warp per block. The pair lists differ a lot in length (1 .. several
+// hundred pairs), so with a fixed block -> warp assignment a CTA lives as long as its longest list while its other
+// warps idle (33 % of the warp slots active, profiles/r1k_full.csv); the warps of a persistent grid take block after
+// block from the counter `queue` instead (with four pairs in flight per lane group: stage 1.26 -> 1.19 ms; the kernel
+// is bound by the L2 sector traffic of its gathers, 2 x 144 bytes per pair, not by the imbalance). (Measured and
+// rejected: the three lane groups sharing ONE pair, each taking one column of Y_a / W_b -- the minimum of L1 wavefronts
+// per pair, but three times the index loads and loop trips per pair: 1.49 ms against 1.32 ms for the stage.)
 __global__ void __launch_bounds__(SB_WARPS * 32, 2) k_schur_blocks_k(size_t first_blk, size_t n_blocks_total, size_t ld,
 	const uint32_t *__restrict__ blk_row, const uint32_t *__restrict__ blk_col, const uint64_t *__restrict__ blk_ptr,
 	const uint32_t *__restrict__ pair_a, const uint32_t *__restrict__ pair_b, const double *__restrict__ Y,
@@ -247,7 +191,7 @@ __global__ void __launch_bounds__(SB_WARPS * 32, 2) k_schur_blocks_k(size_t firs
 			acc.b[i] = 0;
 		}
 		if(grp < 3)
-			schur_accumulate_k<false, UNROLL>(blk_ptr[blk] + grp, blk_ptr[blk + 1], 3, r3, kk, pair_a, pair_b, Y, W, 0, 0, acc);
+			schur_accumulate_k<false>(blk_ptr[blk] + grp, blk_ptr[blk + 1], 3, r3, kk, pair_a, pair_b, Y, W, 0, 0, acc);
 		#pragma unroll
 		for(int i = 0; i < 2; ++ i) {
 			#pragma unroll
@@ -269,96 +213,8 @@ __global__ void __launch_bounds__(SB_WARPS * 32, 2) k_schur_blocks_k(size_t firs
 	}
 }
 
-// off-diagonal blocks (list entries first_blk ..): one warp per block. The pair lists differ a lot in length (1 .. several
-// hundred pairs), so with a fixed block -> warp assignment a CTA lives as long as its longest list while its other
-// warps idle (33 % of the warp slots active, profiles/r1k_full.csv); with `queue` the warps of a persistent grid take
-// block after block from a counter instead (with four pairs in flight per lane group: stage 1.26 -> 1.19 ms; the kernel
-// is bound by the L2 sector traffic of its gathers, 2 x 144 bytes per pair, not by the imbalance). (Measured and rejected: the three lane groups sharing ONE pair, each taking
-// one column of Y_a / W_b -- the minimum of L1 wavefronts per pair, but three times the index loads and loop trips per
-// pair: 1.49 ms against 1.32 ms for the stage.)
-template <int UNROLL>
-__global__ void __launch_bounds__(SB_WARPS * 32, (UNROLL >= 4)? 2 : 4) k_schur_blocks(size_t first_blk, size_t n_blocks_total, size_t ld,
-	const uint32_t *__restrict__ blk_row, const uint32_t *__restrict__ blk_col, const uint64_t *__restrict__ blk_ptr,
-	const uint32_t *__restrict__ pair_a, const uint32_t *__restrict__ pair_b, const double *__restrict__ Y,
-	const double *__restrict__ W, double *__restrict__ S, const uint32_t *__restrict__ slot, unsigned *__restrict__ queue)
-{
-	const int lane = threadIdx.x & 31;
-	const int grp = lane / 9, q9 = lane - grp * 9, r3 = q9 % 3, c3 = q9 / 3;
-	for(;;) {
-	size_t blk;
-	if(queue) {
-		unsigned idx = 0;
-		if(lane == 0)
-			idx = atomicAdd(queue, 1u);
-		blk = first_blk + __shfl_sync(0xffffffffu, idx, 0);
-	} else
-		blk = first_blk + blockIdx.x * (size_t)SB_WARPS + (threadIdx.x >> 5);
-	if(blk >= n_blocks_total) return;
-	const unsigned bi = blk_row[blk], bj = blk_col[blk];
-	SchurAcc acc = {0, 0, 0, 0, 0, 0};
-	if(grp < 3)
-		schur_accumulate<false, UNROLL>(blk_ptr[blk] + grp, blk_ptr[blk + 1], 3, r3, c3, pair_a, pair_b, Y, W, 0, 0, acc);
-	// sum the three groups in a fixed order
-	double v[4] = {acc.s00, acc.s10, acc.s01, acc.s11};
-	#pragma unroll
-	for(int i = 0; i < 4; ++ i) {
-		const double v1 = __shfl_sync(0xffffffffu, v[i], (lane + 9) & 31), v2 = __shfl_sync(0xffffffffu, v[i], (lane + 18) & 31);
-		v[i] = (v[i] + v1) + v2;
-	}
-	if(lane < 9) { // ld == 0: compact block list (block blk at S + 36 blk), else the dense matrix
-		const size_t ldo = ld? ld : 6;
-		double *Sb = ld? S + ((size_t)bj * 6 + 2 * c3) * ld + (size_t)bi * 6 + 2 * r3 :
-			S + (size_t)(slot? slot[blk] : blk) * 36 + 2 * c3 * 6 + 2 * r3;
-		Sb[0] = -v[0];
-		Sb[1] = -v[1];
-		Sb[ldo] = -v[2];
-		Sb[ldo + 1] = -v[3];
-	}
-	if(!queue) return;
-	}
-}
-
 // diagonal blocks (list entries 0 .. C-1, pairs (a, a) = the camera's observations): one CTA per camera, every
 // warp group takes a strided share of the list, the 3 * SB_WARPS partial sums are added in a fixed order
-__global__ void __launch_bounds__(SB_WARPS * 32) k_schur_diag(size_t ld, double alpha, const uint64_t *__restrict__ blk_ptr,
-	const uint32_t *__restrict__ pair_a, const double *__restrict__ Y, const double *__restrict__ W,
-	const double *__restrict__ U, const double *__restrict__ gc, const double *__restrict__ gp,
-	const uint32_t *__restrict__ obs_pt, double *__restrict__ S, double *__restrict__ b, const uint32_t *__restrict__ slot)
-{
-	__shared__ double part[3 * SB_WARPS][9][6];
-	const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-	const size_t bi = blockIdx.x;
-	const int grp = lane / 9, q9 = lane - grp * 9, r3 = q9 % 3, c3 = q9 / 3;
-	SchurAcc acc = {0, 0, 0, 0, 0, 0};
-	if(grp < 3) {
-		schur_accumulate<true, 4>(blk_ptr[bi] + warp * 3 + grp, blk_ptr[bi + 1], 3 * SB_WARPS, r3, c3, pair_a, pair_a, Y, W,
-			gp, obs_pt, acc);
-		double *pp = part[warp * 3 + grp][q9];
-		pp[0] = acc.s00; pp[1] = acc.s10; pp[2] = acc.s01; pp[3] = acc.s11; pp[4] = acc.b0; pp[5] = acc.b1;
-	}
-	__syncthreads();
-	if(threadIdx.x < 9) {
-		double v[6] = {0, 0, 0, 0, 0, 0};
-		for(int s = 0; s < 3 * SB_WARPS; ++ s) {
-			#pragma unroll
-			for(int i = 0; i < 6; ++ i)
-				v[i] += part[s][q9][i];
-		}
-		const double *Ub = U + bi * 36 + 2 * c3 * 6 + 2 * r3; // column-major 6x6
-		const size_t ldo = ld? ld : 6; // ld == 0: compact block list
-		double *Sb = ld? S + (bi * 6 + 2 * c3) * ld + bi * 6 + 2 * r3 : S + (size_t)(slot? slot[bi] : bi) * 36 + 2 * c3 * 6 + 2 * r3;
-		Sb[0] = (Ub[0] + ((r3 == c3)? alpha : 0.0)) - v[0];
-		Sb[1] = Ub[1] - v[1];
-		Sb[ldo] = Ub[6] - v[2];
-		Sb[ldo + 1] = (Ub[7] + ((r3 == c3)? alpha : 0.0)) - v[3];
-		if(c3 == 0) {
-			b[bi * 6 + 2 * r3] = gc[bi * 6 + 2 * r3] - v[4];
-			b[bi * 6 + 2 * r3 + 1] = gc[bi * 6 + 2 * r3 + 1] - v[5];
-		}
-	}
-}
-
-// diagonal blocks, MAP_K lane mapping (see k_schur_blocks_k)
 __global__ void __launch_bounds__(SB_WARPS * 32, 2) k_schur_diag_k(size_t ld, double alpha, const uint64_t *__restrict__ blk_ptr,
 	const uint32_t *__restrict__ pair_a, const double *__restrict__ Y, const double *__restrict__ W,
 	const double *__restrict__ U, const double *__restrict__ gc, const double *__restrict__ gp,
@@ -376,7 +232,7 @@ __global__ void __launch_bounds__(SB_WARPS * 32, 2) k_schur_diag_k(size_t ld, do
 		acc.b[i] = 0;
 	}
 	if(grp < 3)
-		schur_accumulate_k<true, 4>(blk_ptr[bi] + warp * 3 + grp, blk_ptr[bi + 1], 3 * SB_WARPS, r3, kk, pair_a, pair_a, Y, W, gp, obs_pt, acc);
+		schur_accumulate_k<true>(blk_ptr[bi] + warp * 3 + grp, blk_ptr[bi + 1], 3 * SB_WARPS, r3, kk, pair_a, pair_a, Y, W, gp, obs_pt, acc);
 	#pragma unroll
 	for(int i = 0; i < 2; ++ i) {
 		#pragma unroll
@@ -480,43 +336,20 @@ void schur_form_reduced_system(spp_ctx *ctx, double alpha, double alpha_diag, bo
 	}
 	if(!sparse_rcs)
 		s.S.zero(ctx->stream);
-	static const int map_k = getenv("SPP_SCHUR_MAPK")? atoi(getenv("SPP_SCHUR_MAPK")) : 4;
 	if(s.C) { // list entries 0 .. C-1 are the diagonal blocks
-		if(map_k)
-			k_schur_diag_k<<<(unsigned)s.C, SB_WARPS * 32, 0, ctx->stream>>>(ld, alpha_diag, s.blk_ptr.p(), s.pair_a.p(), s.Y.p(),
-				s.W.p(), s.U.p(), s.gc.p(), s.gp.p(), s.obs_pt.p(), S_out, s.b.p(), slot);
-		else
-			k_schur_diag<<<(unsigned)s.C, SB_WARPS * 32, 0, ctx->stream>>>(ld, alpha_diag, s.blk_ptr.p(), s.pair_a.p(), s.Y.p(),
-				s.W.p(), s.U.p(), s.gc.p(), s.gp.p(), s.obs_pt.p(), S_out, s.b.p(), slot);
+		k_schur_diag_k<<<(unsigned)s.C, SB_WARPS * 32, 0, ctx->stream>>>(ld, alpha_diag, s.blk_ptr.p(), s.pair_a.p(), s.Y.p(),
+			s.W.p(), s.U.p(), s.gc.p(), s.gp.p(), s.obs_pt.p(), S_out, s.b.p(), slot);
 		LAUNCH_CHECK(ctx);
 	}
 	if(s.n_blocks > s.C) {
-		static const int unroll = getenv("SPP_SCHUR_UNROLL")? atoi(getenv("SPP_SCHUR_UNROLL")) : 4;
-		static const int use_queue = getenv("SPP_SCHUR_QUEUE")? atoi(getenv("SPP_SCHUR_QUEUE")) : 1;
-		unsigned *queue = 0;
-		unsigned grid = n_blocks(s.n_blocks - s.C, SB_WARPS);
-		if(use_queue) {
-			static int n_sms = 0;
-			if(!n_sms)
-				SPP_CUDA(cudaDeviceGetAttribute(&n_sms, cudaDevAttrMultiProcessorCount, ctx->device));
-			s.schur_queue.resize(1);
-			queue = s.schur_queue.p();
-			SPP_CUDA(cudaMemsetAsync(queue, 0, sizeof(unsigned), ctx->stream));
-			grid = std::min(grid, (unsigned)n_sms * ((unroll >= 4)? 2u : 4u));
-		}
-		if(map_k && use_queue) {
-			if(map_k >= 4)
-				k_schur_blocks_k<4><<<grid, SB_WARPS * 32, 0, ctx->stream>>>(s.C, s.n_blocks, ld,
-					s.blk_row.p(), s.blk_col.p(), s.blk_ptr.p(), s.pair_a.p(), s.pair_b.p(), s.Y.p(), s.W.p(), S_out, slot, queue);
-			else
-				k_schur_blocks_k<2><<<grid, SB_WARPS * 32, 0, ctx->stream>>>(s.C, s.n_blocks, ld,
-					s.blk_row.p(), s.blk_col.p(), s.blk_ptr.p(), s.pair_a.p(), s.pair_b.p(), s.Y.p(), s.W.p(), S_out, slot, queue);
-		} else if(unroll >= 4)
-			k_schur_blocks<4><<<grid, SB_WARPS * 32, 0, ctx->stream>>>(s.C, s.n_blocks, ld,
-				s.blk_row.p(), s.blk_col.p(), s.blk_ptr.p(), s.pair_a.p(), s.pair_b.p(), s.Y.p(), s.W.p(), S_out, slot, queue);
-		else
-			k_schur_blocks<2><<<grid, SB_WARPS * 32, 0, ctx->stream>>>(s.C, s.n_blocks, ld,
-				s.blk_row.p(), s.blk_col.p(), s.blk_ptr.p(), s.pair_a.p(), s.pair_b.p(), s.Y.p(), s.W.p(), S_out, slot, queue);
+		static int n_sms = 0;
+		if(!n_sms)
+			SPP_CUDA(cudaDeviceGetAttribute(&n_sms, cudaDevAttrMultiProcessorCount, ctx->device));
+		s.schur_queue.resize(1);
+		SPP_CUDA(cudaMemsetAsync(s.schur_queue.p(), 0, sizeof(unsigned), ctx->stream));
+		const unsigned grid = std::min(n_blocks(s.n_blocks - s.C, SB_WARPS), (unsigned)n_sms * 2u); // two CTAs per SM
+		k_schur_blocks_k<<<grid, SB_WARPS * 32, 0, ctx->stream>>>(s.C, s.n_blocks, ld, s.blk_row.p(), s.blk_col.p(),
+			s.blk_ptr.p(), s.pair_a.p(), s.pair_b.p(), s.Y.p(), s.W.p(), S_out, slot, s.schur_queue.p());
 		LAUNCH_CHECK(ctx);
 	}
 }

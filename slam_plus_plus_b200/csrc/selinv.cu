@@ -25,7 +25,6 @@
 #include "spp_ctx.h"
 #include <cuda_pipeline_primitives.h>
 #include <algorithm>
-#include <stdlib.h>
 
 namespace spp {
 
@@ -243,34 +242,28 @@ void snode_selected_inverse(spp_ctx *ctx)
 		SPP_CUDA(cudaFuncSetAttribute(k_selinv_gemm<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)selinv_gemm_smem(false)));
 		attr_done = true;
 	}
-	static const bool single_stream = getenv("SPP_SNODE_SINGLE_STREAM") != 0;
 	sc.d_sel_main.resize(std::max<size_t>(sc.selinv_main_doubles, 1));
-	sc.d_sel_lane.resize(std::max<size_t>(sc.selinv_lane_doubles * (single_stream? 1 : SupernodalChol::N_STREAMS), 1));
+	sc.d_sel_lane.resize(std::max<size_t>(sc.selinv_lane_doubles * SupernodalChol::N_STREAMS, 1));
 	bool lane_used[SupernodalChol::N_STREAMS] = {false};
 	for(size_t ss = ns; ss > 0; -- ss) {
 		const size_t s = ss - 1;
 		const size_t ld = sc.panel_ld[s], h = 6 * (size_t)(sn.row_ptr[s + 1] - sn.row_ptr[s]);
 		const bool on_lane = selinv_on_lane(ld, (h + SN_SEL_HP - 1) / SN_SEL_HP * SN_SEL_HP);
 		const int lane = int(s % SupernodalChol::N_STREAMS);
-		cudaStream_t ss_ = (on_lane && !single_stream)? sc.side[lane] : st;
-		double *scratch = on_lane? sc.d_sel_lane.p() + (single_stream? 0 : (size_t)lane * sc.selinv_lane_doubles) : sc.d_sel_main.p();
-		if(!single_stream) {
-			if(sn.parent[s] != 0xffffffffu)
-				SPP_CUDA(cudaStreamWaitEvent(ss_, sc.ev_x[sn.parent[s]], 0));
-			else
-				SPP_CUDA(cudaStreamWaitEvent(ss_, sc.ev_factor[ns - 1], 0));
-		}
+		cudaStream_t ss_ = on_lane? sc.side[lane] : st;
+		double *scratch = on_lane? sc.d_sel_lane.p() + (size_t)lane * sc.selinv_lane_doubles : sc.d_sel_main.p();
+		if(sn.parent[s] != 0xffffffffu)
+			SPP_CUDA(cudaStreamWaitEvent(ss_, sc.ev_x[sn.parent[s]], 0));
+		else
+			SPP_CUDA(cudaStreamWaitEvent(ss_, sc.ev_factor[ns - 1], 0));
 		selinv_supernode(ctx, ss_, s, scratch);
-		if(!single_stream)
-			SPP_CUDA(cudaEventRecord(sc.ev_x[s], ss_));
+		SPP_CUDA(cudaEventRecord(sc.ev_x[s], ss_));
 		if(on_lane) lane_used[lane] = true;
 	}
-	if(!single_stream) { // join the side lanes
-		for(int i = 0; i < SupernodalChol::N_STREAMS; ++ i) {
-			if(!lane_used[i]) continue;
-			SPP_CUDA(cudaEventRecord(sc.ev_target[i % ns], sc.side[i]));
-			SPP_CUDA(cudaStreamWaitEvent(st, sc.ev_target[i % ns], 0));
-		}
+	for(int i = 0; i < SupernodalChol::N_STREAMS; ++ i) { // join the side lanes
+		if(!lane_used[i]) continue;
+		SPP_CUDA(cudaEventRecord(sc.ev_target[i % ns], sc.side[i]));
+		SPP_CUDA(cudaStreamWaitEvent(st, sc.ev_target[i % ns], 0));
 	}
 }
 

@@ -51,7 +51,7 @@ struct SchurSystem {
 	DBuf<uint32_t> joint_idx, joint_dim;
 	DBuf<uint64_t> joint_off;
 	DBuf<uint8_t> joint_jobs;
-	DBuf<unsigned> schur_queue; // [1] work counter of k_schur_blocks
+	DBuf<unsigned> schur_queue; // [1] work counter of k_schur_blocks_k
 	DBuf<double> b, b_copy; // [n] reduced right-hand side / camera increment
 	DBuf<double> dxc, dxp; // [6C], [3P] increments
 	bool keep_reduced;
@@ -226,14 +226,10 @@ struct SupernodalChol {
 
 struct DenseChol {
 	DBuf<double> work;        // inverse diagonal blocks, [n_blk][128 x 128]
-	DBuf<long long> dbg;      // clock64 marks of k_potrf128 (profile mode)
 	DBuf<int> info;           // [0] first non-positive pivot (1-based), [1..] block-row flags of the backsolve
 	cudaStream_t bulk_stream; // trailing updates that overlap the next panel
 	cudaStream_t row_stream;  // look-ahead update of the next panel's tile row
 	cudaEvent_t ev_potrf[2], ev_first[2], ev_panel[2], ev_bulk[2], ev_row[2];
-	bool profile;             // SPP_CHOL_PROFILE: serialised per-kernel timing to stderr
-	bool potrf_exclusive;     // the diagonal-block kernel takes a whole SM (default; SPP_CHOL_SHARED_SM turns it off)
-	int force_tile;           // SPP_CHOL_TILE: force the bulk tile shape (0: 128x128, 1: 128x64, 2: 64x64)
 	// persistent dataflow factorisation (chol_dataflow.cuh)
 	DBuf<int> df_flags;       // task / role counters, watchdog, tile flags (zeroed before every launch)
 	struct DfTaskList { DBuf<uint32_t> codes; size_t n_tasks; DfTaskList() : n_tasks(0) {} };
@@ -243,7 +239,7 @@ struct DenseChol {
 	const void *df_A, *df_Rinv;
 	size_t df_ld, df_cols;
 	int n_sms;
-	DenseChol() : bulk_stream(0), row_stream(0), profile(false), potrf_exclusive(true), force_tile(-1), df_nb(0), df_njh(0),
+	DenseChol() : bulk_stream(0), row_stream(0), df_nb(0), df_njh(0),
 		df_n_tasks(0), df_A(0), df_Rinv(0), df_ld(0), df_cols(0), n_sms(0) {}
 };
 

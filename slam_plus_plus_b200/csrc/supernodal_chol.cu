@@ -26,7 +26,6 @@
 #include "spp_ctx.h"
 #include <cuda_pipeline_primitives.h>
 #include <algorithm>
-#include <numeric>
 #include <stdlib.h>
 
 namespace spp {
@@ -46,6 +45,14 @@ void allreduce_device(spp_ctx *ctx, double *d_ptr, size_t n);
 #define SN_LDS (SN_BK + 4)
 #define SN_STAGES 3
 #define SN_GEMV_COLS 64 // columns per CTA of the backward-solve GEMV: a short dependent chain per thread, many CTAs
+
+// relaxed amalgamation (supernodal_symbolic): a supernode merges into its parent while the explicit zeros stay below this
+// share of the merged panel, or while the merged width is at most this many block columns
+static const double SN_RELAX_ZEROS = 0.05;
+static const size_t SN_RELAX_SMALL = 16;
+// supernodes at least this many columns wide are factored by the dataflow kernel (k_chol_dataflow), narrower ones by
+// the look-ahead panel factorisation, whose panels were chain-bound on them
+static const size_t SN_DATAFLOW_MIN = 1024;
 
 static inline size_t round_up(size_t x, size_t m) { return (x + m - 1) / m * m; }
 
@@ -85,9 +92,7 @@ void snode_symbolic(spp_ctx *ctx, size_t n, const std::vector<uint32_t> &blk_row
 		sc.h_order.assign(sc.user_order.begin(), sc.user_order.end());
 	} else // approximate minimum degree, the reference's permutation (amd_exact.cpp)
 		amd_exact_ordering(n, col_ptr.data(), row_idx.data(), sc.h_order);
-	static const double relax_zeros = getenv("SPP_SNODE_RELAX")? atof(getenv("SPP_SNODE_RELAX")) : 0.05;
-	static const size_t relax_small = getenv("SPP_SNODE_SMALL")? (size_t)atoi(getenv("SPP_SNODE_SMALL")) : 16;
-	supernodal_symbolic(n, col_ptr.data(), row_idx.data(), sc.h_order, relax_zeros, relax_small, (size_t)1 << 30, sc.sn);
+	supernodal_symbolic(n, col_ptr.data(), row_idx.data(), sc.h_order, SN_RELAX_ZEROS, SN_RELAX_SMALL, (size_t)1 << 30, sc.sn);
 	const Supernodes &sn = sc.sn;
 	const size_t ns = sn.n_super();
 	std::vector<uint32_t> inv(n);
@@ -503,7 +508,6 @@ void snode_factor(spp_ctx *ctx, const double *d_Sblk, const double *d_b)
 	static bool attr_done_on[64] = {false}; // the attribute belongs to the (kernel, device) pair
 	bool &attr_done = attr_done_on[(ctx->device >= 0 && ctx->device < 64)? ctx->device : 0];
 	if(!attr_done) {
-		SPP_CUDA(cudaFuncSetAttribute(k_snode_update<128, 128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)snode_update_smem<128, 128>()));
 		SPP_CUDA(cudaFuncSetAttribute(k_snode_update<64, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)snode_update_smem<64, 64>()));
 		SPP_CUDA(cudaFuncSetAttribute(k_snode_update<128, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)snode_update_smem<128, 64>()));
 		attr_done = true;
@@ -511,8 +515,6 @@ void snode_factor(spp_ctx *ctx, const double *d_Sblk, const double *d_b)
 	const Supernodes &sn = sc.sn;
 	const size_t ns = sn.n_super(), n = sc.n;
 	cudaStream_t st = ctx->stream;
-	static const bool profile = getenv("SPP_SNODE_PROFILE") != 0;
-	static const bool single_stream = profile || getenv("SPP_SNODE_SINGLE_STREAM") != 0;
 	if(!sc.side[0]) {
 		int prio_lo = 0, prio_hi = 0;
 		SPP_CUDA(cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));
@@ -550,22 +552,9 @@ void snode_factor(spp_ctx *ctx, const double *d_Sblk, const double *d_b)
 				SPP_CUDA(cudaMemsetAsync(L + sc.panel_off[s], 0, (size_t)sc.panel_ld[s] * sc.panel_cols[s] * sizeof(double), st));
 		}
 	}
-	// SPP_SNODE_PROFILE: serialised per-supernode timing of the two parts of the numeric phase (diagnostics)
-	std::vector<float> t_factor(profile? ns : 0), t_update(profile? ns : 0);
-	auto lap = [&](float *acc) {
-		if(!profile) return;
-		cudaEventRecord(ctx->ev[5], st);
-		cudaEventSynchronize(ctx->ev[5]);
-		float ms = 0;
-		cudaEventElapsedTime(&ms, ctx->ev[4], ctx->ev[5]);
-		if(acc) *acc = ms;
-		cudaEventRecord(ctx->ev[4], st);
-	};
-	lap(0);
 	char assembled_seen[SupernodalChol::N_STREAMS] = {0};
 	int side_used[SupernodalChol::N_STREAMS] = {0};
-	if(!single_stream)
-		SPP_CUDA(cudaEventRecord(sc.ev_x[0], st)); // "panels assembled" (the backward solve re-records ev_x later)
+	SPP_CUDA(cudaEventRecord(sc.ev_x[0], st)); // "panels assembled" (the backward solve re-records ev_x later)
 	// factorisation, elimination order (a postorder: every descendant of t precedes t)
 	auto factor_and_update = [&](size_t s) {
 		double *Ps = L + sc.panel_off[s];
@@ -573,7 +562,7 @@ void snode_factor(spp_ctx *ctx, const double *d_Sblk, const double *d_b)
 		// a supernode with a single diagonal block is factored on the side stream that carries the updates into it (no
 		// event needed: same stream), so the many narrow supernodes of the lower tree levels run side by side; the wide
 		// ones use the look-ahead panel factorisation on the main stream
-		const bool on_side = !single_stream && ld == SN_NB;
+		const bool on_side = ld == SN_NB;
 		cudaStream_t sf = on_side? sc.side[s % SupernodalChol::N_STREAMS] : st;
 		if(on_side) {
 			if(!assembled_seen[s % SupernodalChol::N_STREAMS]) { // the panels were assembled on the main stream
@@ -585,14 +574,12 @@ void snode_factor(spp_ctx *ctx, const double *d_Sblk, const double *d_b)
 			if(pending[s]) // every update into this panel went to one side stream, in elimination order
 				SPP_CUDA(cudaStreamWaitEvent(st, sc.ev_target[s], 0));
 			// wide supernodes: the persistent dataflow factorisation (one kernel, no read-modify-write passes over the panel)
-			static const size_t df_min = getenv("SPP_SNODE_DATAFLOW_MIN")? (size_t)atol(getenv("SPP_SNODE_DATAFLOW_MIN")) : 1024;
-			if(df_min && ld >= df_min && dense_chol_dataflow_enabled())
+			if(ld >= SN_DATAFLOW_MIN && dense_chol_dataflow_enabled())
 				dense_chol_factor_dataflow(ctx, Ps, ld, cols, sc.d_Rinv.p() + (size_t)sc.rinv_first[s] * SN_NB * SN_NB, sc.d_info.p());
 			else
 				dense_chol_factor_panel(ctx, Ps, ld, cols, sc.d_Rinv.p() + (size_t)sc.rinv_first[s] * SN_NB * SN_NB, sc.d_info.p());
 		}
-		if(profile) lap(&t_factor[s]);
-		if(!single_stream && (sc.upd_ptr[s + 1] > sc.upd_ptr[s] || on_side))
+		if(sc.upd_ptr[s + 1] > sc.upd_ptr[s] || on_side)
 			SPP_CUDA(cudaEventRecord(sc.ev_factor[s], sf));
 		if(on_side)
 			side_used[s % SupernodalChol::N_STREAMS] = (int)s + 1; // joined before the backward solve
@@ -601,16 +588,10 @@ void snode_factor(spp_ctx *ctx, const double *d_Sblk, const double *d_b)
 		for(uint64_t q = sc.upd_ptr[s]; q < sc.upd_ptr[s + 1]; ++ q) {
 			const SnodeUpdate &u = sc.updates[q];
 			double *Pt = L + sc.panel_off[u.t];
-			cudaStream_t su = single_stream? st : sc.side[u.t % SupernodalChol::N_STREAMS];
-			if(!single_stream)
-				SPP_CUDA(cudaStreamWaitEvent(su, sc.ev_factor[s], 0));
+			cudaStream_t su = sc.side[u.t % SupernodalChol::N_STREAMS];
+			SPP_CUDA(cudaStreamWaitEvent(su, sc.ev_factor[s], 0));
 			const size_t tiles = (size_t)((u.M + 127) / 128) * ((u.N + 127) / 128);
-			static const int big_tile = getenv("SPP_SNODE_TILE")? atoi(getenv("SPP_SNODE_TILE")) : 1;
-			if(tiles >= 96 && big_tile == 0) {
-				dim3 grid((u.N + 127) / 128, (u.M + 127) / 128);
-				k_snode_update<128, 128><<<grid, 512, snode_update_smem<128, 128>(), su>>>(Ps, ld, u.col0, (uint32_t)(cols - 1), u.M, u.N,
-					n_kt, Pt, sc.panel_ld[u.t], sc.d_cmap.p() + u.map_off);
-			} else if(tiles >= 48) { // two CTAs per SM
+			if(tiles >= 48) { // two CTAs per SM
 				dim3 grid((u.N + 63) / 64, (u.M + 127) / 128);
 				k_snode_update<128, 64><<<grid, 256, snode_update_smem<128, 64>(), su>>>(Ps, ld, u.col0, (uint32_t)(cols - 1), u.M, u.N,
 					n_kt, Pt, sc.panel_ld[u.t], sc.d_cmap.p() + u.map_off);
@@ -620,12 +601,9 @@ void snode_factor(spp_ctx *ctx, const double *d_Sblk, const double *d_b)
 					n_kt, Pt, sc.panel_ld[u.t], sc.d_cmap.p() + u.map_off);
 			}
 			LAUNCH_CHECK(ctx);
-			if(!single_stream) {
-				SPP_CUDA(cudaEventRecord(sc.ev_target[u.t], su));
-				pending[u.t] = 1;
-			}
+			SPP_CUDA(cudaEventRecord(sc.ev_target[u.t], su));
+			pending[u.t] = 1;
 		}
-		if(profile) lap(&t_update[s]);
 	};
 	if(!dist) {
 		for(size_t s = 0; s < ns; ++ s)
@@ -644,19 +622,16 @@ void snode_factor(spp_ctx *ctx, const double *d_Sblk, const double *d_b)
 		}
 		for(size_t s = 0; s < ns; ++ s)
 			if(sc.owner[s] < 0) allreduce_device(ctx, L + sc.panel_off[s], (size_t)sc.panel_ld[s] * sc.panel_cols[s]);
-		if(!single_stream) { // side streams that factor narrow shared supernodes wait for the sums, not just for the assembly
-			SPP_CUDA(cudaEventRecord(sc.ev_x[0], st));
-			for(int i = 0; i < SupernodalChol::N_STREAMS; ++ i) assembled_seen[i] = 0;
-		}
+		// side streams that factor narrow shared supernodes wait for the sums, not just for the assembly
+		SPP_CUDA(cudaEventRecord(sc.ev_x[0], st));
+		for(int i = 0; i < SupernodalChol::N_STREAMS; ++ i) assembled_seen[i] = 0;
 		// ... and every rank factors the top of the tree
 		for(size_t s = 0; s < ns; ++ s)
 			if(sc.owner[s] < 0) factor_and_update(s);
 	}
-	if(!single_stream) {
-		for(int i = 0; i < SupernodalChol::N_STREAMS; ++ i) { // supernodes factored on the side streams (roots among them)
-			if(side_used[i])
-				SPP_CUDA(cudaStreamWaitEvent(st, sc.ev_factor[side_used[i] - 1], 0));
-		}
+	for(int i = 0; i < SupernodalChol::N_STREAMS; ++ i) { // supernodes factored on the side streams (roots among them)
+		if(side_used[i])
+			SPP_CUDA(cudaStreamWaitEvent(st, sc.ev_factor[side_used[i] - 1], 0));
 	}
 	if(dist) { // one status for all ranks; the increments of the subtrees are summed at the end: start from zero
 		k_snode_info_to_flag<<<1, 1, 0, st>>>(sc.d_info.p(), sc.d_flag.p());
@@ -664,29 +639,6 @@ void snode_factor(spp_ctx *ctx, const double *d_Sblk, const double *d_b)
 		allreduce_device(ctx, sc.d_flag.p(), 1);
 		k_snode_flag_to_info<<<1, 1, 0, st>>>(sc.d_flag.p(), sc.d_info.p());
 		LAUNCH_CHECK(ctx);
-	}
-	if(profile) {
-		double tf = 0, tu = 0, ff = 0, fu = 0, tf_small = 0, tu_small = 0;
-		size_t n_small = 0;
-		for(size_t s = 0; s < ns; ++ s) {
-			const double w = 6.0 * (sn.first[s + 1] - sn.first[s]), h = 6.0 * (sn.row_ptr[s + 1] - sn.row_ptr[s]);
-			tf += t_factor[s]; tu += t_update[s];
-			ff += w * w * w / 3 + w * w * h; fu += w * h * h;
-			if(w < 512) { tf_small += t_factor[s]; tu_small += t_update[s]; ++ n_small; }
-		}
-		fprintf(stderr, "[spp snode profile] %zu supernodes: panel factor %.2f ms (%.2f TFLOP/s), updates %.2f ms (%.2f TFLOP/s); "
-			"%zu supernodes narrower than 512: factor %.2f ms, updates %.2f ms\n", ns, tf, ff / tf * 1e-9, tu, fu / tu * 1e-9,
-			n_small, tf_small, tu_small);
-		std::vector<size_t> idx(ns);
-		std::iota(idx.begin(), idx.end(), 0);
-		std::sort(idx.begin(), idx.end(), [&](size_t a, size_t b) { return t_factor[a] + t_update[a] > t_factor[b] + t_update[b]; });
-		for(size_t k = 0; k < std::min<size_t>(ns, 12); ++ k) {
-			const size_t s = idx[k];
-			const double w = 6.0 * (sn.first[s + 1] - sn.first[s]), h = 6.0 * (sn.row_ptr[s + 1] - sn.row_ptr[s]);
-			fprintf(stderr, "[spp snode profile]   s %zu: w %.0f h %.0f, %llu targets: factor %.3f ms (%.1f TFLOP/s), updates %.3f ms (%.1f TFLOP/s)\n",
-				s, w, h, (unsigned long long)(sc.upd_ptr[s + 1] - sc.upd_ptr[s]), t_factor[s], (w * w * w / 3 + w * w * h) / t_factor[s] * 1e-9,
-				t_update[s], w * h * h / std::max(t_update[s], 1e-6f) * 1e-9);
-		}
 	}
 }
 
@@ -700,18 +652,10 @@ int snode_factor_solve(spp_ctx *ctx, const double *d_Sblk, const double *d_b, do
 	const size_t ns = sn.n_super(), n = sc.n;
 	cudaStream_t st = ctx->stream;
 	double *L = sc.d_L.p();
-	static const bool profile = getenv("SPP_SNODE_PROFILE") != 0;
-	static const bool single_stream = profile || getenv("SPP_SNODE_SINGLE_STREAM") != 0;
 	const bool dist = sc.distributed && ctx->world > 1;
 	if(dist) // the increments of the subtrees are summed at the end: start from zero
 		SPP_CUDA(cudaMemsetAsync(d_dx, 0, n * 6 * sizeof(double), st)); // (d_b, which d_dx may alias, went into the panels)
-	if(!single_stream)
-		SPP_CUDA(cudaEventRecord(sc.ev_factor[ns - 1], st)); // "factorisation complete"
-	auto lap = [&](float *acc) {
-		cudaEventRecord(ctx->ev[5], st);
-		cudaEventSynchronize(ctx->ev[5]);
-		cudaEventElapsedTime(acc, ctx->ev[4], ctx->ev[5]);
-	};
+	SPP_CUDA(cudaEventRecord(sc.ev_factor[ns - 1], st)); // "factorisation complete"
 	// backward solve, root to leaves; y_s sits in the rhs column of panel s. A supernode needs the x of its ancestors
 	// only: supernodes go round-robin to the side streams and wait for their parent's event (which implies the
 	// grandparents'), so independent subtrees are solved side by side
@@ -724,14 +668,12 @@ int snode_factor_solve(spp_ctx *ctx, const double *d_Sblk, const double *d_b, do
 		const size_t h = 6 * (size_t)(sn.row_ptr[s + 1] - sn.row_ptr[s]);
 		double *y = Ps + (ld + h) * ld;
 		const int lane = int(s % SupernodalChol::N_STREAMS);
-		cudaStream_t sb = single_stream? st : sc.side[lane];
-		double *part = sc.d_part.p() + (single_stream? 0 : (size_t)lane * std::max<size_t>(sc.max_part, 1));
-		if(!single_stream) {
-			if(sn.parent[s] != 0xffffffffu)
-				SPP_CUDA(cudaStreamWaitEvent(sb, sc.ev_x[sn.parent[s]], 0));
-			else
-				SPP_CUDA(cudaStreamWaitEvent(sb, sc.ev_factor[ns - 1], 0)); // the factorisation is complete (recorded below)
-		}
+		cudaStream_t sb = sc.side[lane];
+		double *part = sc.d_part.p() + (size_t)lane * std::max<size_t>(sc.max_part, 1);
+		if(sn.parent[s] != 0xffffffffu)
+			SPP_CUDA(cudaStreamWaitEvent(sb, sc.ev_x[sn.parent[s]], 0));
+		else
+			SPP_CUDA(cudaStreamWaitEvent(sb, sc.ev_factor[ns - 1], 0)); // the factorisation is complete (recorded above)
 		if(h) {
 			const size_t n_chunks = (h + SN_GEMV_COLS - 1) / SN_GEMV_COLS;
 			k_snode_gemv<<<dim3((unsigned)(ld / 128), (unsigned)n_chunks), 128, 0, sb>>>(Ps, ld, h, sc.d_rows.p() + sn.row_ptr[s],
@@ -745,22 +687,14 @@ int snode_factor_solve(spp_ctx *ctx, const double *d_Sblk, const double *d_b, do
 		k_snode_store_x<<<n_blocks(w, 128), 128, 0, sb>>>(w, 6 * (size_t)sn.first[s], y, sc.d_order.p(), sc.d_x.p(), d_dx,
 			!dist || sc.owner[s] >= 0 || ctx->rank == 0);
 		LAUNCH_CHECK(ctx);
-		if(!single_stream)
-			SPP_CUDA(cudaEventRecord(sc.ev_x[s], sb));
+		SPP_CUDA(cudaEventRecord(sc.ev_x[s], sb));
 	}
-	if(!single_stream) { // join the side streams
-		for(int i = 0; i < SupernodalChol::N_STREAMS; ++ i) {
-			SPP_CUDA(cudaEventRecord(sc.ev_target[i % ns], sc.side[i]));
-			SPP_CUDA(cudaStreamWaitEvent(st, sc.ev_target[i % ns], 0));
-		}
+	for(int i = 0; i < SupernodalChol::N_STREAMS; ++ i) { // join the side streams
+		SPP_CUDA(cudaEventRecord(sc.ev_target[i % ns], sc.side[i]));
+		SPP_CUDA(cudaStreamWaitEvent(st, sc.ev_target[i % ns], 0));
 	}
 	if(dist)
 		allreduce_device(ctx, d_dx, n * 6); // every rank needs all the camera increments
-	if(profile) {
-		float t_back = 0;
-		lap(&t_back);
-		fprintf(stderr, "[spp snode profile] backward solve %.2f ms\n", t_back);
-	}
 	if(ctx->async_mode && ctx->async_info) { // the caller synchronises later and reads the status there
 		SPP_CUDA(cudaMemcpyAsync(ctx->async_info, sc.d_info.p(), sizeof(int), cudaMemcpyDeviceToHost, st));
 		return SPP_OK;
