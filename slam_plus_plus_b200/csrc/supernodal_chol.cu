@@ -56,6 +56,15 @@ static const size_t SN_DATAFLOW_MIN = 1024;
 
 static inline size_t round_up(size_t x, size_t m) { return (x + m - 1) / m * m; }
 
+// the code path of a supernode and of an update, from the panel shapes: the numeric phase dispatches on these, the
+// SPP_SNODE_VERBOSE line of the analysis counts them
+static inline bool snode_on_side(size_t ld) { return ld == SN_NB; }               // one diagonal block: a side stream
+static inline bool snode_dataflow(size_t ld) { return ld >= SN_DATAFLOW_MIN; }    // k_chol_dataflow (SPP_CHOL_DATAFLOW != 0)
+static inline bool snode_update_tile128(const SnodeUpdate &u)                     // k_snode_update<128, 64>: two CTAs per SM
+{
+	return (size_t)((u.M + 127) / 128) * ((u.N + 127) / 128) >= 48;
+}
+
 // ---- host: symbolic -----------------------------------------------------------------------------------------
 
 // blk_row / blk_col: the upper block list of the reduced camera system (i <= j, any order, diagonal blocks present)
@@ -268,10 +277,23 @@ void snode_symbolic(spp_ctx *ctx, size_t n, const std::vector<uint32_t> &blk_row
 	sc.d_info.resize(1 + n_rinv);
 	sc.d_flag.resize(1);
 	SPP_CUDA(cudaStreamSynchronize(st));
-	if(getenv("SPP_SNODE_VERBOSE"))
-		fprintf(stderr, "[spp snode] n %zu, S blocks %zu, supernodes %zu, factor blocks %llu (exact %llu), panels %.2f GB, %.3e flops, %zu updates\n",
+	if(getenv("SPP_SNODE_VERBOSE")) {
+		size_t n_side = 0, n_look = 0, n_flow = 0, n_sel_lane = 0, max_ld = 0, max_h = 0, n_tile128 = 0;
+		for(size_t s = 0; s < ns; ++ s) {
+			const size_t ld = sc.panel_ld[s], h = 6 * (size_t)(sn.row_ptr[s + 1] - sn.row_ptr[s]);
+			if(snode_on_side(ld)) ++ n_side; else if(snode_dataflow(ld)) ++ n_flow; else ++ n_look;
+			n_sel_lane += selinv_on_lane(ld, round_up(h, SN_SEL_HP));
+			max_ld = std::max(max_ld, ld);
+			max_h = std::max(max_h, h);
+		}
+		for(const SnodeUpdate &u : sc.updates) n_tile128 += snode_update_tile128(u);
+		fprintf(stderr, "[spp snode] n %zu, S blocks %zu, supernodes %zu, factor blocks %llu (exact %llu), panels %.2f GB, %.3e flops, %zu updates; "
+			"supernodes on the side streams %zu, look-ahead %zu, dataflow %zu (ld >= %zu); largest ld %zu, largest h %zu; "
+			"updates on 128x64 tiles %zu, on 64x64 tiles %zu; selected inversion on the side lanes %zu\n",
 			n, nb, ns, (unsigned long long)sn.nnzb_factor, (unsigned long long)sn.nnzb_exact, total * 8e-9, sc.factor_flops,
-			sc.updates.size());
+			sc.updates.size(), n_side, n_look, n_flow, SN_DATAFLOW_MIN, max_ld, max_h, n_tile128, sc.updates.size() - n_tile128,
+			n_sel_lane);
+	}
 	sc.sym_row = blk_row; sc.sym_col = blk_col; sc.sym_user_order = sc.user_order;
 	sc.sym_world = ctx->world; sc.sym_rank = ctx->rank;
 	sc.sym_kept = true;
@@ -562,7 +584,7 @@ void snode_factor(spp_ctx *ctx, const double *d_Sblk, const double *d_b)
 		// a supernode with a single diagonal block is factored on the side stream that carries the updates into it (no
 		// event needed: same stream), so the many narrow supernodes of the lower tree levels run side by side; the wide
 		// ones use the look-ahead panel factorisation on the main stream
-		const bool on_side = ld == SN_NB;
+		const bool on_side = snode_on_side(ld);
 		cudaStream_t sf = on_side? sc.side[s % SupernodalChol::N_STREAMS] : st;
 		if(on_side) {
 			if(!assembled_seen[s % SupernodalChol::N_STREAMS]) { // the panels were assembled on the main stream
@@ -574,7 +596,7 @@ void snode_factor(spp_ctx *ctx, const double *d_Sblk, const double *d_b)
 			if(pending[s]) // every update into this panel went to one side stream, in elimination order
 				SPP_CUDA(cudaStreamWaitEvent(st, sc.ev_target[s], 0));
 			// wide supernodes: the persistent dataflow factorisation (one kernel, no read-modify-write passes over the panel)
-			if(ld >= SN_DATAFLOW_MIN && dense_chol_dataflow_enabled())
+			if(snode_dataflow(ld) && dense_chol_dataflow_enabled())
 				dense_chol_factor_dataflow(ctx, Ps, ld, cols, sc.d_Rinv.p() + (size_t)sc.rinv_first[s] * SN_NB * SN_NB, sc.d_info.p());
 			else
 				dense_chol_factor_panel(ctx, Ps, ld, cols, sc.d_Rinv.p() + (size_t)sc.rinv_first[s] * SN_NB * SN_NB, sc.d_info.p());
@@ -590,8 +612,7 @@ void snode_factor(spp_ctx *ctx, const double *d_Sblk, const double *d_b)
 			double *Pt = L + sc.panel_off[u.t];
 			cudaStream_t su = sc.side[u.t % SupernodalChol::N_STREAMS];
 			SPP_CUDA(cudaStreamWaitEvent(su, sc.ev_factor[s], 0));
-			const size_t tiles = (size_t)((u.M + 127) / 128) * ((u.N + 127) / 128);
-			if(tiles >= 48) { // two CTAs per SM
+			if(snode_update_tile128(u)) {
 				dim3 grid((u.N + 63) / 64, (u.M + 127) / 128);
 				k_snode_update<128, 64><<<grid, 256, snode_update_smem<128, 64>(), su>>>(Ps, ld, u.col0, (uint32_t)(cols - 1), u.M, u.N,
 					n_kt, Pt, sc.panel_ld[u.t], sc.d_cmap.p() + u.map_off);
